@@ -2,9 +2,11 @@
 """Benchmark of the ideal-ballooning hot path: field-line solves/sec (fp64, lambda_max + eigenvector).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
-                    [--workload d3d|ncsx|hberg|salpha|adjoint] [--equilibria E] [--strong]
+                    [--workload d3d|ncsx|hberg|salpha|adjoint] [--equilibria E] [--strong] [--dump-outputs DIR]
 
-One *step* = one pass of the hot path over one batch of synthetic input.
+One *step* = one pass of the hot path over one batch of synthetic input; ``--steps`` is the number of timed steps.  The
+inputs are seeded: the same arguments give the same inputs in every run, and ``--dump-outputs`` stores what the last timed
+step computed, so that two builds can be compared output for output.
 
 scan workloads (BASELINE.json configs[1..3]; default ``d3d`` = configs[1], the config the metric is quoted on):
     K1 geometry (ns x nalpha field lines) -> K2+K3 with the guarded per-surface arg-max fused into the solver kernel
@@ -371,7 +373,7 @@ def run_reference_arm(args):
         return
     vals = []
     t_all = time.perf_counter()
-    steps = max(1, min(args.steps, 3))
+    steps = args.steps
     for _ in range(steps):
         v, cores, sample, wall, kind_cpu = cpu_reference_rate(args.workload)
         vals.append(v)
@@ -415,6 +417,7 @@ class Harness:
         self.flush = torch.empty(256 * 1024 * 1024 // 8, dtype=torch.float64, device=self.dev)     # > 126 MB L2
         self.sampler = None
         self.is_last = False
+        self.last_out = None
 
     def barrier(self):
         if self.world > 1:
@@ -427,9 +430,10 @@ class Harness:
             self.dist.all_reduce(t, op=self.dist.ReduceOp.MAX)
         return t.item()
 
-    def timed(self, step, nstage, steps=None, warmup=None, sample_clocks=True):
+    def timed(self, step, nstage, steps=None, warmup=None, sample_clocks=True, keep_last=False):
         """`step(timers)` records nstage+1 events.  Returns (total seconds = max over ranks of the summed step times, per-stage
-        ms array (steps, nstage), per-step ms, wall seconds)."""
+        ms array (steps, nstage), per-step ms, wall seconds).  `keep_last`: what the last timed step returned is left in
+        ``self.last_out`` (for --dump-outputs; the caller clears it)."""
         torch = self.torch
         steps = steps or self.args.steps
         warmup = max(self.args.warmup, 3) if warmup is None else warmup
@@ -467,9 +471,12 @@ class Harness:
             t_wall = time.perf_counter()
             for k in range(steps):
                 self.is_last = k == steps - 1
-                step(timers[k])
+                out = step(timers[k])
+                if not self.is_last:
+                    out = None                  # released right away, so every step reuses the blocks the previous one freed
                 self.flush.zero_()              # L2 flush between timed iterations (outside the event brackets)
             self.is_last = False
+            self.last_out = out if keep_last else None
             self.barrier()
         finally:
             if gc_was:
@@ -497,6 +504,27 @@ class Harness:
 def rec(t, ev_idx):
     if t is not None:
         t[ev_idx].record()
+
+
+def dump_outputs(dirname, arrays, limit=60 << 20):
+    """``--dump-outputs``: write each device tensor of ``arrays`` (one row per solve / point / surface on axis 0) as
+    ``dirname/<name>.npy`` in float64, under ``limit`` bytes in all.  Smallest first, an array is stored whole when it fits
+    an equal share of what is left, else as the rows of a fixed seeded sample (their indices in ``<name>_rows.npy``): the
+    same arguments always store the same elements, so two builds can be compared output for output."""
+    import torch
+    os.makedirs(dirname, exist_ok=True)
+    items = sorted(arrays.items(), key=lambda kv: kv[1].numel())
+    left = limit
+    for i, (name, t) in enumerate(items):
+        share = left // (len(items) - i)
+        if 8 * t.numel() > share:
+            row = 8 * t[0].numel() + 8
+            rows = np.sort(np.random.default_rng(0).choice(t.shape[0], share // row, replace=False))
+            np.save(os.path.join(dirname, name + "_rows.npy"), rows.astype(np.float64))
+            t = t.index_select(0, torch.from_numpy(rows).to(t.device))
+            left -= 8 * len(rows)
+        np.save(os.path.join(dirname, name + ".npy"), t.double().cpu().numpy())
+        left -= 8 * t.numel()
 
 
 def fp64_rooflines(H, entries):
@@ -559,16 +587,21 @@ def run_scan(H, args):
                 if H.is_last:
                     g.wait()
             rec(t, 3)
-            return sol
+            return sol, g.recv, sig
         return step
 
     main_case = make_case(E, 0 if args.strong else 1000 * rank, args.strong)
     step = make_step(main_case)
-    sol = step(None)
+    sol = step(None)[0]
     torch.cuda.synchronize()
     nbad = int(np.count_nonzero((sol.info >> 16).cpu().numpy() & 3))
     mean_iters = float((sol.info & 0xFFFF).double().mean().item())
-    total_s, stage, t_step, wall = H.timed(step, 3)
+    total_s, stage, t_step, wall = H.timed(step, 3, keep_last=bool(args.dump_outputs))
+    if args.dump_outputs and rank == 0:
+        sol_l, surface_max, sig_l = H.last_out
+        dump_outputs(args.dump_outputs, {"gamma": sol_l.lam, "X": sol_l.X, "flags": sol_l.info >> 16,
+                                         "surface_max": surface_max.reshape(-1, 2), "sigma0": sig_l})
+    H.last_out = sol_l = None
     nsolve_all = main_case["ns_total"] * na * nt
     value = nsolve_all * args.steps / total_s
     t_geo, t_solve, t_coll = stage[:, 0], stage[:, 1], stage[:, 2]
@@ -577,7 +610,7 @@ def run_scan(H, args):
     single = None
     if not args.strong and E != 1 and not args.no_single:
         c1 = make_case(1, 777 + 1000 * rank, False)
-        k1 = max(10, min(args.steps, 50))
+        k1 = max(10, min(args.steps, 50))      # the secondary figures (this one, e2e) keep their own step counts
         tot1, st1, ts1, _ = H.timed(make_step(c1), 3, steps=k1, sample_clocks=False)
         single = {"value": c1["nsolve"] * world * k1 / tot1, "unit": "solves/s", "ms_per_step": 1e3 * tot1 / k1,
                   "solves_per_step_per_gpu": c1["nsolve"],
@@ -722,7 +755,11 @@ def run_salpha(H, args):
     torch.cuda.synchronize()
     nbad = int(np.count_nonzero((sol.info >> 16).cpu().numpy() & 3))
     mean_iters = float((sol.info & 0xFFFF).double().mean().item())
-    total_s, stage, t_step, wall = H.timed(step, 2)
+    total_s, stage, t_step, wall = H.timed(step, 2, keep_last=bool(args.dump_outputs))
+    if args.dump_outputs and rank == 0:
+        sol_l, cls_l = H.last_out
+        dump_outputs(args.dump_outputs, {"gamma": sol_l.lam, "X": sol_l.X, "flags": sol_l.info >> 16, "unstable": cls_l})
+    H.last_out = sol_l = None
     nsolve_all = len(shat) * len(alpha) * len(theta0)
     value = nsolve_all * args.steps / total_s
     clocks = H.clocks()
@@ -803,13 +840,17 @@ def run_adjoint(H, args):
         if world > 1:                    # the one exchange of this workload: gradients of every rank's points (16 B per point)
             H.dist.all_gather_into_tensor(grads.view(-1), grad.view(-1))
         rec(t, 3)
-        return val, grad, info
+        return val, grad, info, X, dX
 
-    val, grad, info = step(None)
+    val, grad, info = step(None)[:3]
     torch.cuda.synchronize()
     nbad = int(np.count_nonzero((info >> 16).cpu().numpy() & 3))
     mean_iters = float((info & 0xFFFF).double().mean().item())
-    total_s, stage, t_step, wall = H.timed(step, 3)
+    total_s, stage, t_step, wall = H.timed(step, 3, keep_last=bool(args.dump_outputs))
+    if args.dump_outputs and rank == 0:
+        val_l, grad_l, info_l, X_l, dX_l = H.last_out
+        dump_outputs(args.dump_outputs, {"val": val_l, "grad": grad_l, "X": X_l, "dX": dX_l, "flags": info_l >> 16})
+    H.last_out = X_l = dX_l = None
     value = world * npts * args.steps / total_s
     clocks = H.clocks()
     e2e = None
@@ -890,10 +931,17 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-e2e-full", action="store_true", help="skip the second end-to-end figure (X of every solve over PCIe)")
     ap.add_argument("--no-single", action="store_true", help="skip the single-equilibrium measurement of the default line")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed (rank 0) as DIR/<name>.npy, float64, at most 64 MB: arrays "
+                         "too large for that as a fixed seeded sample of their rows, indices in DIR/<name>_rows.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.equilibria is None:
         args.equilibria = 37 if args.workload == "d3d" else 1
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs applies to the GPU implementation")
         return run_reference_arm(args)
     H = Harness(args)
     if args.workload == "salpha":

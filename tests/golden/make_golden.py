@@ -159,7 +159,35 @@ def s_alpha_fixture():
     np.savez_compressed(os.path.join(HERE, "s_alpha.npz"), **out)
 
 
+def live_small(u):
+    """The small case of tests/test_oracle.py::test_live_reference_small: the reference's own splines and field line on a
+    synthetic D3D-like equilibrium (seed 5, s = 0.6, alpha = 0.4, 129 points on +-2 pi), and its converged gamma_ball_full at
+    theta0 = 0.3 on the restatement's coefficients of that line (so that the eigensolvers see identical input)."""
+    from oracle import ballooning_oracle as bo
+    from ideal_ballooning_solver_b200 import tables
+    wout = synthetic.make_equilibrium("d3d", seed=5)
+    theta = np.linspace(-2 * np.pi, 2 * np.pi, 129)
+    fl_ref = u.vmec_fieldlines(u.vmec_splines(ref_shim.FakeVmec(wout)), 0.6, np.array([0.4]), theta1d=theta)
+    out = {"geo_" + k: getattr(fl_ref, k)[0][0] for k in bo.HOT_FIELDS}
+    fl = bo.fieldlines(tables.RadialSplines(wout).evaluate([0.6]), np.array([0.4]), theta)
+    cv, gd = bo.theta0_shift(fl, 0.3)
+    with ref_shim.converged_arpack(u):
+        out["lam_conv"], out["X_conv"], *_ = u.gamma_ball_full(bo.dpdrho_of(fl), theta, fl.bmag[0][0], fl.gradpar_theta_pest[0][0],
+                                                               cv, gd, bo.default_vguess(theta), 1.0)
+    return out
+
+
+def live_small_fixture():
+    out = live_small(u)
+    np.savez_compressed(os.path.join(HERE, "live_small.npz"), **out)
+    print("live_small lam_conv", out["lam_conv"])
+
+
 if __name__ == "__main__":
+    if sys.argv[1:] == ["live_small"]:
+        live_small_fixture()
+        sys.exit(0)
+    live_small_fixture()
     s_alpha_fixture()
     # the only real equilibrium shipped with the reference
     wout = ref_shim.wout_from_netcdf(os.path.join(ref_shim.REFERENCE_ROOT, "tests", "comparn_w_COBRAVMEC",

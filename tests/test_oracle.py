@@ -1,6 +1,8 @@
 """CPU: pin the oracle (oracle/ballooning_oracle.py) against the golden fixtures that were generated
 from the UNMODIFIED reference (tests/golden/make_golden.py), and -- when /root/reference is present
 (build container only) -- against the reference itself, live."""
+import os
+
 import numpy as np
 import pytest
 
@@ -104,28 +106,41 @@ def test_scan_theta_grid():
     assert len(bo.scan_theta_grid(80, 0)) == 641 and len(bo.scan_theta_grid(11, 11)) == 969   # ball_scan.py:201-208
 
 
-@pytest.mark.skipif(not ref_shim.reference_available(), reason="/root/reference not present (GPU box)")
+LIVE_SMALL = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "live_small.npz")
+
+
+def _live_small_sources():
+    """The reference's outputs for the small case of ``live_small_fixture`` (tests/golden/make_golden.py): as stored in
+    tests/golden/live_small.npz, and computed live when the unmodified reference is importable."""
+    if os.path.isfile(LIVE_SMALL):
+        D = np.load(LIVE_SMALL)
+        yield "stored", {k: D[k] for k in D.files}
+    if ref_shim.reference_available():
+        import importlib.util
+        spec = importlib.util.spec_from_file_location("make_golden", os.path.join(os.path.dirname(LIVE_SMALL), "make_golden.py"))
+        make_golden = importlib.util.module_from_spec(spec)
+        spec.loader.exec_module(make_golden)
+        yield "live", make_golden.live_small(make_golden.u)
+
+
+@pytest.mark.skipif(not (os.path.isfile(LIVE_SMALL) or ref_shim.reference_available()),
+                    reason="neither tests/golden/live_small.npz nor the unmodified reference (IBS_REFERENCE_ROOT) is present")
 def test_live_reference_small():
-    """Live: the unmodified reference (through oracle/ref_shim.py) vs the restatement on a small case."""
+    """The unmodified reference (its stored outputs, and live through oracle/ref_shim.py when present) vs the restatement on
+    a small case: its own splines and field line on a synthetic D3D-like equilibrium, then gamma_ball_full at theta0 = 0.3."""
     from ideal_ballooning_solver_b200 import synthetic, tables
-    u = ref_shim.load_reference_utils()
-    wout = synthetic.make_equilibrium("d3d", seed=5)
-    vs = u.vmec_splines(ref_shim.FakeVmec(wout))
     theta = np.linspace(-2 * np.pi, 2 * np.pi, 129)
-    fl_ref = u.vmec_fieldlines(vs, 0.6, np.array([0.4]), theta1d=theta)
-    tab = tables.RadialSplines(wout).evaluate([0.6])
+    tab = tables.RadialSplines(synthetic.make_equilibrium("d3d", seed=5)).evaluate([0.6])
     fl = bo.fieldlines(tab, np.array([0.4]), theta)
-    for k in bo.HOT_FIELDS:
-        ref = getattr(fl_ref, k)[0][0]
-        assert np.max(np.abs(getattr(fl, k)[0][0] - ref)) / np.max(np.abs(ref)) < 1e-9, k
     dP = bo.dpdrho_of(fl)
     cv, gd = bo.theta0_shift(fl, 0.3)
-    vg = bo.default_vguess(theta)
-    with ref_shim.converged_arpack(u):
-        ref = u.gamma_ball_full(dP, theta, fl.bmag[0][0], fl.gradpar_theta_pest[0][0], cv, gd, vg, 1.0)
     got = bo.gamma_ball_full(dP, theta, fl.bmag[0][0], fl.gradpar_theta_pest[0][0], cv, gd, method="lambda_max")
-    np.testing.assert_allclose(got[0], ref[0], rtol=1e-10)
-    np.testing.assert_allclose(sign_normalise(got[1]), sign_normalise(ref[1]), rtol=0, atol=1e-8)
+    for source, ref in _live_small_sources():
+        for k in bo.HOT_FIELDS:
+            r = ref["geo_" + k]
+            assert np.max(np.abs(getattr(fl, k)[0][0] - r)) / np.max(np.abs(r)) < 1e-9, (source, k)
+        np.testing.assert_allclose(got[0], ref["lam_conv"], rtol=1e-10, err_msg=source)
+        np.testing.assert_allclose(sign_normalise(got[1]), sign_normalise(ref["X_conv"]), rtol=0, atol=1e-8, err_msg=source)
 
 
 def _derm_cases(G):
