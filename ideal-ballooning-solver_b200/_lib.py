@@ -29,6 +29,8 @@ SIGNATURES = {
                                   c_int, c_double, c_int, c_double, _D, _I, c_void_p]),
     "ibs_geometry_adjoint": (c_int, [_D, _D, _D, _D, _D, _D, _D, c_int, c_int, c_int, c_double, c_double, _D, _D, c_int, c_double,
                                      _D, _D, _D, _D, _D, _D, _D, _D, c_void_p]),
+    "ibs_geometry_adjoint_scal": (c_int, [_D, _D, _D, _D, _D, _D, _D, c_int, c_int, c_int, c_double, c_double, _D, _D, c_int,
+                                          c_double, _D, _D, _D, _D, _D, _D, _D, _D, _D, _D, c_void_p]),
     "ibs_solve_gcf_batch": (c_int, [_D, _D, _D, c_int, c_int, c_double, _D, _D, c_int, _D, _D, _D, _D, _I, c_void_p]),
     "ibs_solve_base_batch": (c_int, [_D, _D, _D, _I, c_int, c_int, c_int, c_double, _D, _D, c_int,
                                      _D, _D, _D, _D, _D, _D, _D, _I, c_void_p]),

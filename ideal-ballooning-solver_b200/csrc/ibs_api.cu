@@ -33,7 +33,8 @@ int geometry_adjoint_dispatch(const double* tab_mn, const double* tab_nyq, const
                               const double* xm_nyq, const double* xn_nyq, int ns, int mnmax, int mnmax_nyq, double phiedge,
                               double aminor_p, const double* alpha, const double* theta, int nl, double phi_center,
                               const double* theta0, const double* dPdrho, const double* sg, const double* sc, const double* sf,
-                              const double* Q, double* grad_mn, double* grad_nyq, cudaStream_t st);
+                              const double* Q, double* grad_mn, double* grad_nyq, double* grad_scal, double* grad_glob,
+                              cudaStream_t st);
 int geometry_full_nfields();
 int geometry_full_dispatch(const double* tab_mn, const double* tab_nyq, const double* bsupumnc, const double* scal,
                            const double* xm, const double* xn, const double* xm_nyq, const double* xn_nyq,
@@ -219,8 +220,25 @@ int ibs_geometry_adjoint(const double* tab_mn, const double* tab_nyq, const doub
                 dlam_df && Q && grad_mn_out && grad_nyq_out, "null pointer");
     IBS_REQUIRE(aminor_p > 0.0 && phiedge != 0.0, "Aminor_p must be > 0 and phiedge != 0");
     return geometry_adjoint_dispatch(tab_mn, tab_nyq, scal, xm, xn, xm_nyq, xn_nyq, ns, mnmax, mnmax_nyq, phiedge, aminor_p, alpha, theta,
+                                     nl, phi_center, theta0, dPdrho, dlam_dg, dlam_dc, dlam_df, Q, grad_mn_out, grad_nyq_out, nullptr,
+                                     nullptr, (cudaStream_t)stream);
+}
+
+int ibs_geometry_adjoint_scal(const double* tab_mn, const double* tab_nyq, const double* scal,
+                              const double* xm, const double* xn, const double* xm_nyq, const double* xn_nyq,
+                              int ns, int mnmax, int mnmax_nyq, double phiedge, double aminor_p,
+                              const double* alpha, const double* theta, int nl, double phi_center,
+                              const double* theta0, const double* dPdrho, const double* dlam_dg, const double* dlam_dc,
+                              const double* dlam_df, const double* Q, double* grad_mn_out, double* grad_nyq_out,
+                              double* grad_scal_out, double* grad_glob_out, void* stream) {
+    IBS_REQUIRE(ns >= 0 && nl >= 1 && mnmax >= 1 && mnmax_nyq >= 1, "bad sizes");
+    if (ns == 0) return IBS_OK;
+    IBS_REQUIRE(tab_mn && tab_nyq && scal && xm && xn && xm_nyq && xn_nyq && alpha && theta && theta0 && dPdrho && dlam_dg && dlam_dc &&
+                dlam_df && Q && grad_mn_out && grad_nyq_out && grad_scal_out && grad_glob_out, "null pointer");
+    IBS_REQUIRE(aminor_p > 0.0 && phiedge != 0.0, "Aminor_p must be > 0 and phiedge != 0");
+    return geometry_adjoint_dispatch(tab_mn, tab_nyq, scal, xm, xn, xm_nyq, xn_nyq, ns, mnmax, mnmax_nyq, phiedge, aminor_p, alpha, theta,
                                      nl, phi_center, theta0, dPdrho, dlam_dg, dlam_dc, dlam_df, Q, grad_mn_out, grad_nyq_out,
-                                     (cudaStream_t)stream);
+                                     grad_scal_out, grad_glob_out, (cudaStream_t)stream);
 }
 
 int ibs_solve_gcf_batch(const double* g, const double* c, const double* f, int nsolve, int N, double h,

@@ -15,8 +15,15 @@
 //   stage B (one thread per (surface, mode)):  the transposed mode sum over the points of the line,
 //       d lam / d rmnc[mn] = sum_j ( v_R cos a - m v_Rt sin a + n v_Rp sin a ),  a = m theta_vmec - n phi,   etc.
 // Gradients are with respect to the per-surface tables tab_mn (6 rows) and tab_nyq (7 rows) at fixed scalars (iota, shat,
-// p', iota'): the same perturbations scan.hellmann_feynman_gamma takes.  Not a hot kernel: ns field lines (each surface's
-// arg-max line), direct mode sums.
+// p', iota') and globals (phiedge, Aminor_p).  ibs_geometry_adjoint_scal adds the stage-A instantiation SCAL = true, which
+// forms per point only the total d Phi_j / dx of the seven scalars K1 reads -- x = s, iota, iota', p', shat (scal columns
+// 0-4), phiedge, Aminor_p -- by seven forward sweeps, and geo_adjoint_scal_sum_kernel sums them over the line in a fixed order
+// (deterministic).  The table part is the same two kernels with the same launches as ibs_geometry_adjoint, so its outputs are
+// bit-identical (a point kernel doing both the table and the scalar sweeps did not reproduce them bit for bit).  iota also
+// moves the field line, phi = phi_c + (theta_p - alpha) / iota, hence the mode sums through a = m theta_vmec - n phi with
+//     d S_r / d iota = (P_r + T_r theta_phi) d phi / d iota,   P_r = d S_r / d phi at fixed theta_vmec,
+//     theta_phi = d theta_vmec / d phi = -S_Lp / (1 + S_Lt)    (implicit function of the Newton residual).
+// Not a hot kernel: ns field lines (each surface's arg-max line), direct mode sums.
 #include "ibs_common.cuh"
 
 namespace ibs {
@@ -34,18 +41,29 @@ __device__ __forceinline__ D1 operator-(D1 a) { return {-a.v, -a.d}; }
 __device__ __forceinline__ D1 operator*(D1 a, D1 b) { return {a.v * b.v, a.d * b.v + a.v * b.d}; }
 __device__ __forceinline__ D1 operator/(D1 a, D1 b) { const double q = a.v / b.v; return {q, (a.d - q * b.d) / b.v}; }
 __device__ __forceinline__ D1 dabs(D1 a) { return a.v < 0.0 ? D1{-a.v, -a.d} : a; }
+// the per-surface constants are double (table sweeps) or D1 (scalar sweeps)
+__device__ __forceinline__ double cabs(double a) { return fabs(a); }
+__device__ __forceinline__ D1 cabs(D1 a) { return dabs(a); }
+__device__ __forceinline__ double csqrt(double a) { return sqrt(a); }
+__device__ __forceinline__ D1 csqrt(D1 a) { const double r = sqrt(a.v); return {r, 0.5 * a.d / r}; }
+__device__ __forceinline__ double cval(double a) { return a; }
+__device__ __forceinline__ double cval(D1 a) { return a.v; }
 
 constexpr int NSUM = 19;
 enum { S_R, S_Rs, S_Rt, S_Rp, S_Zs, S_Zt, S_Zp, S_Ls, S_Lt, S_Lp, S_sqrtg, S_B, S_Bs, S_Bt, S_Bp, S_Bsupp, S_Bsubs, S_Bsubt, S_Bsubp };
 
+constexpr int NSX = 7;    // scalar sweeps: scal columns 0..4 (s, iota, iota', p', shat), phiedge, Aminor_p
+
+template <class C>
 struct PointConst {
-    double sp, cp, dphi;                  // sin / cos(phi), phi - phi_center
-    double iota, d_iota, dpds, shat, s_val, psi_e, L_ref;
+    C sp, cp, dphi;                       // sin / cos(phi), phi - phi_center
+    C iota, d_iota, dpds, shat, s_val, psi_e, L_ref;
     double th0, dP, sg, sc, sf, qw;       // theta0, dPdrho, the three sensitivities of this point, Q / (2 N)
 };
 
 // Phi_j as a function of the 19 mode sums (the pointwise algebra of geo_point_epilogue, ibs_geometry.cu, on T = D1)
-__device__ D1 phi_point(const D1 (&S)[NSUM], const PointConst& k) {
+template <class C>
+__device__ D1 phi_point(const D1 (&S)[NSUM], const PointConst<C>& k) {
     const D1 R = S[S_R], R_s = S[S_Rs], R_t = S[S_Rt], R_p = S[S_Rp], Z_s = S[S_Zs], Z_t = S[S_Zt], Z_p = S[S_Zp];
     const D1 L_s = S[S_Ls], L_t = S[S_Lt], L_p = S[S_Lp];
     const D1 sqrtg = S[S_sqrtg], B = S[S_B], B_s = S[S_Bs], B_t = S[S_Bt], B_p = S[S_Bp], Bsup_p = S[S_Bsupp];
@@ -67,9 +85,10 @@ __device__ D1 phi_point(const D1 (&S)[NSUM], const PointConst& k) {
                         Bsub_s * B_p * a_t) * isg;
     const D1 ga_ga = gax * gax + gay * gay + gaz * gaz, ga_gq = gax * gqx + gay * gqy + gaz * gqz, gq_gq = gqx * gqx + gqy * gqy + gqz * gqz;
     const D1 BxgB_gq = (Bsub_t * B_p - Bsub_p * B_t) * isg * psi_e;
-    const double L_ref = k.L_ref, B_ref = 2.0 * fabs(k.psi_e) / (L_ref * L_ref);
-    const double sgn = (k.psi_e > 0.0) ? 1.0 : ((k.psi_e < 0.0) ? -1.0 : 0.0);
-    const double sqrt_s = sqrt(k.s_val), mu0 = 4.0 * 3.141592653589793 * 1.0e-7;
+    const C L_ref = k.L_ref, B_ref = 2.0 * cabs(k.psi_e) / (L_ref * L_ref);
+    const double sgn = (cval(k.psi_e) > 0.0) ? 1.0 : ((cval(k.psi_e) < 0.0) ? -1.0 : 0.0);
+    const C sqrt_s = csqrt(k.s_val);
+    const double mu0 = 4.0 * 3.141592653589793 * 1.0e-7;
     const D1 B3 = B * B * B;
     const D1 bmag = B / D1(B_ref);
     const D1 gradpar = D1(L_ref * k.iota) * Bsup_p / B;
@@ -98,15 +117,18 @@ struct GeoAdjParams {
     double phi_center, psi_e, L_ref;
     double* work;          // [ns][NSUM + 3][nl]: v_r (19), u, theta_vmec, phi
     double* grad_mn; double* grad_nyq;
+    double* work_scal;     // [ns][NSX][nl]: d Phi_j / dx of the scalar sweeps (ibs_geometry_adjoint_scal only)
+    double* grad_scal; double* grad_glob;      // [ns][IBS_NSCAL], [ns][2]
 };
 
+template <bool SCAL>
 __global__ void __launch_bounds__(128)
 geo_adjoint_point_kernel(const GeoAdjParams p) {
     const long long pt = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (pt >= (long long)p.ns * p.nl) return;
     const int js = (int)(pt / p.nl), jl = (int)(pt - (long long)js * p.nl);
     const double* sc = p.scal + (size_t)js * IBS_NSCAL;
-    PointConst k;
+    PointConst<double> k;
     k.s_val = sc[0]; k.iota = sc[1]; k.d_iota = sc[2]; k.dpds = sc[3]; k.shat = sc[4];
     k.psi_e = p.psi_e; k.L_ref = p.L_ref;
     const double theta_p = p.theta[jl], phi = p.phi_center + (theta_p - p.alpha[js]) / k.iota;
@@ -132,8 +154,10 @@ geo_adjoint_point_kernel(const GeoAdjParams p) {
         if (fabs(dth) <= 4.5e-16 * fmax(1.0, fabs(th))) break;
     }
     // the 19 sums and their theta_vmec-derivatives
-    double S[NSUM], T[NSUM];
+    double S[NSUM], T[NSUM], P[NSUM];      // P_r = d S_r / d phi at fixed theta_vmec (SCAL only)
     for (int r = 0; r < NSUM; ++r) { S[r] = 0.0; T[r] = 0.0; }
+    if constexpr (SCAL)
+        for (int r = 0; r < NSUM; ++r) P[r] = 0.0;
     for (int q = 0; q < mn; ++q) {
         const double m = p.xm[q], n = p.xn[q];
         double sa, ca;
@@ -149,6 +173,11 @@ geo_adjoint_point_kernel(const GeoAdjParams p) {
         S[S_Ls] += ls * sa;      T[S_Ls] += ls * m * ca;
         S[S_Lt] += l * m * ca;   T[S_Lt] -= l * m * m * sa;
         S[S_Lp] -= l * n * ca;   T[S_Lp] += l * n * m * sa;
+        if constexpr (SCAL) {
+            P[S_R] += r * n * sa;    P[S_Rs] += rs * n * sa;  P[S_Rt] += r * m * n * ca;  P[S_Rp] -= r * n * n * ca;
+            P[S_Zs] -= zs * n * ca;  P[S_Zt] += z * m * n * sa;  P[S_Zp] -= z * n * n * sa;
+            P[S_Ls] -= ls * n * ca;  P[S_Lt] += l * m * n * sa;  P[S_Lp] -= l * n * n * sa;
+        }
     }
     for (int q = 0; q < mq; ++q) {
         const double m = p.xm_nyq[q], n = p.xn_nyq[q];
@@ -164,20 +193,46 @@ geo_adjoint_point_kernel(const GeoAdjParams p) {
         S[S_Bsubs] += s_ * sa;   T[S_Bsubs] += s_ * m * ca;
         S[S_Bsubt] += u_ * ca;   T[S_Bsubt] -= u_ * m * sa;
         S[S_Bsubp] += v_ * ca;   T[S_Bsubp] -= v_ * m * sa;
+        if constexpr (SCAL) {
+            P[S_sqrtg] += g * n * sa;  P[S_B] += b * n * sa;  P[S_Bs] += bs * n * sa;  P[S_Bt] += b * m * n * ca;
+            P[S_Bp] -= b * n * n * ca;  P[S_Bsupp] += bv * n * sa;  P[S_Bsubs] -= s_ * n * ca;  P[S_Bsubt] += u_ * n * sa;
+            P[S_Bsubp] += v_ * n * sa;
+        }
     }
-    // v_r = d Phi / d S_r by 19 forward sweeps; dPhi/dtheta_vmec = sum_r v_r T_r
-    double* w = p.work + (size_t)js * (NSUM + 3) * p.nl + jl;
-    double dth = 0.0;
-    for (int r = 0; r < NSUM; ++r) {
-        D1 Sd[NSUM];
-        for (int q = 0; q < NSUM; ++q) Sd[q] = D1(S[q], q == r ? 1.0 : 0.0);
-        const double v = phi_point(Sd, k).d;
-        w[(size_t)r * p.nl] = v;
-        dth = fma(v, T[r], dth);
+    if constexpr (!SCAL) {
+        // v_r = d Phi / d S_r by 19 forward sweeps; dPhi/dtheta_vmec = sum_r v_r T_r
+        double* w = p.work + (size_t)js * (NSUM + 3) * p.nl + jl;
+        double dth = 0.0;
+        for (int r = 0; r < NSUM; ++r) {
+            D1 Sd[NSUM];
+            for (int q = 0; q < NSUM; ++q) Sd[q] = D1(S[q], q == r ? 1.0 : 0.0);
+            const double v = phi_point(Sd, k).d;
+            w[(size_t)r * p.nl] = v;
+            dth = fma(v, T[r], dth);
+        }
+        w[(size_t)NSUM * p.nl] = -dth / (1.0 + S[S_Lt]);          // weight of d(lmns) sin a (implicit theta_vmec)
+        w[(size_t)(NSUM + 1) * p.nl] = th;
+        w[(size_t)(NSUM + 2) * p.nl] = phi;
+    } else {
+        // total d Phi_j / dx, one sweep per scalar x; only iota moves the point (phi, hence sin / cos phi and the sums)
+        const double dphi_di = -k.dphi / k.iota;
+        const double th_phi = -S[S_Lp] / (1.0 + S[S_Lt]);
+        double* ws = p.work_scal + (size_t)js * NSX * p.nl + jl;
+        for (int x = 0; x < NSX; ++x) {
+            const auto seed = [x](int which, double d) { return x == which ? d : 0.0; };
+            const double e = seed(1, dphi_di);
+            PointConst<D1> kd;
+            kd.sp = D1(k.sp, k.cp * e); kd.cp = D1(k.cp, -k.sp * e); kd.dphi = D1(k.dphi, e);
+            kd.s_val = D1(k.s_val, seed(0, 1.0)); kd.iota = D1(k.iota, seed(1, 1.0)); kd.d_iota = D1(k.d_iota, seed(2, 1.0));
+            kd.dpds = D1(k.dpds, seed(3, 1.0)); kd.shat = D1(k.shat, seed(4, 1.0));
+            kd.psi_e = D1(k.psi_e, seed(5, -1.0 / (2.0 * 3.141592653589793)));         // psi_e = -phiedge / 2 pi
+            kd.L_ref = D1(k.L_ref, seed(6, 1.0));                                      // L_ref = Aminor_p
+            kd.th0 = k.th0; kd.dP = k.dP; kd.sg = k.sg; kd.sc = k.sc; kd.sf = k.sf; kd.qw = k.qw;
+            D1 Sd[NSUM];
+            for (int r = 0; r < NSUM; ++r) Sd[r] = D1(S[r], (P[r] + T[r] * th_phi) * e);
+            ws[(size_t)x * p.nl] = phi_point(Sd, kd).d;
+        }
     }
-    w[(size_t)NSUM * p.nl] = -dth / (1.0 + S[S_Lt]);          // weight of d(lmns) sin a (implicit theta_vmec)
-    w[(size_t)(NSUM + 1) * p.nl] = th;
-    w[(size_t)(NSUM + 2) * p.nl] = phi;
 }
 
 // stage B: one thread per (surface, mode); modes 0 .. mnmax-1 of the (R, Z, lambda) set, then the Nyquist set
@@ -225,24 +280,46 @@ geo_adjoint_mode_kernel(const GeoAdjParams p) {
     }
 }
 
+// stage B of the scalar sweeps: one thread per (surface, scalar), the sum over the line in point order
+__global__ void __launch_bounds__(128)
+geo_adjoint_scal_sum_kernel(const GeoAdjParams p) {
+    const int t = blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= p.ns * NSX) return;
+    const int js = t / NSX, x = t - js * NSX;
+    const double* ws = p.work_scal + (size_t)t * p.nl;
+    double a = 0.0;
+    for (int j = 0; j < p.nl; ++j) a += ws[j];
+    if (x < 5) p.grad_scal[(size_t)js * IBS_NSCAL + x] = a;
+    else p.grad_glob[(size_t)js * 2 + (x - 5)] = a;
+    if (x == 0)                                                    // pressure and the spare columns: K1 does not read them
+        for (int c = 5; c < IBS_NSCAL; ++c) p.grad_scal[(size_t)js * IBS_NSCAL + c] = 0.0;
+}
+
 int geometry_adjoint_dispatch(const double* tab_mn, const double* tab_nyq, const double* scal, const double* xm, const double* xn,
                               const double* xm_nyq, const double* xn_nyq, int ns, int mnmax, int mnmax_nyq, double phiedge,
                               double aminor_p, const double* alpha, const double* theta, int nl, double phi_center,
                               const double* theta0, const double* dPdrho, const double* sg, const double* sc, const double* sf,
-                              const double* Q, double* grad_mn, double* grad_nyq, cudaStream_t st) {
+                              const double* Q, double* grad_mn, double* grad_nyq, double* grad_scal, double* grad_glob,
+                              cudaStream_t st) {
     if (ns == 0) return IBS_OK;
+    const bool scal_out = grad_scal != nullptr;
     GeoAdjParams p;
     p.tab_mn = tab_mn; p.tab_nyq = tab_nyq; p.scal = scal; p.xm = xm; p.xn = xn; p.xm_nyq = xm_nyq; p.xn_nyq = xn_nyq;
     p.ns = ns; p.mnmax = mnmax; p.mnmax_nyq = mnmax_nyq; p.nl = nl; p.alpha = alpha; p.theta = theta; p.theta0 = theta0; p.dPdrho = dPdrho;
     p.sg = sg; p.sc = sc; p.sf = sf; p.Q = Q; p.phi_center = phi_center; p.psi_e = -phiedge / (2.0 * 3.141592653589793); p.L_ref = aminor_p;
-    p.grad_mn = grad_mn; p.grad_nyq = grad_nyq;
+    p.grad_mn = grad_mn; p.grad_nyq = grad_nyq; p.grad_scal = grad_scal; p.grad_glob = grad_glob;
     keep_pool_cached();
-    IBS_CUDA_CHECK(cudaMallocAsync((void**)&p.work, (size_t)ns * (NSUM + 3) * nl * sizeof(double), st));
+    const size_t nwork = (size_t)ns * (NSUM + 3) * nl;
+    IBS_CUDA_CHECK(cudaMallocAsync((void**)&p.work, (nwork + (scal_out ? (size_t)ns * NSX * nl : 0)) * sizeof(double), st));
+    p.work_scal = scal_out ? p.work + nwork : nullptr;
     const long long npt = (long long)ns * nl;
-    geo_adjoint_point_kernel<<<(unsigned)((npt + 127) / 128), 128, 0, st>>>(p);
+    const unsigned npb = (unsigned)((npt + 127) / 128);
+    geo_adjoint_point_kernel<false><<<npb, 128, 0, st>>>(p);
+    if (scal_out) geo_adjoint_point_kernel<true><<<npb, 128, 0, st>>>(p);
     int rc = (cudaGetLastError() == cudaSuccess) ? IBS_OK : IBS_ERR_CUDA;
     if (rc == IBS_OK) {
         geo_adjoint_mode_kernel<<<dim3((mnmax + mnmax_nyq + 127) / 128, ns), 128, 0, st>>>(p);
+        if (scal_out) geo_adjoint_scal_sum_kernel<<<(ns * NSX + 127) / 128, 128, 0, st>>>(p);
         if (cudaGetLastError() != cudaSuccess) rc = IBS_ERR_CUDA;
     }
     if (rc != IBS_OK) set_error("geometry adjoint kernel launch failed");

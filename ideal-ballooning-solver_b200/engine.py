@@ -304,9 +304,12 @@ def adjoint_sensitivities(lam, X, dX, f):
     return tuple(outs)
 
 
-def geometry_adjoint(tables: DeviceTables, alpha, theta, theta0, dPdrho, dlam_dg, dlam_dc, dlam_df, Q, phi_center: float = 0.0):
+def geometry_adjoint(tables: DeviceTables, alpha, theta, theta0, dPdrho, dlam_dg, dlam_dc, dlam_df, Q, phi_center: float = 0.0,
+                     want_scalars: bool = False):
     """Reverse mode of K1 (``ibs_geometry_adjoint``): ``d lambda / d tab_mn (ns, 6, mnmax)`` and ``d lambda / d tab_nyq
-    (ns, 7, mnmax_nyq)`` for one field line per surface, from the per-point Hellmann-Feynman sensitivities."""
+    (ns, 7, mnmax_nyq)`` for one field line per surface, from the per-point Hellmann-Feynman sensitivities.
+    ``want_scalars=True`` (``ibs_geometry_adjoint_scal``) also returns ``d lambda / d scal (ns, 8)`` (per column, the others
+    held fixed; columns 5-7 are 0) and ``(d lambda / d phiedge, d lambda / d Aminor_p) (ns, 2)``."""
     _lib.require_cuda()
     lib = _lib.load()
     dev = tables.tab_mn.device
@@ -318,11 +321,18 @@ def geometry_adjoint(tables: DeviceTables, alpha, theta, theta0, dPdrho, dlam_dg
     xm, xn, xmq, xnq = up(tables.xm), up(tables.xn), up(tables.xm_nyq), up(tables.xn_nyq)
     gmn = torch.empty_like(tables.tab_mn)
     gnq = torch.empty_like(tables.tab_nyq)
+    args = (_ptr(tables.tab_mn), _ptr(tables.tab_nyq), _ptr(tables.scal), _ptr(xm), _ptr(xn), _ptr(xmq), _ptr(xnq),
+            ns, xm.numel(), xmq.numel(), tables.phiedge, tables.Aminor_p, _ptr(alpha), _ptr(theta), nl,
+            float(phi_center), _ptr(theta0), _ptr(dP), _ptr(sg), _ptr(sc), _ptr(sf), _ptr(Q), _ptr(gmn), _ptr(gnq))
+    if want_scalars:
+        gsc = torch.empty_like(tables.scal)
+        ggl = torch.empty((ns, 2), dtype=torch.float64, device=dev)
+        with torch.cuda.device(dev):
+            rc = lib.ibs_geometry_adjoint_scal(*args, _ptr(gsc), _ptr(ggl), _stream())
+        _lib.check(rc, "ibs_geometry_adjoint_scal")
+        return gmn, gnq, gsc, ggl
     with torch.cuda.device(dev):
-        rc = lib.ibs_geometry_adjoint(_ptr(tables.tab_mn), _ptr(tables.tab_nyq), _ptr(tables.scal), _ptr(xm), _ptr(xn), _ptr(xmq), _ptr(xnq),
-                                      ns, xm.numel(), xmq.numel(), tables.phiedge, tables.Aminor_p, _ptr(alpha), _ptr(theta), nl,
-                                      float(phi_center), _ptr(theta0), _ptr(dP), _ptr(sg), _ptr(sc), _ptr(sf), _ptr(Q), _ptr(gmn), _ptr(gnq),
-                                      _stream())
+        rc = lib.ibs_geometry_adjoint(*args, _stream())
     _lib.check(rc, "ibs_geometry_adjoint")
     return gmn, gnq
 

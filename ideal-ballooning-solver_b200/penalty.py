@@ -5,10 +5,12 @@ its forward-difference Jacobian, exactly as the reference's optimiser forms them
 ``sims_runner_NCSX.py:254-261``: ``df0[i] = (f0_i - f0_0) / step_i * 0.5 / sqrt(f0_0)``.
 Second half of f3: ``hf_jacobian`` forms the same Jacobian from ONE scan of the base equilibrium plus the first-order
 change of every surface's maximum growth rate under each perturbed equilibrium instead of ``ndofs + 1`` full scans.  That
-change comes either from ``scan.table_gradient(...).predict(tables0, tables_pert)`` -- reverse mode through K1
-(``ibs_geometry_adjoint``): the gradient with respect to every Fourier table coefficient once, then one dot product per
-degree of freedom -- or from ``scan.hellmann_feynman_gamma`` (K1 on the arg-max field lines of each perturbed table set +
-one K4 contraction, no eigen-solve), its finite-perturbation form.
+change comes either from ``scan.table_gradient(..., scalars=True).predict(tables0, tables_pert)`` -- reverse mode through
+K1 (``ibs_geometry_adjoint_scal``): the gradient with respect to every Fourier table coefficient, the surface scalars (iota,
+iota', p', shat, s), phiedge and Aminor_p once, then one dot product per degree of freedom (``scalars=False`` counts the
+Fourier tables only: enough for DOFs that move neither iota, the pressure nor phiedge) -- or from
+``scan.hellmann_feynman_gamma`` (K1 on the arg-max field lines of each perturbed table set + one K4 contraction, no
+eigen-solve), its finite-perturbation form.
 The perturbed equilibria themselves (VMEC runs) stay outside this package.
 """
 from __future__ import annotations

@@ -437,22 +437,30 @@ class TableGradient:
     gamma: np.ndarray          # (ns,) growth rate at (alpha*, theta0*)
     grad_mn: torch.Tensor      # (ns, 6, mnmax)      d gamma / d tab_mn
     grad_nyq: torch.Tensor     # (ns, 7, mnmax_nyq)  d gamma / d tab_nyq
+    grad_scal: Optional[torch.Tensor] = None    # (ns, 8)  d gamma / d scal (table_gradient(..., scalars=True))
+    grad_glob: Optional[torch.Tensor] = None    # (ns, 2)  d gamma / d (phiedge, Aminor_p)
 
     def predict(self, tables0: engine.DeviceTables, tables_pert) -> np.ndarray:
-        """First-order change of every surface's growth rate for each perturbed table set: ``(ndof, ns)``."""
+        """First-order change of every surface's growth rate for each perturbed table set: ``(ndof, ns)``.  With the scalar
+        gradients present the changes of ``scal``, ``phiedge`` and ``Aminor_p`` count too; without them they are ignored."""
         out = []
         for tp in tables_pert:
             d = ((tp.tab_mn - tables0.tab_mn) * self.grad_mn).sum(dim=(1, 2)) + ((tp.tab_nyq - tables0.tab_nyq) * self.grad_nyq).sum(dim=(1, 2))
+            if self.grad_scal is not None:
+                d = (d + ((tp.scal - tables0.scal) * self.grad_scal).sum(1) + (tp.phiedge - tables0.phiedge) * self.grad_glob[:, 0]
+                     + (tp.Aminor_p - tables0.Aminor_p) * self.grad_glob[:, 1])
             out.append(d.cpu().numpy())
         return np.array(out).reshape(len(out), -1)
 
 
-def table_gradient(tables0: engine.DeviceTables, alpha_star, theta0_star, theta) -> TableGradient:
+def table_gradient(tables0: engine.DeviceTables, alpha_star, theta0_star, theta, scalars: bool = False) -> TableGradient:
     """SURVEY.md section 8 row f3: the gradient of every surface's maximum growth rate with respect to EVERY Fourier table
     coefficient of its surface, from one eigen-solve per surface -- reverse mode through K1 (``ibs_geometry_adjoint``): K1 on
     the arg-max line -> K2/K3 -> per-point Hellmann-Feynman sensitivities (K4, ``utils.py:1676-1680``) -> adjoint of the
     geometry.  The ``ndofs`` perturbed-equilibrium scans of ``sims_runner_NCSX.py:245-262`` become ``ndofs`` dot products
-    (``TableGradient.predict``); ``hellmann_feynman_gamma`` (one K1 per DOF) is the finite-perturbation form of the same."""
+    (``TableGradient.predict``); ``hellmann_feynman_gamma`` (one K1 per DOF) is the finite-perturbation form of the same.
+    ``scalars=True`` (``ibs_geometry_adjoint_scal``) adds the gradient with respect to the surface scalars (iota, iota', p',
+    shat, s) and to phiedge / Aminor_p: needed whenever a degree of freedom moves iota, the pressure or phiedge."""
     dev = tables0.tab_mn.device
     theta_np = theta.cpu().numpy() if isinstance(theta, torch.Tensor) else np.asarray(theta, dtype=np.float64)
     h = engine.grid_spacing(theta_np)
@@ -463,8 +471,8 @@ def table_gradient(tables0: engine.DeviceTables, alpha_star, theta0_star, theta)
     sg, sc, sf = engine.adjoint_sensitivities(sol.lam, sol.X, sol.dX, sol.f)
     dP = geo.dPdrho.reshape(-1)
     Q = (sc * sol.c).sum(dim=1) / (-dP)
-    gmn, gnq = engine.geometry_adjoint(tables0, a.reshape(-1), theta_np, t0, dP, sg, sc, sf, Q)
-    return TableGradient(sol.lam.cpu().numpy(), gmn, gnq)
+    grads = engine.geometry_adjoint(tables0, a.reshape(-1), theta_np, t0, dP, sg, sc, sf, Q, want_scalars=scalars)
+    return TableGradient(sol.lam.cpu().numpy(), *grads)
 
 
 def save_results(path: str, dof_idx: int, iter0: int, result: BallScanResult) -> None:

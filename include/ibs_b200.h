@@ -107,7 +107,8 @@ int ibs_geometry_full(const double* tab_mn, const double* tab_nyq, const double*
  * ndofs + 1 perturbed-equilibrium scans of sims_runner_NCSX.py:245-262 by ONE scan + this call + dot products with the
  * table perturbations).  Chains the Hellmann-Feynman sensitivities of ibs_adjoint_sensitivities (utils.py:1676-1680) through
  * g, c, f (utils.py:1560-1562), the theta0 shift (ball_scan.py:267-268), dPdrho (ball_scan.py:262), the pointwise geometry
- * (utils.py:474-720), the theta_vmec root (utils.py:391-416) and the mode sums (utils.py:432-468), at fixed iota(s), p'(s).
+ * (utils.py:474-720), the theta_vmec root (utils.py:391-416) and the mode sums (utils.py:432-468), at fixed iota(s), p'(s)
+ * (ibs_geometry_adjoint_scal below adds the derivatives with respect to those scalars).
  *   tables / modes as ibs_geometry_full (ALL device pointers); alpha [ns], theta0 [ns], dPdrho [ns]: the line of each surface;
  *   dlam_dg, dlam_dc, dlam_df [ns][nl]; Q [ns] = sum_j dlam_dc_j c_j / (-dPdrho);
  *   grad_mn_out [ns][6][mnmax], grad_nyq_out [ns][7][mnmax_nyq]: d lambda / d tab_mn, d lambda / d tab_nyq.              */
@@ -117,6 +118,23 @@ int ibs_geometry_adjoint(const double* tab_mn, const double* tab_nyq, const doub
                          const double* alpha, const double* theta, int nl, double phi_center,
                          const double* theta0, const double* dPdrho, const double* dlam_dg, const double* dlam_dc,
                          const double* dlam_df, const double* Q, double* grad_mn_out, double* grad_nyq_out, void* stream);
+
+/* The same reverse mode, plus the derivative of each surface's lambda with respect to the scalar inputs K1 reads.  Arguments
+ * as ibs_geometry_adjoint (same order; grad_mn_out and grad_nyq_out are bit-identical to its outputs), then
+ *   grad_scal_out [ns][8]: d lambda / d scal[js][k] in the column order of scal (s, iota, d_iota_d_s, d_pressure_d_s, shat;
+ *          columns 5-7 -- pressure and the two spares -- are not read by K1 and are exactly 0);
+ *   grad_glob_out [ns][2]: (d lambda / d phiedge, d lambda / d Aminor_p) of each surface's lambda.
+ * Each is a partial derivative per column with the other columns held fixed: iota, iota' and shat = -2 s iota' / iota are
+ * separate inputs of K1.  A consistent perturbation of an equilibrium moves all three; the dot product of these gradients
+ * with the actual column differences then gives the total first-order change.  One fixed-order sum per surface: two calls
+ * on the same input give identical bits.                                                                                 */
+int ibs_geometry_adjoint_scal(const double* tab_mn, const double* tab_nyq, const double* scal,
+                              const double* xm, const double* xn, const double* xm_nyq, const double* xn_nyq,
+                              int ns, int mnmax, int mnmax_nyq, double phiedge, double aminor_p,
+                              const double* alpha, const double* theta, int nl, double phi_center,
+                              const double* theta0, const double* dPdrho, const double* dlam_dg, const double* dlam_dc,
+                              const double* dlam_df, const double* Q, double* grad_mn_out, double* grad_nyq_out,
+                              double* grad_scal_out, double* grad_glob_out, void* stream);
 
 /* ---- K2+K3: discretisation + lambda_max + eigenfunction -------------------------------------------
  * Batched gamma_ball_full (utils.py:1550-1624): g, c, f -> half-grid g, second-order finite
