@@ -155,32 +155,24 @@ argmax_kernel(const double* __restrict__ gamma, int ngrid, double* __restrict__ 
     __shared__ int snan[RED_THREADS / 32];
     const int s = blockIdx.x;
     const double* gm = gamma + (size_t)s * ngrid;
-    double bv = -1e308 * 10;   // -inf
+    double bv = -INFINITY;
     int bi = 0x7fffffff, anynan = 0;
     for (int j = threadIdx.x; j < ngrid; j += blockDim.x) {
         const double v = gm[j];
         if (v != v) anynan = 1;
-        if (v > bv || (v == bv && j < bi)) { bv = v; bi = j; }
+        best_merge(bv, bi, v, j);
     }
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) {
-        const double ov = __shfl_xor_sync(FULL, bv, o);
-        const int oi = __shfl_xor_sync(FULL, bi, o);
-        anynan |= __shfl_xor_sync(FULL, anynan, o);
-        if (ov > bv || (ov == bv && oi < bi)) { bv = ov; bi = oi; }
-    }
+    warp_best(bv, bi, anynan);
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     if (lane == 0) { sv[warp] = bv; si[warp] = bi; snan[warp] = anynan; }
     __syncthreads();
     if (threadIdx.x == 0) {
         for (int w = 1; w < (int)(blockDim.x >> 5); ++w) {
             anynan |= snan[w];
-            if (sv[w] > bv || (sv[w] == bv && si[w] < bi)) { bv = sv[w]; bi = si[w]; }
+            best_merge(bv, bi, sv[w], si[w]);
         }
         double v; int k; double sg;
-        if (anynan) { v = __longlong_as_double(0x7ff8000000000000LL); k = -2; sg = 0.05; }     // np.max propagates NaN; the reference would raise
-        else if (bv == 0.0) { v = bv; k = -1; sg = 0.05; }                                      // ball_scan.py:279-282
-        else { v = bv; k = bi; sg = __dadd_rn(__dmul_rn(1.3, fabs(bv)), 0.05); }     // (two roundings, like numpy: no FMA contraction)                                    // ball_scan.py:283-295 (first index in row-major order)
+        guarded_max(bv, bi, anynan, v, k, sg);
         if (val) val[s] = v;
         if (idx) idx[s] = k;
         if (sigma0) sigma0[s] = sg;

@@ -99,6 +99,30 @@ __device__ __forceinline__ int warp_sum_i(int v) {
     return v;
 }
 
+// ---- per-surface arg-max with the guards of ball_scan.py:279-295 ------------------------------------------
+// (value, first flat index) maximum with the tie rule of np.where(...)[k][0] (ball_scan.py:284-285): larger value wins, equal
+// values keep the smaller index; NaN is tracked separately (np.max propagates it)
+__device__ __forceinline__ void best_merge(double& bv, int& bi, double ov, int oi) {
+    if (ov > bv || (ov == bv && oi < bi)) { bv = ov; bi = oi; }
+}
+__device__ __forceinline__ void warp_best(double& bv, int& bi, int& anynan) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        const double ov = __shfl_xor_sync(FULL, bv, o);
+        const int oi = __shfl_xor_sync(FULL, bi, o);
+        anynan |= __shfl_xor_sync(FULL, anynan, o);
+        best_merge(bv, bi, ov, oi);
+    }
+}
+// The reduced (bv, bi, anynan) of a surface -> what the reference reports: NaN anywhere gives (NaN, -2) (np.max propagates
+// it; the reference would raise), an all-zero maximum the guard's (0, -1), otherwise (max, first index); sigma0 = 0.05 for
+// both guards, else 1.3 |max| + 0.05 with two roundings, like numpy (no FMA contraction).
+__device__ __forceinline__ void guarded_max(double bv, int bi, int anynan, double& val, int& idx, double& sigma0) {
+    if (anynan) { val = __longlong_as_double(0x7ff8000000000000LL); idx = -2; sigma0 = 0.05; }
+    else if (bv == 0.0) { val = bv; idx = -1; sigma0 = 0.05; }                                      // ball_scan.py:279-282
+    else { val = bv; idx = bi; sigma0 = __dadd_rn(__dmul_rn(1.3, fabs(bv)), 0.05); }                 // ball_scan.py:283-295
+}
+
 // ---- TMA bulk copy global -> shared, completion on an mbarrier -------------------------------------------
 __device__ __forceinline__ void mbar_init(uint64_t* bar, unsigned count) {
     asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"((unsigned)__cvta_generic_to_shared(bar)), "r"(count));

@@ -5,7 +5,7 @@
 //   scan_prep_kernel   one CTA per field line: the six theta0-independent coefficient rows of the line as 48-byte
 //                      records, for the fine grid and up to four coarser ones (every 2nd/4th/8th/16th point), scaled by
 //                      a power of two so that max g ~ 1; bounds of the spectrum valid for the line's whole theta0 range
-//   scan_solve_kernel  persistent warps; a warp takes (line, group of 32*SPL theta0) items from a global counter.
+//   scan_solve_kernel  persistent warps; a warp takes (line, group of 32 theta0) items from a global counter.
 //                      The records are streamed through a per-warp ring of shared-memory tiles with TMA bulk copies
 //                      (cp.async.bulk + mbarrier, a ring of 3 stages: two ahead); every lane reads the SAME record
 //                      (broadcast LDS.128) and advances its own solve.  No shuffles in the passes, no block barriers, no
@@ -33,7 +33,7 @@ constexpr int SC_RING = SC_NSTAGE * SC_STAGE;      // doubles per warp (9 KB wit
 #endif
 constexpr int SC_WARPS = IBS_SCAN_WARPS;           // warps per CTA (they never synchronise with each other)
 #ifndef IBS_SCAN_CTAS1
-#define IBS_SCAN_CTAS1 2      // CTAs per SM the SPL = 1 kernel is compiled for (register cap 65536 / (128 * CTAS))
+#define IBS_SCAN_CTAS1 2      // CTAs per SM scan_solve_kernel is compiled for (register cap 65536 / (128 * CTAS))
 #endif
 
 struct ScanParams {
@@ -48,7 +48,6 @@ struct ScanParams {
     double* lam_out; double* lam_matrix_out; double* X_out; double* dX_out; int* info_out;
     double* warm; unsigned* warm_flag;     // lane-per-chain kernel: [nline * groups][16][WREC] warm-start records handed to the next line, [nline * groups] ready flags (zeroed); null: off
     double* X_rows;           // where the eigenfunctions go: X_out, or scratch when only dX is wanted (null: no eigenfunction output)
-    double* shift_ws; int* info_ws;      // two-kernel form: converged shift and counters handed from the iteration kernel to the output kernel
     unsigned* counter;
     // fused per-surface arg-max (ball_scan.py:279-295); items_per_surface = 0: off
     int items_per_surface, lines_per_surface;
@@ -57,18 +56,25 @@ struct ScanParams {
     double* best_out; double* sigma0_out;  // [nsurf][2] packed (max, flat index as a double), [nsurf] (nullable)
 };
 
-// (value, first flat index) maximum with the tie rule of np.where(...)[k][0] (ball_scan.py:284-285): larger value wins, equal
-// values keep the smaller index; NaN is tracked separately (np.max propagates it)
-__device__ __forceinline__ void best_merge(double& bv, int& bi, double ov, int oi) {
-    if (ov > bv || (ov == bv && oi < bi)) { bv = ov; bi = oi; }
-}
-__device__ __forceinline__ void warp_best(double& bv, int& bi, int& anynan) {
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) {
-        const double ov = __shfl_xor_sync(FULL, bv, o);
-        const int oi = __shfl_xor_sync(FULL, bi, o);
-        anynan |= __shfl_xor_sync(FULL, anynan, o);
-        best_merge(bv, bi, ov, oi);
+// ---- fused arg-max: each item's best (value, index) goes to its slot; the LAST item of a surface to finish (prev = the
+// surface's count of finished items before this one, from lane 0) reduces the slots and writes the guarded result
+__device__ __forceinline__ void surface_argmax_last(const ScanParams& p, int surf, unsigned prev, int lane) {
+    prev = __shfl_sync(FULL, prev, 0);
+    if (prev != (unsigned)p.items_per_surface - 1u) return;
+    __threadfence();
+    double bv = -INFINITY; int bi = 0x7fffffff, anynan = 0;
+    const int i0 = surf * p.items_per_surface;
+    for (int i = lane; i < p.items_per_surface; i += 32) {
+        const double v = __ldcg(p.item_val + i0 + i);
+        const int k = __ldcg(p.item_idx + i0 + i);
+        if (k == -2) anynan = 1; else best_merge(bv, bi, v, k);
+    }
+    warp_best(bv, bi, anynan);
+    if (lane == 0) {
+        double val, sg; int idx;
+        guarded_max(bv, bi, anynan, val, idx, sg);
+        p.best_out[2 * surf] = val; p.best_out[2 * surf + 1] = (double)idx;
+        if (p.sigma0_out) p.sigma0_out[surf] = sg;
     }
 }
 
@@ -136,37 +142,23 @@ struct DevCtx {
     // the fix-up reads rows that OTHER lanes of the warp have written: L2 loads after a warp-level fence
     __device__ __forceinline__ void sync_mem() const { __syncwarp(); }
     __device__ __forceinline__ double ld(const double* p) const { return __ldcg(p); }
-    // zero-fill invalid solves / form dX of the solves flagged wr[]: one solve at a time, its rows dealt out over the 32 lanes
-    template <int SPL>
-    __device__ __forceinline__ void fixup(const bool (&wr)[SPL], double* const (&Xrow)[SPL], double* const (&dXrow)[SPL], int N_,
-                                          const SolveOut (&out)[SPL], double h, bool want_dX) {
+    // zero-fill invalid solves / form dX of the flagged solves: one solve at a time, its rows dealt out over the 32 lanes
+    __device__ __forceinline__ void fixup(bool flag, double* Xrow, double* dXrow, int N_, bool bad, double h, bool want_dX) {
         __syncwarp();
-#pragma unroll
-        for (int q = 0; q < SPL; ++q) {
-            unsigned m = __ballot_sync(FULL, wr[q] && (out[q].bad || want_dX));
-            while (m) {
-                const int l = __ffs(m) - 1;
-                m &= m - 1;
-                const bool bad = __shfl_sync(FULL, (int)out[q].bad, l) != 0;
-                double* X = reinterpret_cast<double*>(__shfl_sync(FULL, reinterpret_cast<unsigned long long>(Xrow[q]), l));
-                double* dX = reinterpret_cast<double*>(__shfl_sync(FULL, reinterpret_cast<unsigned long long>(dXrow[q]), l));
-                fixup_solve(*this, X, want_dX ? dX : nullptr, N_, bad, h, lane, 32);
-            }
+        unsigned m = __ballot_sync(FULL, flag);
+        while (m) {
+            const int l = __ffs(m) - 1;
+            m &= m - 1;
+            const bool bd = __shfl_sync(FULL, (int)bad, l) != 0;
+            double* X = reinterpret_cast<double*>(__shfl_sync(FULL, reinterpret_cast<unsigned long long>(Xrow), l));
+            double* dX = reinterpret_cast<double*>(__shfl_sync(FULL, reinterpret_cast<unsigned long long>(dXrow), l));
+            fixup_solve(*this, X, want_dX ? dX : nullptr, N_, bd, h, lane, 32);
         }
         __syncwarp();
     }
 };
 
-#ifndef IBS_SCAN_CTAS_ITER
-#define IBS_SCAN_CTAS_ITER 3     // CTAs per SM the iteration-only kernel (two-kernel form) is compiled for
-#endif
-template <int SPL, int MODE>
-__global__ void
-#ifdef IBS_SCAN_MAXNREG
-__maxnreg__(IBS_SCAN_MAXNREG)          // tuning builds: explicit register cap (cannot be combined with __launch_bounds__)
-#else
-__launch_bounds__(SC_WARPS * 32, (MODE == MODE_ITER) ? IBS_SCAN_CTAS_ITER : ((SPL == 1) ? IBS_SCAN_CTAS1 : 2))
-#endif
+__global__ void __launch_bounds__(SC_WARPS * 32, IBS_SCAN_CTAS1)
 scan_solve_kernel(const ScanParams p) {
     extern __shared__ __align__(128) double sc_smem[];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -174,8 +166,7 @@ scan_solve_kernel(const ScanParams p) {
     ctx.ring = sc_smem + warp * SC_RING;
     ctx.bars = reinterpret_cast<uint64_t*>(sc_smem + SC_WARPS * SC_RING) + warp * SC_NSTAGE;
     // the thread's block of cold state (odd stride in doubles: conflict-free across the lanes of a warp)
-    ColdState<SPL>& cold = *reinterpret_cast<ColdState<SPL>*>(sc_smem + SC_WARPS * SC_RING + SC_WARPS * SC_NSTAGE +
-                                                            (size_t)threadIdx.x * ColdStride<SPL>::value);
+    ColdState& cold = *reinterpret_cast<ColdState*>(sc_smem + SC_WARPS * SC_RING + SC_WARPS * SC_NSTAGE + (size_t)threadIdx.x * COLD_STRIDE);
     ctx.parity = 0; ctx.lane = lane; ctx.N = p.N;
     if (lane == 0) {
         for (int s = 0; s < SC_NSTAGE; ++s) mbar_init(&ctx.bars[s], 1);
@@ -189,54 +180,32 @@ scan_solve_kernel(const ScanParams p) {
         item = __shfl_sync(FULL, item, 0);
         if (item >= p.nitems) break;
         const int line = item / p.groups, grp = item - line * p.groups;
-        double th0[SPL], sg[SPL];
-        bool act[SPL];
-        double* Xrow[SPL]; double* dXrow[SPL];
-        size_t sidx[SPL];
-#pragma unroll
-        for (int q = 0; q < SPL; ++q) {
-            const int idx = grp * (32 * SPL) + q * 32 + lane;
-            act[q] = idx < p.nth0;
-            sidx[q] = (size_t)line * p.nth0 + (act[q] ? idx : p.nth0 - 1);
-            th0[q] = p.theta0[sidx[q]];
-            sg[q] = p.sigma ? p.sigma[sidx[q]] : 0.0;
-            Xrow[q] = (act[q] && p.X_rows) ? p.X_rows + sidx[q] * N : nullptr;
-            dXrow[q] = (act[q] && p.dX_out) ? p.dX_out + sidx[q] * N : nullptr;
-        }
+        const int idx = grp * 32 + lane;
+        const bool act = idx < p.nth0;
+        const size_t sidx = (size_t)line * p.nth0 + (act ? idx : p.nth0 - 1);
+        const double th0 = p.theta0[sidx];
+        const double sg = p.sigma ? p.sigma[sidx] : 0.0;
+        double* Xrow = (act && p.X_rows) ? p.X_rows + sidx * N : nullptr;
+        double* dXrow = (act && p.dX_out) ? p.dX_out + sidx * N : nullptr;
         ItemProblem P;
         P.N = N; P.nlev = p.nlev; P.h = p.h; P.U = p.bounds[2 * line]; P.Lb = p.bounds[2 * line + 1];
         P.want_X = p.X_rows != nullptr; P.want_dX = p.dX_out != nullptr;
         ctx.line_base = p.poly + (size_t)line * p.rows_total * REC;
-        ItemResult res[SPL];
-        if (MODE == MODE_OUT) {
-#pragma unroll
-            for (int q = 0; q < SPL; ++q) { res[q].rho = p.shift_ws[sidx[q]]; res[q].info = p.info_ws[sidx[q]]; res[q].gam = 0.0; }
+        ItemResult res;
+        solve_item(ctx, P, th0, act, sg, p.sigma != nullptr, Xrow, dXrow, res, cold);
+        if (act) {
+            p.lam_out[sidx] = res.gam;
+            if (p.lam_matrix_out) p.lam_matrix_out[sidx] = res.rho;
+            if (p.info_out) p.info_out[sidx] = res.info;
         }
-        solve_item<SPL, MODE>(ctx, P, th0, act, sg, p.sigma != nullptr, Xrow, dXrow, res, cold);
-#pragma unroll
-        for (int q = 0; q < SPL; ++q)
-            if (act[q]) {
-                if (MODE == MODE_ITER) {           // hand over to the output kernel
-                    p.shift_ws[sidx[q]] = res[q].rho;
-                    p.info_ws[sidx[q]] = res[q].info;
-                } else {
-                    p.lam_out[sidx[q]] = res[q].gam;
-                    if (p.lam_matrix_out) p.lam_matrix_out[sidx[q]] = res[q].rho;
-                    if (p.info_out) p.info_out[sidx[q]] = res[q].info;
-                }
-            }
-        if (MODE != MODE_ITER && p.items_per_surface > 0) {
-            // ---- fused arg-max: the item's best -> its slot; the LAST item of a surface to finish reduces the slots
+        if (p.items_per_surface > 0) {
             const int surf = line / p.lines_per_surface;
             double bv = -INFINITY; int bi = 0x7fffffff, anynan = 0;
-#pragma unroll
-            for (int q = 0; q < SPL; ++q)
-                if (act[q]) {
-                    const double v = res[q].gam;
-                    const int flat = (line - surf * p.lines_per_surface) * p.nth0 + grp * (32 * SPL) + q * 32 + lane;
-                    if (v != v) anynan = 1;
-                    best_merge(bv, bi, v, flat);
-                }
+            if (act) {
+                const double v = res.gam;
+                if (v != v) anynan = 1;
+                best_merge(bv, bi, v, (line - surf * p.lines_per_surface) * p.nth0 + idx);
+            }
             warp_best(bv, bi, anynan);
             unsigned prev = 0;
             if (lane == 0) {
@@ -245,26 +214,7 @@ scan_solve_kernel(const ScanParams p) {
                 __threadfence();
                 prev = atomicAdd(&p.surf_count[surf], 1u);
             }
-            prev = __shfl_sync(FULL, prev, 0);
-            if (prev == (unsigned)p.items_per_surface - 1u) {
-                __threadfence();
-                bv = -INFINITY; bi = 0x7fffffff; anynan = 0;
-                const int i0 = surf * p.items_per_surface;
-                for (int i = lane; i < p.items_per_surface; i += 32) {
-                    const double v = __ldcg(p.item_val + i0 + i);
-                    const int k = __ldcg(p.item_idx + i0 + i);
-                    if (k == -2) anynan = 1; else best_merge(bv, bi, v, k);
-                }
-                warp_best(bv, bi, anynan);
-                if (lane == 0) {
-                    double val, idx, sg;
-                    if (anynan) { val = __longlong_as_double(0x7ff8000000000000LL); idx = -2.0; sg = 0.05; }     // np.max propagates NaN
-                    else if (bv == 0.0) { val = bv; idx = -1.0; sg = 0.05; }                                      // ball_scan.py:279-282
-                    else { val = bv; idx = (double)bi; sg = __dadd_rn(__dmul_rn(1.3, fabs(bv)), 0.05); }     // (two roundings, like numpy: no FMA contraction)                              // ball_scan.py:283-295
-                    p.best_out[2 * surf] = val; p.best_out[2 * surf + 1] = idx;
-                    if (p.sigma0_out) p.sigma0_out[surf] = sg;
-                }
-            }
+            surface_argmax_last(p, surf, prev, lane);
         }
     }
 }
@@ -272,12 +222,6 @@ scan_solve_kernel(const ScanParams p) {
 // ---- lane-per-chain kernel (ibs_scan2_core.cuh): 16 solves per warp, lane = 16 h + i runs chain h of solve i ---------------
 #ifndef IBS_SCAN2_CTAS
 #define IBS_SCAN2_CTAS 4          // CTAs of 4 warps per SM the kernel is compiled for (register cap 65536 / (128 * CTAS))
-#endif
-#ifndef IBS_SCAN2_ROWK_SMEM
-#define IBS_SCAN2_ROWK_SMEM 0       // matching row from the ring instead of L2: measured 2.89 vs 2.81 ms (select + shuffles cost more than the hidden L2 read)
-#endif
-#ifndef IBS_SCAN2_PREFETCH_K
-#define IBS_SCAN2_PREFETCH_K 0      // measured: 3.09 vs 3.03 ms with the prefetch (the L1 line rarely survives until the join)
 #endif
 constexpr int S2_TILE = scan2::T0 * REC;           // doubles per tile (35 records)
 constexpr int S2_STAGE = 2 * S2_TILE;              // ascending tile (forward lanes) + descending tile (backward lanes)
@@ -341,32 +285,7 @@ struct Dev2Ctx {
     }
     __device__ __forceinline__ double xd(double v) const { return __shfl_xor_sync(FULL, v, 16); }
     __device__ __forceinline__ int xi(int v) const { return __shfl_xor_sync(FULL, v, 16); }
-    // the join of a pass reads the record of the matching row from global memory: ask for it when the pass starts, so that the
-    // L2 round trip is over by then (it is ~20 % of the issue time of a pass on the coarsest level)
-    __device__ __forceinline__ void prefetch_k(int lev, int k) const {
-#if IBS_SCAN2_PREFETCH_K
-        const double* q = line_base + ((size_t)level_offset(N, lev) + k) * REC;
-        asm volatile("prefetch.global.L1 [%0];" :: "l"(q));
-        asm volatile("prefetch.global.L1 [%0];" :: "l"(q + REC - 1));       // (a 48-byte record may straddle two 32-byte sectors' lines)
-#endif
-    }
-    // (t_k, F_k) of the matching row for the join of a pass.  Row k is the LAST row both chains process, so its record is still
-    // in the ring -- for the lane whose chain is the longer one (the ring runs on for it; the shorter chain's last stage may
-    // have been overwritten): that lane reads it from shared memory and hands the two numbers to its partner.  (It used to
-    // be an L2 round trip per pass, ~9 per item, exposed at the join.)
-    __device__ __forceinline__ void row_k(int Nl_, int k, double th0, double lam, double& tk, double& Fk) const {
-#if IBS_SCAN2_ROWK_SMEM
-        const int qf = k, qb = Nl_ - 1 - k, qe = h ? qb : qf;
-        const bool mine = h ? (qb > qf) : (qf >= qb);                         // my chain is the longer one (ties: the forward lane)
-        double t = 0.0, F = 0.0;
-        if (mine) scan2::row_tF(load_rec(ptr(scan2::stage_of(qe), qe)), th0, lam, t, F);
-        const double to = xd(t), Fo = xd(F);
-        tk = mine ? t : to; Fk = mine ? F : Fo;
-#else
-        scan2::row_tF(rec_k(k), th0, lam, tk, Fk);
-#endif
-    }
-    __device__ __forceinline__ Rec rec_k(int k) const {        // record of the matching row (global memory; L2)
+    __device__ __forceinline__ Rec rec_k(int k) const {        // record of the matching row for the join of a pass (global memory; L2)
         const double2* q = reinterpret_cast<const double2*>(lvl + (size_t)k * REC);
         const double2 a = __ldg(q), b = __ldg(q + 1), c = __ldg(q + 2);
         Rec r; r.G0 = a.x; r.G1 = a.y; r.G2 = b.x; r.C0 = b.y; r.C1 = c.x; r.R = c.y;
@@ -375,17 +294,15 @@ struct Dev2Ctx {
     // ---- the passes of solve_item2: my chain, the partner's end state by shuffle, the join
     __device__ __forceinline__ void eval(int lev, int Nl_, int k, double th0, double lam, double& r, double& S, int& nodes) {
         const int qf = k, qb = Nl_ - 1 - k;
-        prefetch_k(lev, k);
         const scan2::EvalEnd me = scan2::eval_lane(*this, lev, Nl_, h ? qb : qf, qf > qb ? qf : qb, th0, lam);
         scan2::EvalEnd ot;
         ot.X = xd(me.X); ot.W = xd(me.W); ot.S = xd(me.S); ot.nodes = xi(me.nodes);
         double tk, Fk;
-        row_k(Nl_, k, th0, lam, tk, Fk);
+        scan2::row_tF(rec_k(k), th0, lam, tk, Fk);
         scan2::eval_join(h ? ot : me, h ? me : ot, tk, Fk, th0, lam, r, S, nodes);
     }
     __device__ __forceinline__ void out1(int lev, int Nl_, int k, double th0, double lam, SolveOut& out, bool check) {
         const int qf = k, qb = Nl_ - 1 - k;
-        prefetch_k(lev, k);
         // (check is warp-uniform: a property of the line)
         const Sweep me = check ? scan2::out_lane<false, true>(*this, lev, Nl_, h ? qb : qf, qf > qb ? qf : qb, h != 0, th0, lam, 0.0, 0, nullptr)
                                : scan2::out_lane<false, false>(*this, lev, Nl_, h ? qb : qf, qf > qb ? qf : qb, h != 0, th0, lam, 0.0, 0, nullptr);
@@ -394,7 +311,7 @@ struct Dev2Ctx {
         ot.a0e = xd(me.a0e); ot.a0o = xd(me.a0o); ot.a1e = xd(me.a1e); ot.a1o = xd(me.a1o); ot.aDe = xd(me.aDe); ot.aDo = xd(me.aDo);
         ot.aEnd = xd(me.aEnd); ot.vmax = xd(me.vmax); ot.jmax = xi(me.jmax); ot.bad = xi((int)me.bad) != 0;
         double tk, Fk;
-        row_k(Nl_, k, th0, lam, tk, Fk);
+        scan2::row_tF(rec_k(k), th0, lam, tk, Fk);
         scan2::out_join(h ? ot : me, h ? me : ot, tk, Fk, th0, lam, k, out);
     }
     __device__ __forceinline__ void out2(int lev, int Nl_, int k, double th0, double lam, const SolveOut& out, double* Xw) {
@@ -438,8 +355,8 @@ scan2_solve_kernel(const ScanParams p) {
     ctx.ring = sc_smem + warp * S2_RING;
     ctx.bars = reinterpret_cast<uint64_t*>(sc_smem + SC_WARPS * S2_RING) + warp * SC_NSTAGE;
     // one block of cold state per PAIR of lanes (both run the same bookkeeping and store the same values)
-    ColdState<1>& cold = *reinterpret_cast<ColdState<1>*>(sc_smem + SC_WARPS * S2_RING + SC_WARPS * SC_NSTAGE +
-                                                          (size_t)(warp * scan2::NH + li) * ColdStride<1>::value);
+    ColdState& cold = *reinterpret_cast<ColdState*>(sc_smem + SC_WARPS * S2_RING + SC_WARPS * SC_NSTAGE +
+                                                    (size_t)(warp * scan2::NH + li) * COLD_STRIDE);
     ctx.parity = 0; ctx.lane = lane; ctx.h = h; ctx.N = p.N; ctx.warm = p.warm;
     if (lane == 0) {
         for (int s = 0; s < SC_NSTAGE; ++s) mbar_init(&ctx.bars[s], 1);
@@ -502,8 +419,8 @@ scan2_solve_kernel(const ScanParams p) {
             if (p.lam_matrix_out) p.lam_matrix_out[sidx] = res.rho;
             if (p.info_out) p.info_out[sidx] = res.info;
         }
-        // ---- publication of this item: its warm-start record (written inside solve_item2) and, for the fused arg-max (see
-        // scan_solve_kernel; the forward lanes carry the solves), its best (value, index) -- ONE fence for both (a fence
+        // ---- publication of this item: its warm-start record (written inside solve_item2) and, for the fused arg-max (the
+        // forward lanes carry the solves), its best (value, index) -- ONE fence for both (a fence
         // waits for the warp's outstanding stores, here the whole X output of the writing pass: ~2 % of the kernel each)
         const bool fused = p.items_per_surface > 0;
         const int surf = line / p.lines_per_surface;
@@ -530,26 +447,7 @@ scan2_solve_kernel(const ScanParams p) {
                 if (w_out >= 0) *reinterpret_cast<volatile unsigned*>(p.warm_flag + slot) = 1u;
                 prev = atomicAdd(&p.surf_count[surf], 1u);
             }
-            prev = __shfl_sync(FULL, prev, 0);
-            if (prev == (unsigned)p.items_per_surface - 1u) {
-                __threadfence();
-                bv = -INFINITY; bi = 0x7fffffff; anynan = 0;
-                const int i0 = surf * p.items_per_surface;
-                for (int i = lane; i < p.items_per_surface; i += 32) {
-                    const double v = __ldcg(p.item_val + i0 + i);
-                    const int k = __ldcg(p.item_idx + i0 + i);
-                    if (k == -2) anynan = 1; else best_merge(bv, bi, v, k);
-                }
-                warp_best(bv, bi, anynan);
-                if (lane == 0) {
-                    double val, idxd, sgm;
-                    if (anynan) { val = __longlong_as_double(0x7ff8000000000000LL); idxd = -2.0; sgm = 0.05; }
-                    else if (bv == 0.0) { val = bv; idxd = -1.0; sgm = 0.05; }
-                    else { val = bv; idxd = (double)bi; sgm = __dadd_rn(__dmul_rn(1.3, fabs(bv)), 0.05); }
-                    p.best_out[2 * surf] = val; p.best_out[2 * surf + 1] = idxd;
-                    if (p.sigma0_out) p.sigma0_out[surf] = sgm;
-                }
-            }
+            surface_argmax_last(p, surf, prev, lane);
         } else if (w_out >= 0 && lane == 0) {
             *reinterpret_cast<volatile unsigned*>(p.warm_flag + slot) = 1u;
         }
@@ -655,51 +553,25 @@ bool scan_solver_eligible(const SolveParams& p) {
     return true;
 }
 
-template <int SPL, int MODE>
-static int scan_launch(const ScanParams& sp, cudaStream_t stream) {
-    auto kern = scan_solve_kernel<SPL, MODE>;
-    const size_t smem = (size_t)SC_WARPS * SC_RING * sizeof(double) + (size_t)SC_WARPS * SC_NSTAGE * sizeof(uint64_t) +
-                        (size_t)SC_WARPS * 32 * ColdStride<SPL>::value * sizeof(double);
-    static bool configured[IBS_MAX_DEVICES] = {false};     // per instantiation and per device (the attribute is per device)
+// Launch of a lane kernel: persistent CTAs of SC_WARPS warps, as many as fit (IBS_MAX_CTAS_PER_SM caps the CTAs per SM) and
+// no more than there are items for.  smem: the warps' record rings, their barriers and one cold-state block per solve.
+template <void (*KERN)(ScanParams)>
+static int lane_launch(const ScanParams& sp, size_t smem, cudaStream_t stream) {
+    static bool configured[IBS_MAX_DEVICES] = {false};     // per kernel and per device (the attribute is per device)
     const int dslot = current_device_slot();
     if (!configured[dslot]) {
-        IBS_CUDA_CHECK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        IBS_CUDA_CHECK(cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+        IBS_CUDA_CHECK(cudaFuncSetAttribute(KERN, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        IBS_CUDA_CHECK(cudaFuncSetAttribute(KERN, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
         configured[dslot] = true;
     }
     int per_sm = 0;
-    IBS_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, SC_WARPS * 32, smem));
+    IBS_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, KERN, SC_WARPS * 32, smem));
     if (per_sm < 1) per_sm = 1;
     if (const char* e = std::getenv("IBS_MAX_CTAS_PER_SM")) { const int v = std::atoi(e); if (v >= 1 && v < per_sm) per_sm = v; }
     const long long cap = (long long)num_sms() * per_sm;
     const long long need = ((long long)sp.nitems + SC_WARPS - 1) / SC_WARPS;
     const int grid = (int)(need < cap ? need : cap);
-    kern<<<grid, SC_WARPS * 32, smem, stream>>>(sp);
-    IBS_CUDA_CHECK(cudaGetLastError());
-    return IBS_OK;
-}
-
-static size_t scan2_smem_bytes() {
-    return (size_t)SC_WARPS * S2_RING * sizeof(double) + (size_t)SC_WARPS * SC_NSTAGE * sizeof(uint64_t) +
-           (size_t)SC_WARPS * scan2::NH * ColdStride<1>::value * sizeof(double);
-}
-static int scan2_launch(const ScanParams& sp, cudaStream_t stream) {
-    const size_t smem = scan2_smem_bytes();
-    static bool configured[IBS_MAX_DEVICES] = {false};
-    const int dslot = current_device_slot();
-    if (!configured[dslot]) {
-        IBS_CUDA_CHECK(cudaFuncSetAttribute(scan2_solve_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        IBS_CUDA_CHECK(cudaFuncSetAttribute(scan2_solve_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-        configured[dslot] = true;
-    }
-    int per_sm = 0;
-    IBS_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, scan2_solve_kernel, SC_WARPS * 32, smem));
-    if (per_sm < 1) per_sm = 1;
-    if (const char* e = std::getenv("IBS_MAX_CTAS_PER_SM")) { const int v = std::atoi(e); if (v >= 1 && v < per_sm) per_sm = v; }
-    const long long cap = (long long)num_sms() * per_sm;
-    const long long need = ((long long)sp.nitems + SC_WARPS - 1) / SC_WARPS;
-    const int grid = (int)(need < cap ? need : cap);
-    scan2_solve_kernel<<<grid, SC_WARPS * 32, smem, stream>>>(sp);
+    KERN<<<grid, SC_WARPS * 32, smem, stream>>>(sp);
     IBS_CUDA_CHECK(cudaGetLastError());
     return IBS_OK;
 }
@@ -710,13 +582,13 @@ static bool use_scan2(int N) {
 }
 
 // One launch set (prep + solver) for the lines [l0, l0 + nline) of the batch p
-static int scan_solve_lines(const SolveParams& p, int l0, int nline, int spl, bool two, cudaStream_t stream) {
+static int scan_solve_lines(const SolveParams& p, int l0, int nline, cudaStream_t stream) {
     const int N = p.N;
     const int nlev = num_levels(N);
     const int rows_total = level_offset(N, nlev + 1);
     const size_t v0 = (size_t)l0 * p.nth0, nsolve = (size_t)nline * p.nth0;
-    const bool s2 = !two && spl == 1 && use_scan2(N);
-    const int groups = s2 ? (p.nth0 + scan2::NH - 1) / scan2::NH : (p.nth0 + 32 * spl - 1) / (32 * spl);
+    const bool s2 = use_scan2(N);
+    const int groups = s2 ? (p.nth0 + scan2::NH - 1) / scan2::NH : (p.nth0 + 31) / 32;
     const int nitems = nline * groups;
     const bool fused = p.lines_per_surface > 0 && p.best_out;
     const int nsurf = fused ? nline / p.lines_per_surface : 0;
@@ -744,10 +616,9 @@ static int scan_solve_lines(const SolveParams& p, int l0, int nline, int spl, bo
         else rounds = 1;
         if (rounds < 2) warm = false;
     }
-    const size_t nzero = 2 + (size_t)nsurf + (warm ? (size_t)nitems : 0);
-    const size_t o_zero = take(nzero * sizeof(unsigned));             // work counters + per-surface counters + warm-start flags: zeroed together
+    const size_t nzero = 1 + (size_t)nsurf + (warm ? (size_t)nitems : 0);
+    const size_t o_zero = take(nzero * sizeof(unsigned));             // work counter + per-surface counters + warm-start flags: zeroed together
     const size_t o_warm = take(warm ? (size_t)nitems * scan2::NH * scan2::WREC * sizeof(double) : 0);
-    const size_t o_hand = take(two ? nsolve * (sizeof(double) + sizeof(int)) : 0);
     const size_t o_ival = take(fused ? (size_t)nitems * sizeof(double) : 0);
     const size_t o_iidx = take(fused ? (size_t)nitems * sizeof(int) : 0);
     const size_t xs_bytes = (p.dX_out && !p.X_out) ? nsolve * N * sizeof(double) : 0;      // X is the scratch dX is formed from
@@ -769,14 +640,12 @@ static int scan_solve_lines(const SolveParams& p, int l0, int nline, int spl, bo
     sp.dX_out = p.dX_out ? p.dX_out + v0 * N : nullptr;
     sp.info_out = p.info_out ? p.info_out + v0 : nullptr;
     sp.X_rows = sp.X_out ? sp.X_out : (xs_bytes ? (double*)(ws + o_xs) : nullptr);
-    sp.shift_ws = two ? (double*)(ws + o_hand) : nullptr;
-    sp.info_ws = two ? (int*)(ws + o_hand + nsolve * sizeof(double)) : nullptr;
     sp.items_per_surface = fused ? p.lines_per_surface * groups : 0;
     sp.lines_per_surface = fused ? p.lines_per_surface : 1;
     sp.item_val = (double*)(ws + o_ival); sp.item_idx = (int*)(ws + o_iidx);
-    sp.surf_count = sp.counter + 2;
+    sp.surf_count = sp.counter + 1;
     sp.warm = warm ? (double*)(ws + o_warm) : nullptr;
-    sp.warm_flag = warm ? sp.counter + 2 + nsurf : nullptr;
+    sp.warm_flag = warm ? sp.counter + 1 + nsurf : nullptr;
     const size_t surf0 = fused ? (size_t)l0 / p.lines_per_surface : 0;
     sp.best_out = fused ? p.best_out + 2 * surf0 : nullptr;
     sp.sigma0_out = (fused && p.sigma0_out) ? p.sigma0_out + surf0 : nullptr;
@@ -787,15 +656,14 @@ static int scan_solve_lines(const SolveParams& p, int l0, int nline, int spl, bo
                                                        rows_total, (double*)(ws + o_poly), (double*)(ws + o_bounds), (int*)(ws + o_safe));
         if (cudaError_t e = cudaGetLastError(); e != cudaSuccess) rc = cuda_fail(e, "scan_prep_kernel launch");
     }
-    if (rc == IBS_OK && s2) {
-        rc = scan2_launch(sp, stream);
-    } else if (rc == IBS_OK) {
-        if (two && spl == 1) {
-            rc = scan_launch<1, MODE_ITER>(sp, stream);
-            if (rc == IBS_OK) { ScanParams sp2 = sp; sp2.counter = sp.counter + 1; rc = scan_launch<1, MODE_OUT>(sp2, stream); }
-        } else {
-            rc = (spl == 2) ? scan_launch<2, MODE_FULL>(sp, stream) : scan_launch<1, MODE_FULL>(sp, stream);
-        }
+    if (rc == IBS_OK) {
+        const size_t ring_bars = (size_t)SC_WARPS * SC_NSTAGE * sizeof(uint64_t);
+        if (s2)        // one cold-state block per pair of lanes
+            rc = lane_launch<scan2_solve_kernel>(sp, (size_t)SC_WARPS * S2_RING * sizeof(double) + ring_bars +
+                                                         (size_t)SC_WARPS * scan2::NH * COLD_STRIDE * sizeof(double), stream);
+        else
+            rc = lane_launch<scan_solve_kernel>(sp, (size_t)SC_WARPS * SC_RING * sizeof(double) + ring_bars +
+                                                        (size_t)SC_WARPS * 32 * COLD_STRIDE * sizeof(double), stream);
     }
     cudaFreeAsync(ws, stream);
     return rc;
@@ -803,11 +671,6 @@ static int scan_solve_lines(const SolveParams& p, int l0, int nline, int spl, bo
 
 int scan_solve_dispatch(const SolveParams& p, cudaStream_t stream) {
     const int nline = p.nsolve / p.nth0;
-    int spl = 1;        // two solves per lane (IBS_SCAN_SPL=2) halve the shared-memory traffic but spill at 255 registers: slower
-    if (const char* e = std::getenv("IBS_SCAN_SPL")) { const int v = std::atoi(e); if (v == 1 || v == 2) spl = v; }
-    // two-kernel form (IBS_SCAN_TWO=1): iteration kernel (fewer registers, more resident warps) + output kernel
-    bool two = false;
-    if (const char* e = std::getenv("IBS_SCAN_TWO")) two = std::atoi(e) != 0;
     keep_pool_cached();
     // The coefficient records take ~95 KB per field line (N = 1025): very large batches are processed in chunks of lines so
     // that the stream-ordered workspace stays below IBS_SCAN_WS_MB (default 8 GB; the chunks are still >> one round of warps).
@@ -823,7 +686,7 @@ int scan_solve_dispatch(const SolveParams& p, cudaStream_t stream) {
     }
     int rc = IBS_OK;
     for (long long l0 = 0; l0 < nline && rc == IBS_OK; l0 += chunk)
-        rc = scan_solve_lines(p, (int)l0, (int)((nline - l0 < chunk) ? (nline - l0) : chunk), spl, two, stream);
+        rc = scan_solve_lines(p, (int)l0, (int)((nline - l0 < chunk) ? (nline - l0) : chunk), stream);
     return rc;
 }
 

@@ -1,5 +1,6 @@
-"""GPU parity of the lane-per-solve scan kernel (ibs_scan_solver.cu) -- through the C ABI -- against the oracle,
-the stored converged-reference values and the team-per-solve kernel (IBS_SCAN=0)."""
+"""GPU parity of the lane kernels of the scan solver (ibs_scan_solver.cu: scan2_solve_kernel, and scan_solve_kernel with
+IBS_SCAN2=0 or for grids scan2 cannot take) -- through the C ABI -- against the oracle, the stored converged-reference
+values and the team-per-solve kernel (IBS_SCAN=0)."""
 import os
 
 import numpy as np
@@ -10,13 +11,11 @@ from helpers import LAM_RTOL, X_ATOL, fixture_base, s_alpha_base, sign_normalise
 pytestmark = pytest.mark.gpu
 
 
-def _solve(base, dP, th0, h, nth0, scan, spl=None, two=False, **kw):
+def _solve(base, dP, th0, h, nth0, scan, scan2=True, **kw):
     from ideal_ballooning_solver_b200 import engine
-    old = {k: os.environ.get(k) for k in ("IBS_SCAN", "IBS_SCAN_SPL", "IBS_SCAN_TWO")}
+    old = {k: os.environ.get(k) for k in ("IBS_SCAN", "IBS_SCAN2")}
     os.environ["IBS_SCAN"] = "1" if scan else "0"
-    os.environ["IBS_SCAN_TWO"] = "1" if two else "0"
-    if spl:
-        os.environ["IBS_SCAN_SPL"] = str(spl)
+    os.environ["IBS_SCAN2"] = "1" if scan2 else "0"
     try:
         return engine.solve_base_batch(base, dP, th0, h, nth0=nth0, **kw)
     finally:
@@ -28,8 +27,9 @@ def _solve(base, dP, th0, h, nth0, scan, spl=None, two=False, **kw):
 
 
 @pytest.mark.parametrize("name", ["synthetic_d3d", "synthetic_ncsx", "synthetic_hberg", "ncsx_wout_op"])
-@pytest.mark.parametrize("nth0,spl", [(5, 1), (37, 1), (70, 2), (64, 2)])
-def test_scan_kernel_matches_team_kernel_and_oracle(cuda_lib, golden, name, nth0, spl):
+@pytest.mark.parametrize("nth0", [5, 37, 70, 64])
+@pytest.mark.parametrize("scan2", [True, False], ids=["scan2", "scan"])
+def test_scan_kernel_matches_team_kernel_and_oracle(cuda_lib, golden, name, nth0, scan2):
     import torch
     from ideal_ballooning_solver_b200 import engine
     from oracle import ballooning_oracle as bo
@@ -45,7 +45,7 @@ def test_scan_kernel_matches_team_kernel_and_oracle(cuda_lib, golden, name, nth0
     t0 = np.linspace(0.0, np.pi / 2, nth0)
     th0 = torch.from_numpy(np.tile(t0, ns * na)).cuda()
     sigma = torch.full((th0.numel(),), 1.0, dtype=torch.float64)
-    new = _solve(base, dP, th0, h, nth0, True, spl, sigma=sigma)
+    new = _solve(base, dP, th0, h, nth0, True, scan2, sigma=sigma)
     old = _solve(base, dP, th0, h, nth0, False, sigma=sigma)
     assert np.all(new.flags.cpu().numpy() == old.flags.cpu().numpy())
     lam_n, lam_o = new.lam.cpu().numpy(), old.lam.cpu().numpy()
@@ -158,27 +158,6 @@ def test_scan_kernel_ineligible_batches_use_team_kernel(cuda_lib, golden):
     assert torch.equal(a.lam, b.lam) and torch.equal(a.X, b.X)
 
 
-@pytest.mark.parametrize("name", ["synthetic_d3d", "synthetic_ncsx"])
-def test_scan_kernel_two_kernel_form(cuda_lib, golden, name):
-    """IBS_SCAN_TWO=1: iteration kernel (fewer registers) + output kernel, the converged shift handed over in memory."""
-    import torch
-    from ideal_ballooning_solver_b200 import engine
-    D = golden(name)
-    theta = D["theta"]
-    h = engine.grid_spacing(theta)
-    fb = fixture_base(D)
-    ns, na = fb.shape[:2]
-    base, dP = torch.from_numpy(fb).cuda(), torch.from_numpy(D["dPdrho"]).cuda()
-    th0 = torch.from_numpy(np.tile(np.linspace(0.0, np.pi / 2, 37), ns * na)).cuda()
-    sigma = torch.full((th0.numel(),), 1.0, dtype=torch.float64)
-    one = _solve(base, dP, th0, h, 37, True, sigma=sigma)
-    two = _solve(base, dP, th0, h, 37, True, two=True, sigma=sigma)
-    assert np.all(two.flags.cpu().numpy() == one.flags.cpu().numpy())
-    np.testing.assert_allclose(two.lam.cpu().numpy(), one.lam.cpu().numpy(), rtol=LAM_RTOL, atol=0)
-    np.testing.assert_allclose(two.X.cpu().numpy(), one.X.cpu().numpy(), rtol=0, atol=X_ATOL)
-    np.testing.assert_allclose(two.dX.cpu().numpy(), one.dX.cpu().numpy(), rtol=0, atol=10 * X_ATOL * max(1.0, float(one.dX.abs().max())))
-
-
 @pytest.mark.parametrize("n", [65, 129, 257, 969])
 def test_scan_kernel_small_and_odd_grids(cuda_lib, n):
     """Grids with 0, 1, 2 coarse levels and one whose coarse levels have an even number of points (969 = 8 * 121 + 1)."""
@@ -261,3 +240,47 @@ def test_lane_per_chain_warm_start_is_deterministic_and_changes_nothing(cuda_lib
     assert float(((best_a[:, 0] - best_c[:, 0]).abs() / best_c[:, 0].abs().clamp_min(1e-6)).max().item()) < 1e-10
     it_w = float((a.info & 0xFFFF).double().mean().item()); it_c = float((c.info & 0xFFFF).double().mean().item())
     assert it_w < 0.95 * it_c, (it_w, it_c)           # (2560 lines = two rounds: half of them warm)
+
+
+@pytest.mark.parametrize("scan2", ["1", "0"], ids=["scan2", "scan"])
+def test_fused_argmax_guards_nan_and_tie(cuda_lib, monkeypatch, scan2):
+    """The guarded per-surface arg-max fused into the lane kernels (ball_scan.py:279-295), on three surfaces of four s-alpha
+    lines x 12 theta0 (N = 1025): a normal one; one with a NaN in one line's gds2, which gives (NaN, -2) and sigma0 = 0.05;
+    one whose theta0 row repeats the theta0 of its maximum, so that two lanes of one item tie exactly and the first index
+    wins.  Bit for bit against the stand-alone arg-max kernel on the returned lambda grid and against the oracle's rule."""
+    import torch
+    from ideal_ballooning_solver_b200 import engine
+    from oracle import ballooning_oracle as bo
+    monkeypatch.setenv("IBS_SCAN", "1")
+    monkeypatch.setenv("IBS_SCAN2", scan2)
+    theta = np.linspace(-4 * np.pi, 4 * np.pi, 1025)
+    h = engine.grid_spacing(theta)
+    nsurf, lps, nth0 = 3, 4, 12
+    cases = [(0.6 + 0.1 * q + 0.05 * l, 0.5 + 0.15 * l) for q in range(nsurf) for l in range(lps)]      # (shat, alpha) per line
+    bases, dPs = zip(*[s_alpha_base(s, a, theta) for s, a in cases])
+    base, dP = np.array(bases), np.array(dPs)
+    base[lps + 1, 4, 300] = np.nan                                       # surface 1: a NaN in one line's gds2
+    t0 = np.tile(np.linspace(0.0, 1.5, nth0), (nsurf * lps, 1))
+
+    def run(t0):
+        sol, best, sig = engine.scan_solve_argmax(torch.from_numpy(base).cuda(), torch.from_numpy(dP).cuda(),
+                                                  torch.from_numpy(t0.ravel().copy()).cuda(), h, nth0, lps)
+        val_r, idx_r, sig_r = engine.scan_argmax(sol.lam.reshape(nsurf, lps * nth0))
+        lam, best, sig = sol.lam.cpu().numpy().reshape(nsurf, lps, nth0), best.cpu().numpy(), sig.cpu().numpy()
+        assert np.array_equal(best[:, 0], val_r.cpu().numpy(), equal_nan=True)
+        assert np.array_equal(best[:, 1], idx_r.cpu().numpy().astype(np.float64))
+        assert np.array_equal(sig, sig_r.cpu().numpy())
+        assert np.isnan(lam[1, 1]).all() and np.isnan(best[1, 0]) and best[1, 1] == -2.0 and sig[1] == 0.05
+        for q in (0, 2):
+            assert np.isfinite(lam[q]).all()
+            ia, it, s0 = bo.argmax_with_guards(lam[q])
+            assert best[q, 1] == ia * nth0 + it and best[q, 0] == lam[q, ia, it] and sig[q] == s0
+        return lam, best
+
+    lam, best = run(t0)
+    la, it = divmod(int(best[2, 1]), nth0)
+    j = it - 1 if it > 0 else it + 1                                     # another lane of the same item (nth0 <= 16)
+    t0[2 * lps + la, j] = t0[2 * lps + la, it]
+    lam, best = run(t0)
+    assert lam[2, la, j] == lam[2, la, it] and np.count_nonzero(lam[2] == lam[2].max()) == 2
+    assert best[2, 1] == la * nth0 + min(j, it)

@@ -108,7 +108,7 @@ extern "C" long scan2_host_solve(const double* poly, const double* bounds, const
             P.want_X = X_out != nullptr; P.want_dX = dX_out != nullptr;
             std::vector<double> xscratch(N);
             ItemResult res;
-            ColdState<1> cold;
+            ColdState cold;
             solve_item2(ctx, P, theta0[s], true, sigma ? sigma[s] : 0.0, sigma != nullptr, X_out ? X_out + s * N : xscratch.data(),
                         dX_out ? dX_out + s * N : nullptr, res, cold, w_in, w_out);
             lam_out[s] = res.gam;

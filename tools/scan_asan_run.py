@@ -17,10 +17,8 @@ for n in (65, 129, 257, 969, 1025, 2049):
     for th0max in (1.0, 15.0):
         th0 = np.linspace(0.0, th0max, 5)
         base, dP = s_alpha_base(0.8, 0.9, theta)
-        for two in (0, 1):
-            lib.scan_host_set_two_kernel(two)
-            R = shc.host_scan_solve(lib, base[None], np.array([dP]), th0[None], theta[1] - theta[0], sigma=np.full(5, 1.0))
-            assert np.all(np.isfinite(R["lam"])), (n, th0max, two)
+        R = shc.host_scan_solve(lib, base[None], np.array([dP]), th0[None], theta[1] - theta[0], sigma=np.full(5, 1.0))
+        assert np.all(np.isfinite(R["lam"])), (n, th0max)
         if lib.scan2_host_size_ok(n):          # the lane-per-chain code: several lines, so that the warm-start records are read and written
             th0w = np.linspace(0.0, th0max, 20)
             bases = np.stack([s_alpha_base(0.8 + 0.01 * q, 0.9, theta)[0] for q in range(3)])

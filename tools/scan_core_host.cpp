@@ -1,4 +1,4 @@
-// CPU harness for the lane code of the scan solver (csrc/ibs_scan_core.cuh): runs solve_item<1> for one lane at a
+// CPU harness for the lane code of the scan solver (csrc/ibs_scan_core.cuh): runs solve_item for one lane at a
 // time with records read straight from memory.  TEST INFRASTRUCTURE ONLY (tests/test_scan_core_host.py): it checks
 // the per-lane arithmetic, indices and iteration logic without a GPU; it is not part of the library and nothing in
 // the product path calls it.
@@ -11,8 +11,6 @@
 
 using namespace ibs::scan;
 static double g_cost = 0.0;
-static bool two_kernel = false;
-extern "C" void scan_host_set_two_kernel(int v) { two_kernel = v != 0; }
 
 namespace {
 struct HostCtx {
@@ -34,11 +32,8 @@ struct HostCtx {
     double* scratch() { return scr.data(); }
     double ld(const double* p) const { return *p; }
     int ldi(const int* p) const { return *p; }
-    template <int SPL>
-    void fixup(const bool (&wr)[SPL], double* const (&Xrow)[SPL], double* const (&dXrow)[SPL], int N_, const SolveOut (&out)[SPL],
-               double h, bool want_dX) {
-        for (int q = 0; q < SPL; ++q)
-            if (wr[q]) fixup_solve(*this, Xrow[q], want_dX ? dXrow[q] : nullptr, N_, out[q].bad, h, 0, 1);
+    void fixup(bool flag, double* X, double* dX, int N_, bool bad, double h, bool want_dX) {
+        if (flag) fixup_solve(*this, X, want_dX ? dX : nullptr, N_, bad, h, 0, 1);
     }
 };
 }  // namespace
@@ -104,23 +99,14 @@ extern "C" long scan_host_solve(const double* poly, const double* bounds, const 
             ItemProblem P;
             P.N = N; P.nlev = nlev; P.h = h; P.U = bounds[2 * line]; P.Lb = bounds[2 * line + 1];
             P.want_X = X_out != nullptr; P.want_dX = dX_out != nullptr;
-            const double th0[1] = {theta0[s]};
-            const bool act[1] = {true};
-            const double sg[1] = {sigma ? sigma[s] : 0.0};
             std::vector<double> xscratch(N);
-            double* const Xrow[1] = {X_out ? X_out + s * N : xscratch.data()};
-            double* const dXrow[1] = {dX_out ? dX_out + s * N : nullptr};
-            ItemResult res[1];
-            ColdState<1> cold;
-            if (two_kernel) {       // the two-kernel form: iterate, then the output passes from the handed-over shift
-                solve_item<1, MODE_ITER>(ctx, P, th0, act, sg, false, Xrow, dXrow, res, cold);
-                solve_item<1, MODE_OUT>(ctx, P, th0, act, sg, sigma != nullptr, Xrow, dXrow, res, cold);
-            } else {
-                solve_item<1, MODE_FULL>(ctx, P, th0, act, sg, sigma != nullptr, Xrow, dXrow, res, cold);
-            }
-            lam_out[s] = res[0].gam;
-            if (lam_matrix_out) lam_matrix_out[s] = res[0].rho;
-            if (info_out) info_out[s] = res[0].info;
+            ItemResult res;
+            ColdState cold;
+            solve_item(ctx, P, theta0[s], true, sigma ? sigma[s] : 0.0, sigma != nullptr, X_out ? X_out + s * N : xscratch.data(),
+                       dX_out ? dX_out + s * N : nullptr, res, cold);
+            lam_out[s] = res.gam;
+            if (lam_matrix_out) lam_matrix_out[s] = res.rho;
+            if (info_out) info_out[s] = res.info;
             passes += ctx.evals; cost += ctx.cost;
         }
     g_cost = cost;

@@ -38,8 +38,6 @@ def build(outdir="/tmp/sch"):
     lib.scan2_host_solve.restype = ctypes.c_long
     lib.scan2_host_solve.argtypes = lib.scan_host_solve.argtypes
     lib.scan2_host_size_ok.restype = ctypes.c_int
-    if os.environ.get("IBS_SCAN_TWO"):
-        lib.scan_host_set_two_kernel(int(os.environ["IBS_SCAN_TWO"]))
     return lib
 
 
