@@ -24,6 +24,8 @@ SIGNATURES = {
     "ibs_fp64_probe": (c_int, [c_int, _D, ctypes.c_longlong, POINTER(c_double), c_void_p]),
     "ibs_geometry_batch": (c_int, [_D, _D, _D, _D, _D, _D, _D, c_int, c_int, c_int, c_double, c_double,
                                    _D, c_int, c_int, _D, c_int, c_double, _D, _D, _D, _I, c_void_p]),
+    "ibs_geometry_tangent_batch": (c_int, [_D, _D, _D, _D, _D, _D, _D, c_int, c_int, c_int, c_double, c_double,
+                                           _D, c_int, c_int, _D, c_int, c_double, _D, _D, _D, _D, _D, _I, c_void_p]),
     "ibs_geometry_full_nfields": (c_int, []),
     "ibs_geometry_full": (c_int, [_D, _D, _D, _D, _D, _D, _D, _D, c_int, c_int, c_int, c_double, c_double, _D, c_int, _D, c_int,
                                   c_int, c_double, c_int, c_double, _D, _I, c_void_p]),
@@ -37,6 +39,7 @@ SIGNATURES = {
     "ibs_adjoint_batch": (c_int, [_D, _D, _D, _D, _D, _D, _D, c_int, c_int, c_int, _D, c_void_p]),
     "ibs_adjoint_sensitivities": (c_int, [_D, _D, _D, _D, c_int, c_int, _D, _D, _D, c_void_p]),
     "ibs_obj_w_grad_batch": (c_int, [_D, _D, _D, c_int, c_int, c_double, c_double, _D, _D, _D, _D, _D, _I, c_void_p]),
+    "ibs_obj_w_grad_tangent_batch": (c_int, [_D, _D, _D, _D, _D, c_int, c_int, c_double, _D, _D, _D, _D, _D, _I, c_void_p]),
     "ibs_scan_argmax": (c_int, [_D, c_int, c_int, _D, _I, _D, c_void_p]),
     "ibs_refine_state_doubles": (c_int, []),
     "ibs_refine_init": (c_int, [_D, c_int, _D, _D, c_double, c_double, c_double, c_double, c_double, _D, _D, c_void_p]),

@@ -141,9 +141,75 @@ obj_grad_kernel(const double* __restrict__ base3, const double* __restrict__ dPd
     }
 }
 
+// obj_grad_kernel with the exact alpha-derivative: one line per point and its alpha-tangent (dbase, ddPdrho from
+// ibs_geometry_tangent_batch) instead of three lines.  (g, c, f)_alpha are the chain rule through LineCoef::gcf; Y1, the
+// theta0 part, the thread layout and the summation order are obj_grad_kernel's, so val and grad[:, 1] are the same bits.
+__global__ void __launch_bounds__(RED_THREADS)
+obj_grad_tangent_kernel(const double* __restrict__ base, const double* __restrict__ dbase, const double* __restrict__ dPdrho,
+                        const double* __restrict__ ddPdrho, const double* __restrict__ theta0, const double* __restrict__ lam,
+                        const double* __restrict__ X, const double* __restrict__ dX, int N, double* __restrict__ val_out,
+                        double* __restrict__ grad_out) {
+    __shared__ double sm[7 * (RED_THREADS / 32)];
+    const int p = blockIdx.x;
+    const size_t row = (size_t)p * N;
+    LineCoef L;
+    L.b = base + (size_t)p * IBS_NBASE * N;
+    L.N = N;
+    L.dP = dPdrho[p];
+    const double* db = dbase + (size_t)p * IBS_NBASE * N;
+    const double ddP = ddPdrho[p];
+    const double th0 = theta0[p], two_th0 = __dmul_rn(2.0, th0), th0sq = __dmul_rn(th0, th0);
+    double v[7] = {0, 0, 0, 0, 0, 0, 0};   // Y1, (c,g,f)_theta0, (c,g,f)_alpha
+    for (int j = threadIdx.x; j < N; j += blockDim.x) {
+        const double w = simpson_weight(j, N);
+        const double x2 = __dmul_rn(X[row + j], X[row + j]), d2 = __dmul_rn(dX[row + j], dX[row + j]);
+        double gc, cc, fc;
+        L.gcf(j, th0, two_th0, th0sq, gc, cc, fc);
+        // utils.py:1669-1673
+        const double* b = L.b;
+        const double B = b[IBS_BASE_BMAG * N + j], gp = fabs(b[IBS_BASE_GRADPAR * N + j]);
+        const double dgd = __dadd_rn(__dmul_rn(2.0, b[IBS_BASE_GDS21 * N + j]), __dmul_rn(two_th0, b[IBS_BASE_GDS22 * N + j]));
+        const double gpB = __dmul_rn(gp, B);
+        const double g_t0 = __ddiv_rn(__dmul_rn(gp, dgd), B);
+        const double c_t0 = __ddiv_rn(__dmul_rn(__dmul_rn(-1.0, L.dP), b[IBS_BASE_CVDRIFT0 * N + j]), gpB);
+        const double f_t0 = __ddiv_rn(__ddiv_rn(dgd, __dmul_rn(B, B)), gpB);
+        // d/d alpha of g = gp gd / B, c = -dP cv / (gp B), f = gd / (B^2 gp B)
+        const double cv = b[IBS_BASE_CVDRIFT * N + j] + th0 * b[IBS_BASE_CVDRIFT0 * N + j];
+        const double gd = b[IBS_BASE_GDS2 * N + j] + two_th0 * b[IBS_BASE_GDS21 * N + j] + th0sq * b[IBS_BASE_GDS22 * N + j];
+        const double dB = db[IBS_BASE_BMAG * N + j];
+        const double dgp = (b[IBS_BASE_GRADPAR * N + j] < 0.0 ? -1.0 : 1.0) * db[IBS_BASE_GRADPAR * N + j];
+        const double dcv = db[IBS_BASE_CVDRIFT * N + j] + th0 * db[IBS_BASE_CVDRIFT0 * N + j];
+        const double dgdv = db[IBS_BASE_GDS2 * N + j] + two_th0 * db[IBS_BASE_GDS21 * N + j] + th0sq * db[IBS_BASE_GDS22 * N + j];
+        const double rB = dB / B, rgpB = (dgp * B + gp * dB) / gpB;           // d log B, d log (gp B)
+        const double g_a = (dgp * gd + gp * dgdv) / B - gc * rB;
+        const double c_a = -(ddP * cv + L.dP * dcv) / gpB - cc * rgpB;
+        const double f_a = dgdv / (B * B * gpB) - fc * (2.0 * rB + rgpB);
+        v[0] += w * __dmul_rn(fc, x2);
+        v[1] += w * __dmul_rn(c_t0, x2);
+        v[2] += w * __dmul_rn(g_t0, d2);
+        v[3] += w * __dmul_rn(f_t0, x2);
+        v[4] += w * __dmul_rn(c_a, x2);
+        v[5] += w * __dmul_rn(g_a, d2);
+        v[6] += w * __dmul_rn(f_a, x2);
+    }
+    block_sum<7>(v, sm);
+    if (threadIdx.x == 0) {
+        const double l = lam[p];
+        const double jt = __dsub_rn(__dsub_rn(__ddiv_rn(v[1], v[0]), __ddiv_rn(v[2], v[0])), __ddiv_rn(__dmul_rn(l, v[3]), v[0]));
+        const double ja = __dsub_rn(__dsub_rn(__ddiv_rn(v[4], v[0]), __ddiv_rn(v[5], v[0])), __ddiv_rn(__dmul_rn(l, v[6]), v[0]));
+        val_out[p] = -1 * l;
+        grad_out[2 * p + 0] = -1 * ja;
+        grad_out[2 * p + 1] = -1 * jt;
+    }
+}
+
 __global__ void centre_lines_kernel(int* line, int n) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i < n) line[i] = 3 * i + 1;
+}
+__global__ void identity_lines_kernel(int* line, int n) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n) line[i] = i;
 }
 
 // Per-surface arg-max with the guards of ball_scan.py:279-295.
@@ -295,9 +361,23 @@ int launch_obj_grad(const double* base3, const double* dPdrho3, const double* th
     IBS_CUDA_CHECK(cudaGetLastError());
     return IBS_OK;
 }
+int launch_obj_grad_tangent(const double* base, const double* dbase, const double* dPdrho, const double* ddPdrho, const double* theta0,
+                            const double* lam, const double* X, const double* dX, int npoint, int N, double* val, double* grad,
+                            cudaStream_t st) {
+    if (npoint == 0) return IBS_OK;
+    obj_grad_tangent_kernel<<<npoint, RED_THREADS, 0, st>>>(base, dbase, dPdrho, ddPdrho, theta0, lam, X, dX, N, val, grad);
+    IBS_CUDA_CHECK(cudaGetLastError());
+    return IBS_OK;
+}
 int launch_centre_lines(int* line, int n, cudaStream_t st) {
     if (n == 0) return IBS_OK;
     centre_lines_kernel<<<(n + 255) / 256, 256, 0, st>>>(line, n);
+    IBS_CUDA_CHECK(cudaGetLastError());
+    return IBS_OK;
+}
+int launch_identity_lines(int* line, int n, cudaStream_t st) {
+    if (n == 0) return IBS_OK;
+    identity_lines_kernel<<<(n + 255) / 256, 256, 0, st>>>(line, n);
     IBS_CUDA_CHECK(cudaGetLastError());
     return IBS_OK;
 }

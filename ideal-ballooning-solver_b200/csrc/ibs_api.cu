@@ -18,6 +18,16 @@ int geometry_dispatch(const double* tab_mn, const double* tab_nyq, const double*
                       const double* alpha, int nalpha, int alpha_per_surface, const double* theta, int nl,
                       double phi_center, double* base_out, double* dPdrho_out, double* theta_vmec_out,
                       int* info_out, cudaStream_t st);
+int geometry_tangent_dispatch(const double* tab_mn, const double* tab_nyq, const double* scal,
+                              const double* xm, const double* xn, const double* xm_nyq, const double* xn_nyq,
+                              int ns, int mnmax, int mnmax_nyq, double phiedge, double aminor_p,
+                              const double* alpha, int nalpha, int alpha_per_surface, const double* theta, int nl,
+                              double phi_center, double* base_out, double* dPdrho_out, double* dbase_out, double* ddPdrho_out,
+                              double* theta_vmec_out, int* info_out, cudaStream_t st);
+int launch_obj_grad_tangent(const double* base, const double* dbase, const double* dPdrho, const double* ddPdrho, const double* theta0,
+                            const double* lam, const double* X, const double* dX, int npoint, int N, double* val, double* grad,
+                            cudaStream_t st);
+int launch_identity_lines(int* line, int n, cudaStream_t st);
 int launch_adjoint(const double* lam, const double* X, const double* dX, const double* f, const double* g_p,
                    const double* c_p, const double* f_p, int nsolve, int nparam, int N, double* grad, cudaStream_t st);
 int launch_sensitivity(const double* lam, const double* X, const double* dX, const double* f, int nsolve, int N,
@@ -191,6 +201,21 @@ int ibs_geometry_batch(const double* tab_mn, const double* tab_nyq, const double
     return geometry_dispatch(tab_mn, tab_nyq, scal, xm, xn, xm_nyq, xn_nyq, ns, mnmax, mnmax_nyq, phiedge, aminor_p, alpha,
                              nalpha, alpha_per_surface, theta, nl, phi_center, base_out, dPdrho_out, theta_vmec_out,
                              info_out, (cudaStream_t)stream);
+}
+
+int ibs_geometry_tangent_batch(const double* tab_mn, const double* tab_nyq, const double* scal,
+                               const double* xm, const double* xn, const double* xm_nyq, const double* xn_nyq,
+                               int ns, int mnmax, int mnmax_nyq, double phiedge, double aminor_p,
+                               const double* alpha, int nalpha, int alpha_per_surface,
+                               const double* theta, int nl, double phi_center, double* base_out, double* dPdrho_out,
+                               double* dbase_out, double* ddPdrho_out, double* theta_vmec_out, int* info_out, void* stream) {
+    IBS_REQUIRE(tab_mn && tab_nyq && scal && xm && xn && xm_nyq && xn_nyq && alpha && theta && base_out && dbase_out, "null pointer");
+    IBS_REQUIRE(ns >= 0 && nalpha >= 0 && nl >= 1 && mnmax >= 1 && mnmax_nyq >= 1, "bad sizes");
+    IBS_REQUIRE(aminor_p > 0.0 && phiedge != 0.0, "Aminor_p must be > 0 and phiedge != 0");
+    if (ns == 0 || nalpha == 0) return IBS_OK;
+    return geometry_tangent_dispatch(tab_mn, tab_nyq, scal, xm, xn, xm_nyq, xn_nyq, ns, mnmax, mnmax_nyq, phiedge, aminor_p, alpha,
+                                     nalpha, alpha_per_surface, theta, nl, phi_center, base_out, dPdrho_out, dbase_out, ddPdrho_out,
+                                     theta_vmec_out, info_out, (cudaStream_t)stream);
 }
 
 int ibs_geometry_full_nfields(void) { return geometry_full_nfields(); }
@@ -371,6 +396,37 @@ int ibs_obj_w_grad_batch(const double* base3, const double* dPdrho3, const doubl
         rc = solve_dispatch(p, true, false, st);
     }
     if (rc == IBS_OK) rc = launch_obj_grad(base3, dPdrho3, theta0, lam, X, dX, npoint, N, del_alpha, val_out, grad_out, st);
+    cudaFreeAsync(ws, st);
+    return rc;
+}
+
+int ibs_obj_w_grad_tangent_batch(const double* base, const double* dbase, const double* dPdrho, const double* ddPdrho,
+                                 const double* theta0, int npoint, int N, double h, const double* lam0, double* val_out,
+                                 double* grad_out, double* X_out, double* dX_out, int* info_out, void* stream) {
+    IBS_REQUIRE(npoint >= 0 && N >= 5 && h > 0.0, "bad sizes");
+    if (npoint == 0) return IBS_OK;
+    IBS_REQUIRE(base && dbase && dPdrho && ddPdrho && theta0 && val_out && grad_out, "null pointer");
+    cudaStream_t st = (cudaStream_t)stream;
+    // the solve is ibs_obj_w_grad_batch's (explicit line per solve, same kernel choice) on line i instead of 3 i + 1
+    const size_t o_line = 0, o_lam = ((size_t)npoint * sizeof(int) + 255) & ~(size_t)255;
+    const size_t o_X = o_lam + (((size_t)npoint * sizeof(double) + 255) & ~(size_t)255);
+    const size_t xbytes = ((size_t)npoint * N * sizeof(double) + 255) & ~(size_t)255;
+    const size_t o_dX = o_X + (X_out ? 0 : xbytes), total = o_dX + (dX_out ? 0 : xbytes);
+    char* ws = nullptr;
+    IBS_CUDA_CHECK(cudaMallocAsync((void**)&ws, total + 256, st));
+    int* line = (int*)(ws + o_line);
+    double* lam = (double*)(ws + o_lam);
+    double* X = X_out ? X_out : (double*)(ws + o_X);
+    double* dX = dX_out ? dX_out : (double*)(ws + o_dX);
+    int rc = launch_identity_lines(line, npoint, st);
+    if (rc == IBS_OK) {
+        SolveParams p = blank_params();
+        p.base = base; p.dPdrho = dPdrho; p.theta0 = theta0; p.line_of_solve = line; p.nth0 = 1;
+        p.nsolve = npoint; p.N = N; p.h = h; p.lam0 = lam0;
+        p.lam_out = lam; p.X_out = X; p.dX_out = dX; p.info_out = info_out;
+        rc = solve_dispatch(p, true, false, st);
+    }
+    if (rc == IBS_OK) rc = launch_obj_grad_tangent(base, dbase, dPdrho, ddPdrho, theta0, lam, X, dX, npoint, N, val_out, grad_out, st);
     cudaFreeAsync(ws, st);
     return rc;
 }

@@ -23,6 +23,7 @@
 #include <cstdlib>
 
 #include "ibs_common.cuh"
+#include "ibs_geometry_ad.cuh"
 
 namespace ibs {
 
@@ -871,6 +872,201 @@ __global__ void dpdrho_kernel(const double* __restrict__ base, int nlines, int n
     if (lane == 0) out[line] = -1.0 * 0.5 * (acc / (double)nl);
 }
 
+// ---- alpha-tangent of K1 (second pass over the packed tables) -------------------------------------------------------------
+// alpha enters K1 only through phi = phi_c + (theta_p - alpha) / iota, so at fixed theta_p
+//     d/d alpha = phi' d/d phi,   phi' = -1 / iota,   theta_vmec' = theta_phi phi',   theta_phi = -L_p / (1 + L_t)
+// (implicit derivative of the converged Newton residual th + lambda(th, phi) = theta_p), and every mode sum moves by
+//     S_r' = (T_r theta_phi + P_r) phi',   T_r = d S_r / d theta_vmec (an m-weight),   P_r = d S_r / d phi (an n-weight).
+// One thread per point, at the theta_vmec the value pass stored.  With the paired layout (E, O) of ibs_geometry.cu, per
+// m and row v: A = sum_k E cos(k nfp phi), B = sum_k O sin(k nfp phi) (k = 0 in A), and their phi-derivatives from the
+// same loads, An = sum_k kn O cos, Bn = sum_k kn E sin (kn = k nfp; d A / d phi = -Bn, d B / d phi = An), plus
+// Ann = sum_k kn^2 E cos, Bnn = sum_k kn^2 O sin for the rows whose n-weighted sums (R_p, Z_p, L_p, B_p) are outputs.
+// A cos-sum is C(A, B) = cm A + sm B, a sin-sum Sn(A, B) = sm A - cm B (cm, sm = cos, sin(m theta_vmec)); then
+//     d C / d theta = -m Sn(A, B),  d Sn / d theta = m C(A, B),  d C / d phi = Sn(An, Bn),  d Sn / d phi = -C(An, Bn).
+// The axisymmetric tables (dense layout, n = 0 only) are the same code with an empty k loop.  The toroidal range is a
+// run-time bound and cos / sin(k nfp phi) advance by the three-term recurrence of geometry3d_kernel: one kernel for every
+// shape.  The pointwise algebra is geo_point_epilogue's on D1 (base_point, ibs_geometry_ad.cuh), seeded with S_r' and with
+// phi' in sin / cos(phi) and in the secular term (phi - phi_c) iota'.
+constexpr int GEO_TAN_THREADS = 128;
+
+__global__ void __launch_bounds__(GEO_TAN_THREADS)
+geometry_tangent_kernel(const GeoParams p, const int NT1, const int NT2, const double* __restrict__ thv, double* __restrict__ dbase) {
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    double* s_mn = reinterpret_cast<double*>(smem_raw);
+    const bool paired = NT1 > 0;                               // geometry_dispatch: NT1 == 0 <=> NT2 == 0 (dense layout)
+    const int sm1 = paired ? (NT1 + 1) * ROWP_MN : ROW_MN, sm2 = paired ? (NT2 + 1) * ROWP_NYQ : ROW_NYQ, jst = paired ? 2 : 1;
+    const int n_mn = p.M1 * sm1, n_nyq = p.M2 * sm2;
+    double* s_nyq = s_mn + n_mn;
+    const int tid = threadIdx.x;
+    const int pts_per_surface = p.nalpha * p.nl;
+    const int tiles_per_surface = (pts_per_surface + GEO_TAN_THREADS - 1) / GEO_TAN_THREADS;
+    const long long W = (long long)p.ns * tiles_per_surface;
+    const long long w_begin = W * blockIdx.x / gridDim.x, w_end = W * (blockIdx.x + 1) / gridDim.x;
+    const double nfp = (double)p.nfp;
+    int js = -1;
+    double s_val = 0, iota = 1, d_iota = 0, dpds = 0, shat = 0;
+    for (long long w = w_begin; w < w_end; ++w) {
+        const int js_w = (int)(w / tiles_per_surface);
+        const int tile = (int)(w - (long long)js_w * tiles_per_surface);
+        if (js_w != js) {
+            js = js_w;
+            __syncthreads();
+            const double* src = p.pk_mn + (size_t)js * n_mn;
+            for (int i = tid; i < n_mn; i += GEO_TAN_THREADS) s_mn[i] = src[i];
+            src = p.pk_nyq + (size_t)js * n_nyq;
+            for (int i = tid; i < n_nyq; i += GEO_TAN_THREADS) s_nyq[i] = src[i];
+            const double* sc = p.scal + (size_t)js * IBS_NSCAL;
+            s_val = sc[0]; iota = sc[1]; d_iota = sc[2]; dpds = sc[3]; shat = sc[4];
+            __syncthreads();
+        }
+        const int pt = tile * GEO_TAN_THREADS + tid;
+        if (pt >= pts_per_surface) continue;
+        const int ja = pt / p.nl, jl = pt - ja * p.nl;
+        const size_t line = (size_t)js * p.nalpha + ja;
+        const double al = p.alpha_per_surface ? p.alpha[(size_t)js * p.nalpha + ja] : p.alpha[ja];
+        const double phi = p.phi_center + (p.theta[jl] - al) / iota;            // as in geometry_kernel
+        const double th = thv[line * p.nl + jl];
+        double s1, c1, s1p = 0.0, c1p = 1.0;
+        sincos(th, &s1, &c1);
+        if (paired) sincos(nfp * phi, &s1p, &c1p);
+        const double tcp = 2.0 * c1p;
+        double S[NSUM], T[NSUM], P[NSUM];
+#pragma unroll
+        for (int r = 0; r < NSUM; ++r) { S[r] = 0.0; T[r] = 0.0; P[r] = 0.0; }
+        // ---- (R, Z, lambda) set: rows 0 r, 2 r_s, 3 z, 5 z_s, 6 l, 8 l_s (the n-weighted rows 1, 4, 7 come from the pairs)
+        {
+            constexpr int RJ[6] = {0, 2, 3, 5, 6, 8};
+            double cm = 1.0, sm = 0.0;
+            for (int m = 0; m < p.M1; ++m) {
+                const double* row = s_mn + (size_t)m * sm1;
+                double A[6], Bq[6], An[6], Bn[6], Ann[3], Bnn[3];
+#pragma unroll
+                for (int i = 0; i < 6; ++i) { A[i] = row[RJ[i] * jst]; Bq[i] = 0.0; An[i] = 0.0; Bn[i] = 0.0; }
+#pragma unroll
+                for (int i = 0; i < 3; ++i) { Ann[i] = 0.0; Bnn[i] = 0.0; }
+                double ck = c1p, sk = s1p, ckm = 1.0, skm = 0.0;
+                for (int k = 1; k <= NT1; ++k) {
+                    const double kn = (double)k * nfp, kc = kn * ck, ks = kn * sk, kkc = kn * kc, kks = kn * ks;
+                    const double* rk = row + k * ROWP_MN;
+#pragma unroll
+                    for (int i = 0; i < 6; ++i) {
+                        const double2 eo = *reinterpret_cast<const double2*>(rk + 2 * RJ[i]);
+                        A[i] = fma(eo.x, ck, A[i]); Bq[i] = fma(eo.y, sk, Bq[i]);
+                        An[i] = fma(eo.y, kc, An[i]); Bn[i] = fma(eo.x, ks, Bn[i]);
+                        if ((i & 1) == 0) { Ann[i / 2] = fma(eo.x, kkc, Ann[i / 2]); Bnn[i / 2] = fma(eo.y, kks, Bnn[i / 2]); }
+                    }
+                    const double cn = fma(tcp, ck, -ckm), sn = fma(tcp, sk, -skm);
+                    ckm = ck; skm = sk; ck = cn; sk = sn;
+                }
+                const double dm = (double)m, dm2 = dm * dm;
+                auto C = [&](double a, double b) { return fma(cm, a, sm * b); };
+                auto Sn = [&](double a, double b) { return fma(sm, a, -(cm * b)); };
+                // r: R (cos-sum), R_t = dR/dtheta, R_p = dR/dphi
+                const double cr = C(A[0], Bq[0]), sr = Sn(A[0], Bq[0]), cnr = C(An[0], Bn[0]), snr = Sn(An[0], Bn[0]);
+                S[S_R] += cr;          T[S_R] -= dm * sr;          P[S_R] += snr;
+                S[S_Rt] -= dm * sr;    T[S_Rt] -= dm2 * cr;        P[S_Rt] += dm * cnr;
+                S[S_Rp] += snr;        T[S_Rp] += dm * cnr;        P[S_Rp] -= C(Ann[0], Bnn[0]);
+                S[S_Rs] += C(A[1], Bq[1]);  T[S_Rs] -= dm * Sn(A[1], Bq[1]);  P[S_Rs] += Sn(An[1], Bn[1]);
+                // z, lambda: sin-sums; their theta- and phi-derivatives are the outputs
+                const double cz = C(A[2], Bq[2]), sz = Sn(A[2], Bq[2]), cnz = C(An[2], Bn[2]), snz = Sn(An[2], Bn[2]);
+                S[S_Zt] += dm * cz;    T[S_Zt] -= dm2 * sz;        P[S_Zt] += dm * snz;
+                S[S_Zp] -= cnz;        T[S_Zp] += dm * snz;        P[S_Zp] -= Sn(Ann[1], Bnn[1]);
+                S[S_Zs] += Sn(A[3], Bq[3]);  T[S_Zs] += dm * C(A[3], Bq[3]);  P[S_Zs] -= C(An[3], Bn[3]);
+                const double cl = C(A[4], Bq[4]), sl = Sn(A[4], Bq[4]), cnl = C(An[4], Bn[4]), snl = Sn(An[4], Bn[4]);
+                S[S_Lt] += dm * cl;    T[S_Lt] -= dm2 * sl;        P[S_Lt] += dm * snl;
+                S[S_Lp] -= cnl;        T[S_Lp] += dm * snl;        P[S_Lp] -= Sn(Ann[2], Bnn[2]);
+                S[S_Ls] += Sn(A[5], Bq[5]);  T[S_Ls] += dm * C(A[5], Bq[5]);  P[S_Ls] -= C(An[5], Bn[5]);
+                const double cnx = fma(cm, c1, -(sm * s1));
+                sm = fma(sm, c1, cm * s1);
+                cm = cnx;
+            }
+        }
+        // theta_vmec moves with phi: fold the (R, Z, lambda) derivatives into d S_r / d phi along the field line now (frees P)
+        const double th_phi = -S[S_Lp] / (1.0 + S[S_Lt]);                        // d theta_vmec / d phi
+#pragma unroll
+        for (int r = S_R; r <= S_Lp; ++r) T[r] = fma(T[r], th_phi, P[r]);
+        // ---- Nyquist set: rows 0 g, 1 b, 3 b_s, 4 bsupv, 5 bsubs, 6 bsubu, 7 bsubv (row 2, n b, from the b pair)
+        {
+            constexpr int RJ[7] = {0, 1, 3, 4, 5, 6, 7};
+            double cm = 1.0, sm = 0.0;
+            for (int m = 0; m < p.M2; ++m) {
+                const double* row = s_nyq + (size_t)m * sm2;
+                double A[7], Bq[7], An[7], Bn[7], Ann = 0.0, Bnn = 0.0;
+#pragma unroll
+                for (int i = 0; i < 7; ++i) { A[i] = row[RJ[i] * jst]; Bq[i] = 0.0; An[i] = 0.0; Bn[i] = 0.0; }
+                double ck = c1p, sk = s1p, ckm = 1.0, skm = 0.0;
+                for (int k = 1; k <= NT2; ++k) {
+                    const double kn = (double)k * nfp, kc = kn * ck, ks = kn * sk;
+                    const double* rk = row + k * ROWP_NYQ;
+#pragma unroll
+                    for (int i = 0; i < 7; ++i) {
+                        const double2 eo = *reinterpret_cast<const double2*>(rk + 2 * RJ[i]);
+                        A[i] = fma(eo.x, ck, A[i]); Bq[i] = fma(eo.y, sk, Bq[i]);
+                        An[i] = fma(eo.y, kc, An[i]); Bn[i] = fma(eo.x, ks, Bn[i]);
+                        if (i == 1) { Ann = fma(eo.x, kn * kc, Ann); Bnn = fma(eo.y, kn * ks, Bnn); }
+                    }
+                    const double cn = fma(tcp, ck, -ckm), sn = fma(tcp, sk, -skm);
+                    ckm = ck; skm = sk; ck = cn; sk = sn;
+                }
+                const double dm = (double)m, dm2 = dm * dm;
+                auto C = [&](double a, double b) { return fma(cm, a, sm * b); };
+                auto Sn = [&](double a, double b) { return fma(sm, a, -(cm * b)); };
+                S[S_sqrtg] += C(A[0], Bq[0]);  T[S_sqrtg] -= dm * Sn(A[0], Bq[0]);  P[S_sqrtg] += Sn(An[0], Bn[0]);
+                const double cb = C(A[1], Bq[1]), sb = Sn(A[1], Bq[1]), cnb = C(An[1], Bn[1]), snb = Sn(An[1], Bn[1]);
+                S[S_B] += cb;          T[S_B] -= dm * sb;          P[S_B] += snb;
+                S[S_Bt] -= dm * sb;    T[S_Bt] -= dm2 * cb;        P[S_Bt] += dm * cnb;
+                S[S_Bp] += snb;        T[S_Bp] += dm * cnb;        P[S_Bp] -= C(Ann, Bnn);
+                S[S_Bs] += C(A[2], Bq[2]);  T[S_Bs] -= dm * Sn(A[2], Bq[2]);  P[S_Bs] += Sn(An[2], Bn[2]);
+                S[S_Bsupp] += C(A[3], Bq[3]);  T[S_Bsupp] -= dm * Sn(A[3], Bq[3]);  P[S_Bsupp] += Sn(An[3], Bn[3]);
+                S[S_Bsubs] += Sn(A[4], Bq[4]);  T[S_Bsubs] += dm * C(A[4], Bq[4]);  P[S_Bsubs] -= C(An[4], Bn[4]);
+                S[S_Bsubt] += C(A[5], Bq[5]);  T[S_Bsubt] -= dm * Sn(A[5], Bq[5]);  P[S_Bsubt] += Sn(An[5], Bn[5]);
+                S[S_Bsubp] += C(A[6], Bq[6]);  T[S_Bsubp] -= dm * Sn(A[6], Bq[6]);  P[S_Bsubp] += Sn(An[6], Bn[6]);
+                const double cnx = fma(cm, c1, -(sm * s1));
+                sm = fma(sm, c1, cm * s1);
+                cm = cnx;
+            }
+        }
+        // ---- tangent of the pointwise algebra
+        const double dphi = -1.0 / iota;                                        // d phi / d alpha
+#pragma unroll
+        for (int r = S_sqrtg; r < NSUM; ++r) T[r] = fma(T[r], th_phi, P[r]);
+        D1 Sd[NSUM];
+#pragma unroll
+        for (int r = 0; r < NSUM; ++r) Sd[r] = D1(S[r], T[r] * dphi);
+        PointConst<D1> k;
+        double sp, cp;
+        sincos(phi, &sp, &cp);
+        k.sp = D1(sp, cp * dphi); k.cp = D1(cp, -sp * dphi); k.dphi = D1(phi - p.phi_center, dphi);
+        k.iota = D1(iota); k.d_iota = D1(d_iota); k.dpds = D1(dpds); k.shat = D1(shat); k.s_val = D1(s_val);
+        k.psi_e = D1(p.psi_e); k.L_ref = D1(p.L_ref);
+        k.th0 = k.dP = k.sg = k.sc = k.sf = k.qw = 0.0;
+        D1 o[IBS_NBASE];
+        base_point(Sd, k, o);
+        double* d = dbase + line * IBS_NBASE * p.nl + jl;
+#pragma unroll
+        for (int r = 0; r < IBS_NBASE; ++r) d[(size_t)r * p.nl] = o[r].d;
+    }
+}
+
+// d(dPdrho) / d alpha = -0.5 mean( d[(cvdrift - gbdrift) bmag^2] / d alpha ); one warp per line, as dpdrho_kernel
+__global__ void ddpdrho_kernel(const double* __restrict__ base, const double* __restrict__ dbase, int nlines, int nl,
+                               double* __restrict__ out) {
+    const int line = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    if (line >= nlines) return;
+    const int lane = threadIdx.x & 31;
+    const double* b = base + (size_t)line * IBS_NBASE * nl;
+    const double* db = dbase + (size_t)line * IBS_NBASE * nl;
+    double acc = 0.0;
+    for (int j = lane; j < nl; j += 32) {
+        const double bm = b[(size_t)IBS_BASE_BMAG * nl + j];
+        const double cg = b[(size_t)IBS_BASE_CVDRIFT * nl + j] - b[(size_t)IBS_BASE_GBDRIFT * nl + j];
+        const double dcg = db[(size_t)IBS_BASE_CVDRIFT * nl + j] - db[(size_t)IBS_BASE_GBDRIFT * nl + j];
+        acc += fma(dcg, bm * bm, 2.0 * cg * bm * db[(size_t)IBS_BASE_BMAG * nl + j]);
+    }
+    acc = warp_sum(acc);
+    if (lane == 0) out[line] = -0.5 * (acc / (double)nl);
+}
+
 // ---- host side ------------------------------------------------------------------------------------------------
 template <int NT1, int NT2>
 static int launch_geometry(const GeoParams& p, cudaStream_t st) {
@@ -921,14 +1117,37 @@ static int launch_geometry3d(const GeoParams& p, int NT1, int NT2, cudaStream_t 
     return IBS_OK;
 }
 
+static int launch_geometry_tangent(const GeoParams& p, int NT1, int NT2, const double* thv, double* dbase, cudaStream_t st) {
+    const size_t smem = (NT1 > 0 ? (size_t)p.M1 * (NT1 + 1) * ROWP_MN + (size_t)p.M2 * (NT2 + 1) * ROWP_NYQ
+                                 : (size_t)p.M1 * ROW_MN + (size_t)p.M2 * ROW_NYQ) * sizeof(double);
+    if (smem > 220 * 1024) { set_error("Fourier tables of one surface do not fit in shared memory"); return IBS_ERR_UNSUPPORTED; }
+    static bool configured[IBS_MAX_DEVICES] = {false};
+    const int dslot = current_device_slot();
+    if (!configured[dslot]) {
+        IBS_CUDA_CHECK(cudaFuncSetAttribute(geometry_tangent_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024));
+        configured[dslot] = true;
+    }
+    int per_sm = 0;
+    IBS_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, geometry_tangent_kernel, GEO_TAN_THREADS, smem));
+    if (per_sm < 1) per_sm = 1;
+    const int tiles = (p.nalpha * p.nl + GEO_TAN_THREADS - 1) / GEO_TAN_THREADS;
+    const long long slots = (long long)num_sms() * per_sm, W = (long long)p.ns * tiles;
+    const int grid = (int)(W < slots ? W : slots);
+    geometry_tangent_kernel<<<grid, GEO_TAN_THREADS, smem, st>>>(p, NT1, NT2, thv, dbase);
+    IBS_CUDA_CHECK(cudaGetLastError());
+    return IBS_OK;
+}
+
 static int gcd_int(int a, int b) { a = std::abs(a); b = std::abs(b); while (b) { int t = a % b; a = b; b = t; } return a; }
 
-int geometry_dispatch(const double* tab_mn, const double* tab_nyq, const double* scal,
-                      const double* xm, const double* xn, const double* xm_nyq, const double* xn_nyq,
-                      int ns, int mnmax, int mnmax_nyq, double phiedge, double aminor_p,
-                      const double* alpha, int nalpha, int alpha_per_surface, const double* theta, int nl,
-                      double phi_center, double* base_out, double* dPdrho_out, double* theta_vmec_out,
-                      int* info_out, cudaStream_t st) {
+// K1, and with dbase_out its alpha-tangent: the value kernel runs unchanged (so its outputs are those of ibs_geometry_batch
+// bit for bit), then geometry_tangent_kernel on the same packed tables at the theta_vmec it stored
+static int geometry_run(const double* tab_mn, const double* tab_nyq, const double* scal,
+                        const double* xm, const double* xn, const double* xm_nyq, const double* xn_nyq,
+                        int ns, int mnmax, int mnmax_nyq, double phiedge, double aminor_p,
+                        const double* alpha, int nalpha, int alpha_per_surface, const double* theta, int nl,
+                        double phi_center, double* base_out, double* dPdrho_out, double* theta_vmec_out,
+                        int* info_out, double* dbase_out, double* ddPdrho_out, cudaStream_t st) {
     // ---- mode bookkeeping (host): toroidal stride, extents, dense-grid index of every mode
     int nfp = 0, mmax1 = 0, mmax2 = 0;
     for (int k = 0; k < mnmax; ++k) { nfp = gcd_int(nfp, (int)std::lround(xn[k])); mmax1 = std::max(mmax1, (int)std::lround(xm[k])); }
@@ -983,8 +1202,11 @@ int geometry_dispatch(const double* tab_mn, const double* tab_nyq, const double*
         d_idx = mc.dev;
     }
     keep_pool_cached();
-    IBS_CUDA_CHECK(cudaMallocAsync((void**)&pk, (n_mn + n_nyq) * sizeof(double), st));
+    // the tangent pass reads theta_vmec: a scratch copy after the tables when the caller does not want it
+    const size_t n_thv = (dbase_out && !theta_vmec_out) ? (size_t)ns * nalpha * nl : 0;
+    IBS_CUDA_CHECK(cudaMallocAsync((void**)&pk, (n_mn + n_nyq + n_thv) * sizeof(double), st));
     IBS_CUDA_CHECK(cudaMemsetAsync(pk, 0, (n_mn + n_nyq) * sizeof(double), st));
+    if (n_thv) theta_vmec_out = pk + n_mn + n_nyq;
     pack_mn_kernel<<<dim3(ns, (mnmax + 127) / 128), 128, 0, st>>>(tab_mn, d_idx, d_idx + mnmax, ns, mnmax, M1, W1, NT1, nfp, pk);
     pack_nyq_kernel<<<dim3(ns, (mnmax_nyq + 127) / 128), 128, 0, st>>>(tab_nyq, d_idx + 2 * mnmax, d_idx + 2 * mnmax + mnmax_nyq, ns,
                                                                      mnmax_nyq, M2, W2, NT2, nfp, pk + n_mn);
@@ -1009,8 +1231,37 @@ int geometry_dispatch(const double* tab_mn, const double* tab_nyq, const double*
         dpdrho_kernel<<<(nlines + 3) / 4, 128, 0, st>>>(base_out, nlines, nl, dPdrho_out);
         if (cudaGetLastError() != cudaSuccess) rc = IBS_ERR_CUDA;
     }
+    if (rc == IBS_OK && dbase_out) {
+        rc = launch_geometry_tangent(p, NT1, NT2, theta_vmec_out, dbase_out, st);
+        if (rc == IBS_OK && ddPdrho_out) {
+            const int nlines = ns * nalpha;
+            ddpdrho_kernel<<<(nlines + 3) / 4, 128, 0, st>>>(base_out, dbase_out, nlines, nl, ddPdrho_out);
+            if (cudaGetLastError() != cudaSuccess) rc = IBS_ERR_CUDA;
+        }
+    }
     cudaFreeAsync(pk, st);
     return rc;
+}
+
+int geometry_dispatch(const double* tab_mn, const double* tab_nyq, const double* scal,
+                      const double* xm, const double* xn, const double* xm_nyq, const double* xn_nyq,
+                      int ns, int mnmax, int mnmax_nyq, double phiedge, double aminor_p,
+                      const double* alpha, int nalpha, int alpha_per_surface, const double* theta, int nl,
+                      double phi_center, double* base_out, double* dPdrho_out, double* theta_vmec_out,
+                      int* info_out, cudaStream_t st) {
+    return geometry_run(tab_mn, tab_nyq, scal, xm, xn, xm_nyq, xn_nyq, ns, mnmax, mnmax_nyq, phiedge, aminor_p, alpha, nalpha,
+                        alpha_per_surface, theta, nl, phi_center, base_out, dPdrho_out, theta_vmec_out, info_out, nullptr, nullptr, st);
+}
+
+int geometry_tangent_dispatch(const double* tab_mn, const double* tab_nyq, const double* scal,
+                              const double* xm, const double* xn, const double* xm_nyq, const double* xn_nyq,
+                              int ns, int mnmax, int mnmax_nyq, double phiedge, double aminor_p,
+                              const double* alpha, int nalpha, int alpha_per_surface, const double* theta, int nl,
+                              double phi_center, double* base_out, double* dPdrho_out, double* dbase_out, double* ddPdrho_out,
+                              double* theta_vmec_out, int* info_out, cudaStream_t st) {
+    return geometry_run(tab_mn, tab_nyq, scal, xm, xn, xm_nyq, xn_nyq, ns, mnmax, mnmax_nyq, phiedge, aminor_p, alpha, nalpha,
+                        alpha_per_surface, theta, nl, phi_center, base_out, dPdrho_out, theta_vmec_out, info_out, dbase_out,
+                        ddPdrho_out, st);
 }
 
 }  // namespace ibs

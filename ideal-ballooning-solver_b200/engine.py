@@ -133,6 +133,43 @@ def geometry_batch(tables: DeviceTables, alpha, theta, phi_center: float = 0.0, 
     return Geometry(base, dP, thv, info)
 
 
+@dataclasses.dataclass
+class GeometryTangent(Geometry):
+    dbase: Optional[torch.Tensor] = None      # (ns, nalpha, 8, nl)  d base / d alpha at fixed theta_pest
+    ddPdrho: Optional[torch.Tensor] = None    # (ns, nalpha)         d dPdrho / d alpha
+
+
+def geometry_tangent_batch(tables: DeviceTables, alpha, theta, phi_center: float = 0.0, want_theta_vmec: bool = False,
+                           want_info: bool = False) -> GeometryTangent:
+    """K1 and its exact alpha-derivative (``ibs_geometry_tangent_batch``): the ``Geometry`` of ``geometry_batch`` (the same
+    bits) plus ``dbase`` and ``ddPdrho``, the derivatives of the eight base arrays and of dPdrho with respect to the field-line
+    label alpha at fixed theta_pest.  ``alpha`` is ``(nalpha,)`` (shared) or ``(ns, nalpha)`` (per surface)."""
+    _lib.require_cuda()
+    lib = _lib.load()
+    dev = tables.tab_mn.device
+    alpha = _f64(alpha, dev, "alpha")
+    theta = _f64(theta, dev, "theta")
+    per_surface = alpha.dim() == 2
+    if per_surface and alpha.shape[0] != tables.ns:
+        raise ValueError("alpha must be (nalpha,) or (ns, nalpha)")
+    ns, nalpha, nl = tables.ns, alpha.shape[-1], theta.numel()
+    base = torch.empty((ns, nalpha, NBASE, nl), dtype=torch.float64, device=dev)
+    dbase = torch.empty_like(base)
+    dP = torch.empty((ns, nalpha), dtype=torch.float64, device=dev)
+    ddP = torch.empty_like(dP)
+    thv = torch.empty((ns, nalpha, nl), dtype=torch.float64, device=dev) if want_theta_vmec else None
+    info = torch.empty((ns, nalpha), dtype=torch.int32, device=dev) if want_info else None
+    with torch.cuda.device(dev):
+        rc = lib.ibs_geometry_tangent_batch(_ptr(tables.tab_mn), _ptr(tables.tab_nyq), _ptr(tables.scal),
+                                            tables.xm.ctypes.data, tables.xn.ctypes.data, tables.xm_nyq.ctypes.data,
+                                            tables.xn_nyq.ctypes.data, ns, len(tables.xm), len(tables.xm_nyq),
+                                            tables.phiedge, tables.Aminor_p, _ptr(alpha), nalpha, int(per_surface),
+                                            _ptr(theta), nl, float(phi_center), _ptr(base), _ptr(dP), _ptr(dbase), _ptr(ddP),
+                                            _ptr(thv), _ptr(info), _stream())
+    _lib.check(rc, "ibs_geometry_tangent_batch")
+    return GeometryTangent(base, dP, thv, info, dbase, ddP)
+
+
 def geometry_full(st: SurfaceTables, alpha, grid, mode: int = 0, theta_shift: float = 0.0, zero_xn_nyq: bool = False,
                   phi_center: float = 0.0, device="cuda"):
     """Every per-point array of the reference's ``vmec_fieldlines`` / ``vmec_fieldlines_axisym`` Struct
@@ -358,6 +395,34 @@ def obj_w_grad_batch(base3, dPdrho3, theta0, h: float, del_alpha: float = 0.004,
         rc = lib.ibs_obj_w_grad_batch(_ptr(base3), _ptr(dP3), _ptr(theta0), npnt, N, float(h), float(del_alpha),
                                       _ptr(lam0), _ptr(val), _ptr(grad), _ptr(X), _ptr(dX), _ptr(info), _stream())
     _lib.check(rc, "ibs_obj_w_grad_batch")
+    return val, grad, X, dX, info
+
+
+def obj_w_grad_tangent_batch(base, dbase, dPdrho, ddPdrho, theta0, h: float, lam0=None, want_X=False):
+    """``obj_w_grad`` with the exact alpha-derivative (``ibs_obj_w_grad_tangent_batch``): ``base`` and ``dbase`` are
+    ``(npoint, 8, N)`` (one line per point and its alpha-tangent, from ``geometry_tangent_batch``), ``dPdrho`` and
+    ``ddPdrho`` ``(npoint,)``.  Returns ``(val, grad, X, dX, info)`` as ``obj_w_grad_batch``; ``val``, ``grad[:, 1]``, ``X``
+    and ``info`` are its bits on the same centre lines, ``grad[:, 0]`` is the chain rule instead of a central difference."""
+    _lib.require_cuda()
+    lib = _lib.load()
+    dev = base.device
+    N = base.shape[-1]
+    base = _f64(base, dev, "base").reshape(-1, NBASE, N)
+    npnt = base.shape[0]
+    dbase = _f64(dbase, dev, "dbase").reshape(npnt, NBASE, N)
+    dP = _f64(dPdrho, dev, "dPdrho").reshape(npnt)
+    ddP = _f64(ddPdrho, dev, "ddPdrho").reshape(npnt)
+    theta0 = _f64(theta0, dev, "theta0").reshape(npnt)
+    lam0 = None if lam0 is None else _f64(lam0, dev, "lam0")
+    val = torch.empty((npnt,), dtype=torch.float64, device=dev)
+    grad = torch.empty((npnt, 2), dtype=torch.float64, device=dev)
+    X = torch.empty((npnt, N), dtype=torch.float64, device=dev) if want_X else None
+    dX = torch.empty((npnt, N), dtype=torch.float64, device=dev) if want_X else None
+    info = torch.empty((npnt,), dtype=torch.int32, device=dev)
+    with torch.cuda.device(dev):
+        rc = lib.ibs_obj_w_grad_tangent_batch(_ptr(base), _ptr(dbase), _ptr(dP), _ptr(ddP), _ptr(theta0), npnt, N, float(h),
+                                              _ptr(lam0), _ptr(val), _ptr(grad), _ptr(X), _ptr(dX), _ptr(info), _stream())
+    _lib.check(rc, "ibs_obj_w_grad_tangent_batch")
     return val, grad, X, dX, info
 
 

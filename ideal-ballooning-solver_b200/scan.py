@@ -270,7 +270,8 @@ class RefineResult:
 
 
 def refine_maxima(tables: engine.DeviceTables, alpha_guess, theta0_guess, theta, maxiter: int = 30, ftol: float = 5.0e-11,
-                  gtol: float = 2.0e-08, method: str = "device", max_rounds: int = 200, sync_every: int = 4) -> RefineResult:
+                  gtol: float = 2.0e-08, method: str = "device", max_rounds: int = 200, sync_every: int = 4,
+                  alpha_derivative: str = "fd") -> RefineResult:
     """Refinement of every surface's coarse maximum (``ball_scan.py:305-314``: ``scipy.optimize.minimize(obj_w_grad,
     x0=(alpha_guess, theta0_guess), jac=True, bounds=((0, pi), (0, pi/2)), options={ftol, gtol, maxiter})``).
 
@@ -278,7 +279,16 @@ def refine_maxima(tables: engine.DeviceTables, alpha_guess, theta0_guess, theta,
     lock step, the optimiser state resident on the GPU; one round = K1 (three field lines per surface) + K2/K3 + K4
     (``ibs_obj_w_grad_batch``) + ``ibs_refine_step``, no host arithmetic; the host only polls the count of running problems
     every ``sync_every`` rounds.  ``method="scipy"``: the reference's own optimiser, one Python thread per surface around the
-    same batched evaluations (kept as the cross-check)."""
+    same batched evaluations (kept as the cross-check).
+
+    ``alpha_derivative`` (device method): ``"fd"`` (default) is the reference's central difference of (g, c, f) over the
+    lines ``alpha -+ 0.002`` (``utils.py:1707-1725``, three field lines per surface and round); ``"exact"`` takes K1 and its
+    alpha-tangent on the centre line only (``engine.geometry_tangent_batch`` + ``engine.obj_w_grad_tangent_batch``): the exact
+    derivative, one field line per surface and round."""
+    if alpha_derivative not in ("fd", "exact"):
+        raise ValueError("alpha_derivative must be 'fd' or 'exact'")
+    if method == "scipy" and alpha_derivative != "fd":
+        raise ValueError("method='scipy' evaluates the reference's obj_w_grad: alpha_derivative must be 'fd'")
     if method == "scipy":
         return _refine_maxima_scipy(tables, alpha_guess, theta0_guess, theta, maxiter, ftol, gtol)
     if method != "device":
@@ -293,8 +303,12 @@ def refine_maxima(tables: engine.DeviceTables, alpha_guess, theta0_guess, theta,
     rounds = 0
     while rounds < max_rounds:
         for _ in range(sync_every):
-            geo = engine.geometry_batch(tables, st.alphas3, theta_d)                      # utils.py:1641-1646: alpha -+ del/2
-            val, grad, _, _, info = engine.obj_w_grad_batch(geo.base, geo.dPdrho, st.theta0, h, del_alpha=DEL_ALPHA)
+            if alpha_derivative == "exact":
+                geo = engine.geometry_tangent_batch(tables, st.alphas3[:, 1:2], theta_d)     # the centre line alpha
+                val, grad, _, _, info = engine.obj_w_grad_tangent_batch(geo.base, geo.dbase, geo.dPdrho, geo.ddPdrho, st.theta0, h)
+            else:
+                geo = engine.geometry_batch(tables, st.alphas3, theta_d)                      # utils.py:1641-1646: alpha -+ del/2
+                val, grad, _, _, info = engine.obj_w_grad_batch(geo.base, geo.dPdrho, st.theta0, h, del_alpha=DEL_ALPHA)
             st.step(val, grad, info, ftol, gtol, maxiter)
             rounds += 1
         if int(st.nactive.item()) == 0:
@@ -358,10 +372,11 @@ class BallScanResult:
 
 def ball_scan(st: SurfaceTables, theta=None, mpol: Optional[int] = None, ntor: Optional[int] = None,
               nalpha_guess: int = NALPHA_GUESS, ntheta0_guess: int = NTHETA0_GUESS, refine: bool = True,
-              device=None, refine_method: str = "device") -> BallScanResult:
+              device=None, refine_method: str = "device", alpha_derivative: str = "fd") -> BallScanResult:
     """The numerical section of ``ball_scan.py:196-339`` for all surfaces of ``st`` at once:
     coarse 24 x 15 (alpha, theta0) grid (``:223-274``) -> guarded arg-max (``:279-295``) -> L-BFGS-B refinement
-    from the coarse maximum with the adjoint gradient (``:305-314``) -> eigenpair at the optimum (``:322-339``)."""
+    from the coarse maximum with the adjoint gradient (``:305-314``) -> eigenpair at the optimum (``:322-339``).
+    ``alpha_derivative`` is passed to ``refine_maxima``."""
     if theta is None:
         theta = scan_theta_grid(mpol, ntor)
     theta = np.asarray(theta, dtype=np.float64)
@@ -373,7 +388,7 @@ def ball_scan(st: SurfaceTables, theta=None, mpol: Optional[int] = None, ntor: O
     a_star, t_star = res.alpha_guess.cpu().numpy(), res.theta0_guess.cpu().numpy()
     ref = None
     if refine:
-        ref = refine_maxima(dt, a_star, t_star, theta, method=refine_method)
+        ref = refine_maxima(dt, a_star, t_star, theta, method=refine_method, alpha_derivative=alpha_derivative)
         a_star, t_star = ref.alpha, ref.theta0
     # ball_scan.py:322-339: geometry and eigenpair at the optimum
     geo = engine.geometry_batch(dt, torch.from_numpy(a_star[:, None].copy()).to(device), theta)

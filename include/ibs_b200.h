@@ -86,6 +86,19 @@ int ibs_geometry_batch(const double* tab_mn, const double* tab_nyq, const double
                        double* base_out, double* dPdrho_out, double* theta_vmec_out, int* info_out,
                        void* stream);
 
+/* K1 and its exact alpha-derivative.  Same arguments and value outputs as ibs_geometry_batch (base_out, dPdrho_out,
+ * theta_vmec_out and info_out are bit-identical to its), plus the tangent d/dalpha at fixed theta_pest of every base
+ * array and of dPdrho.  alpha enters only through phi = phi_center + (theta - alpha)/iota; theta_vmec moves with it by the
+ * implicit derivative of its root equation.  A second pass over the packed tables after the value kernel.
+ *   dbase_out [ns*nalpha][8][nl] (required); ddPdrho_out [ns*nalpha] or NULL.                                       */
+int ibs_geometry_tangent_batch(const double* tab_mn, const double* tab_nyq, const double* scal,
+                               const double* xm, const double* xn, const double* xm_nyq, const double* xn_nyq,
+                               int ns, int mnmax, int mnmax_nyq, double phiedge, double aminor_p,
+                               const double* alpha, int nalpha, int alpha_per_surface,
+                               const double* theta, int nl, double phi_center,
+                               double* base_out, double* dPdrho_out, double* dbase_out, double* ddPdrho_out,
+                               double* theta_vmec_out, int* info_out, void* stream);
+
 /* Full-output geometry: every per-point array of the Struct returned by vmec_fieldlines (utils.py:723-864) and by
  * vmec_fieldlines_axisym (utils.py:872-1542) -- the ~70 arrays gyrokinetic-geometry consumers read beyond the eight of
  * the ballooning path.  Not a hot kernel (direct mode sums; any mode list).  ALL pointers are device pointers.
@@ -197,6 +210,16 @@ int ibs_obj_w_grad_batch(const double* base3, const double* dPdrho3, const doubl
                          int npoint, int N, double h, double del_alpha, const double* lam0,
                          double* val_out, double* grad_out, double* X_out, double* dX_out,
                          int* info_out, void* stream);
+
+/* obj_w_grad with the exact alpha-derivative: one field line per point (base [npoint][8][N], dPdrho [npoint]) and its
+ * alpha-tangent from ibs_geometry_tangent_batch (dbase [npoint][8][N], ddPdrho [npoint]) instead of three lines.  The
+ * solve, val_out, grad_out[:, 1], X_out, dX_out and info_out are those of ibs_obj_w_grad_batch on the same centre lines
+ * bit for bit; grad_out[:, 0] = -dlam/dalpha from the chain rule through g, c, f (utils.py:1560-1562) instead of their
+ * central difference (utils.py:1707-1725).  lam0 [npoint] or NULL; X_out, dX_out [npoint][N] or NULL; info_out or NULL. */
+int ibs_obj_w_grad_tangent_batch(const double* base, const double* dbase, const double* dPdrho, const double* ddPdrho,
+                                 const double* theta0, int npoint, int N, double h, const double* lam0,
+                                 double* val_out, double* grad_out, double* X_out, double* dX_out,
+                                 int* info_out, void* stream);
 
 /* ---- scan: per-surface arg-max with the reference's guards (ball_scan.py:279-295) ----------------
  * gamma [ns][ngrid] (row-major (alpha, theta0) grid flattened).  For each surface:
