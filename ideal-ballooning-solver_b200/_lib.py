@@ -45,6 +45,8 @@ SIGNATURES = {
     "ibs_refine_init": (c_int, [_D, c_int, _D, _D, c_double, c_double, c_double, c_double, c_double, _D, _D, c_void_p]),
     "ibs_refine_step": (c_int, [_D, c_int, _D, _D, _I, c_double, c_double, c_int, c_double, _D, _D, _I, c_void_p]),
     "ibs_count_above_batch": (c_int, [_D, _D, _D, c_int, c_int, c_double, _D, _I, c_void_p]),
+    "ibs_marginal_batch": (c_int, [_D, _D, _D, _I, c_int, c_int, c_int, c_double, c_double, c_double, _D, _D, _D, _D, _I,
+                                   c_void_p]),
     "ibs_scan_solve_argmax": (c_int, [_D, _D, _D, c_int, c_int, c_int, c_int, c_double, _D, c_int, _D, _D, _D, _I, _D, _D, c_void_p]),
     "ibs_scan_host": (c_int, [_D, _D, _D, _D, _D, _D, _D, c_int, c_int, c_int, c_double, c_double,
                               _D, c_int, _D, c_int, _D, c_int, c_double, _D, _D, _I, _D, _D, _D, _I]),

@@ -15,7 +15,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIBDIR = os.path.join(HERE, "lib")
 LIB = os.path.join(LIBDIR, "libibs_b200.so")
-SOURCES = ["ibs_api.cu", "ibs_solver.cu", "ibs_scan_solver.cu", "ibs_geometry.cu", "ibs_geometry_full.cu", "ibs_geometry_adjoint.cu", "ibs_adjoint.cu"]
+SOURCES = ["ibs_api.cu", "ibs_solver.cu", "ibs_scan_solver.cu", "ibs_geometry.cu", "ibs_geometry_full.cu", "ibs_geometry_adjoint.cu", "ibs_adjoint.cu", "ibs_marginal.cu"]
 NVCC_FLAGS = ["-O3", "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo",
               "-Xcompiler", "-fPIC", "-DIBS_BUILD", "-fmad=true"]
 

@@ -18,6 +18,7 @@ from .tables import SurfaceTables
 NBASE = 8
 BASE_NAMES = ("bmag", "gradpar_theta_pest", "cvdrift", "cvdrift0", "gds2", "gds21", "gds22", "gbdrift")
 FLAG_NOT_CONVERGED, FLAG_BAD_INPUT, FLAG_SIGMA_NOT_MAX = 1, 2, 4
+FLAG_STABLE_TO_KMAX, FLAG_NOT_CONVEX = 8, 16            # marginal_batch only
 
 
 def _ptr(t: Optional[torch.Tensor]):
@@ -305,6 +306,58 @@ def count_above_batch(g, c, f, h: float, lam) -> torch.Tensor:
         rc = lib.ibs_count_above_batch(_ptr(g), _ptr(c), _ptr(f), n, N, float(h), _ptr(lam), _ptr(out), _stream())
     _lib.check(rc, "ibs_count_above_batch")
     return out
+
+
+@dataclasses.dataclass
+class Marginal:
+    kappa: torch.Tensor                        # (nsolve,) critical pressure-gradient factor kappa*; +inf: stable up to kappa_max
+    dlam_dkappa: Optional[torch.Tensor]        # (nsolve,) d lam_max / d kappa at kappa*
+    dkappa_dtheta0: Optional[torch.Tensor]     # (nsolve,) d kappa* / d theta0
+    X: Optional[torch.Tensor]                  # (nsolve, N) null vector at kappa*, >= 0 with max 1
+    info: torch.Tensor                         # (nsolve,) int32: sweeps | flags << 16
+
+    @property
+    def sweeps(self):
+        return self.info & 0xFFFF
+
+    @property
+    def flags(self):
+        return self.info >> 16
+
+
+def marginal_batch(base, dPdrho, theta0, h: float, nth0: Optional[int] = None, line_of_solve=None, kappa_max: float = 1e3,
+                   rtol: float = 1e-12, want_X: bool = False, want_derivs: bool = False) -> Marginal:
+    """Critical pressure-gradient factor of each solve: the smallest ``kappa`` at which the discrete pencil, with ``p'``
+    scaled by ``kappa`` at fixed geometry (``cvdrift -> gbdrift + kappa (cvdrift - gbdrift)``, ``dPdrho -> kappa dPdrho``),
+    has an eigenvalue above 0.  ``kappa* < 1`` means unstable as given.  Batch shape as :func:`solve_base_batch`."""
+    _lib.require_cuda()
+    lib = _lib.load()
+    dev = base.device
+    N = base.shape[-1]
+    base = _f64(base, dev, "base").reshape(-1, NBASE, N)
+    dP = _f64(dPdrho, dev, "dPdrho").reshape(-1)
+    theta0 = _f64(theta0, dev, "theta0").reshape(-1)
+    n = theta0.numel()
+    if line_of_solve is not None:
+        line_of_solve = torch.as_tensor(line_of_solve).to(device=dev, dtype=torch.int32).contiguous()
+        if line_of_solve.numel() != n:
+            raise ValueError("line_of_solve must have one entry per solve")
+    elif nth0 is None:
+        if n % base.shape[0]:
+            raise ValueError("give nth0 or line_of_solve")
+        nth0 = n // base.shape[0]
+    if line_of_solve is None and nth0 * base.shape[0] < n:
+        raise ValueError("not enough field lines for the requested solves")
+    new = lambda: torch.empty((n,), dtype=torch.float64, device=dev)
+    kappa = new()
+    dl, dk = (new(), new()) if want_derivs else (None, None)
+    X = torch.empty((n, N), dtype=torch.float64, device=dev) if want_X else None
+    info = torch.empty((n,), dtype=torch.int32, device=dev)
+    with torch.cuda.device(dev):
+        rc = lib.ibs_marginal_batch(_ptr(base), _ptr(dP), _ptr(theta0), _ptr(line_of_solve), int(nth0 or 1), n, N, float(h),
+                                    float(kappa_max), float(rtol), _ptr(kappa), _ptr(dl), _ptr(dk), _ptr(X), _ptr(info), _stream())
+    _lib.check(rc, "ibs_marginal_batch")
+    return Marginal(kappa, dl, dk, X, info)
 
 
 # ---------------------------------------------------------------------------------------------

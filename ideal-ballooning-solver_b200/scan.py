@@ -98,6 +98,48 @@ def coarse_scan(tables: engine.DeviceTables, alpha, theta0, theta, want_X: bool 
     return ScanResult(gamma, val, idx, sig, a_guess, t_guess, X, sol.info, geo)
 
 
+@dataclasses.dataclass
+class MarginalScanResult:
+    kappa: torch.Tensor            # (ns, nalpha, nth0) critical pressure-gradient factor kappa* of every solve
+    kappa_min: torch.Tensor        # (ns,) smallest kappa* of each surface (< 1: unstable as given)
+    idx: torch.Tensor              # (ns,) its flat (alpha, theta0) index (first minimum)
+    alpha_crit: torch.Tensor       # (ns,)
+    theta0_crit: torch.Tensor      # (ns,)
+    X: Optional[torch.Tensor]      # (ns, nl) null vector of each surface's minimum (if requested)
+    info: torch.Tensor             # (ns, nalpha, nth0) sweeps | flags << 16
+    geometry: engine.Geometry
+
+
+def marginal_scan(tables: engine.DeviceTables, alpha, theta0, theta, kappa_max: float = 1e3, rtol: float = 1e-12,
+                  want_X: bool = False) -> MarginalScanResult:
+    """Distance of every surface from ballooning instability on the coarse (alpha, theta0) grid: K1 for ``ns x nalpha``
+    field lines, ``engine.marginal_batch`` for every solve, and per surface the smallest kappa* with its (alpha, theta0).
+    The reduction is ``engine.scan_argmax(-kappa)``: first index among equal values, and kappa* > 0 keeps its all-zero
+    guard from firing.  +inf (stable up to ``kappa_max``) enters as the largest double, so a surface stable everywhere
+    reports ``kappa_min = inf`` at index 0; a NaN (bad input) gives ``kappa_min = nan`` and index -2."""
+    dev = tables.tab_mn.device
+    alpha_t = torch.as_tensor(np.asarray(alpha, dtype=np.float64)).to(dev) if not isinstance(alpha, torch.Tensor) else alpha
+    theta0_t = torch.as_tensor(np.asarray(theta0, dtype=np.float64)).to(dev) if not isinstance(theta0, torch.Tensor) else theta0
+    theta_np = theta.cpu().numpy() if isinstance(theta, torch.Tensor) else np.asarray(theta, dtype=np.float64)
+    geo = engine.geometry_batch(tables, alpha_t, theta_np)
+    ns, na, nt = tables.ns, alpha_t.shape[-1], theta0_t.numel()
+    h = engine.grid_spacing(theta_np)
+    m = engine.marginal_batch(geo.base, geo.dPdrho, theta0_t.repeat(ns * na), h, nth0=nt, kappa_max=kappa_max, rtol=rtol)
+    kappa = m.kappa.reshape(ns, na, nt)
+    big = torch.finfo(torch.float64).max
+    neg, idx, _ = engine.scan_argmax((-kappa).clamp(min=-big))
+    kmin = torch.where(neg == -big, torch.full_like(neg, float("inf")), -neg)
+    safe = idx.clamp(min=0).long()
+    ia, it = safe // nt, safe % nt
+    a_crit = alpha_t.gather(1, ia[:, None])[:, 0] if alpha_t.dim() == 2 else alpha_t[ia]
+    X = None
+    if want_X:
+        line = torch.arange(ns, device=dev, dtype=torch.int64) * na + ia
+        X = engine.marginal_batch(geo.base, geo.dPdrho, theta0_t[it], h, line_of_solve=line, kappa_max=kappa_max, rtol=rtol,
+                                  want_X=True).X
+    return MarginalScanResult(kappa, kmin, idx, a_crit, theta0_t[it], X, m.info.reshape(ns, na, nt), geo)
+
+
 class SurfaceGather:
     """The one exchange step of the scan (replaces the three ``MPI.Gather`` of ``ball_scan.py:345-347``) with NO kernel
     but the collective itself: the solver writes each local surface's packed ``(max, index)`` pair straight into this

@@ -54,6 +54,9 @@ extern "C" {
 #define IBS_FLAG_NOT_CONVERGED 1   /* iteration cap hit                                          */
 #define IBS_FLAG_BAD_INPUT 2       /* non-finite input, or g <= 0 / f <= 0 somewhere            */
 #define IBS_FLAG_SIGMA_NOT_MAX 4   /* eigenvalue nearest sigma (ARPACK semantics) is not lambda_max */
+#define IBS_FLAG_STABLE_TO_KMAX 8  /* ibs_marginal_batch: no crossing up to kappa_max (kappa* = +inf)   */
+#define IBS_FLAG_NOT_CONVEX 16     /* ibs_marginal_batch: c2 < 0 somewhere, the crossing found is not
+                                      certified to be the first one                                   */
 
 int ibs_version(void);
 const char* ibs_last_error(void);
@@ -267,6 +270,23 @@ int ibs_refine_step(double* state, int n, const double* val, const double* grad,
  * count_out[i] = number of eigenvalues of the pencil greater than lam[i]; unstable <=> count(0) > 0. */
 int ibs_count_above_batch(const double* g, const double* c, const double* f, int nsolve, int N, double h,
                           const double* lam, int* count_out, void* stream);
+
+/* ---- marginal stability: critical pressure-gradient factor ------------------------------------------
+ * kappa* = inf { kappa > 0 : the discrete pencil has an eigenvalue > 0 } when p' is scaled by kappa at fixed geometry,
+ * i.e. on the base arrays cvdrift -> gbdrift + kappa (cvdrift - gbdrift) and dPdrho -> kappa dPdrho, so that
+ * c(kappa) = kappa c1 + kappa^2 c2 with c1 = -dPdrho (gbdrift + theta0 cvdrift0) / (|gradpar| bmag) and
+ * c2 = -dPdrho (cvdrift - gbdrift) / (|gradpar| bmag); g and f do not depend on kappa.  kappa* follows the matrix
+ * eigenvalue lam_matrix (what a Sturm count at lam = 0 certifies), not the Simpson quotient.
+ * Batch shape and lines as ibs_solve_base_batch (theta0 [nsolve]; line_of_solve or line = i / nth0); 5 <= N <= 65538.
+ *   kappa_out [nsolve]: kappa* to the bracket width rtol kappa* (the smallest kappa certified unstable); +inf with
+ *     IBS_FLAG_STABLE_TO_KMAX when no crossing is found up to kappa_max (always when dPdrho = 0); NaN with BAD_INPUT.
+ *   X_out [nsolve][N] or NULL: the null vector of K(kappa*), >= 0 with max 1 (the nodeless ground state).
+ *   dlam_dkappa_out / dkappa_dtheta0_out [nsolve] or NULL: x^T dK/dkappa x / x^T F x and -x^T dK/dtheta0 x / x^T dK/dkappa x.
+ *   info_out [nsolve] or NULL: sweeps | flags << 16 (NOT_CONVERGED, BAD_INPUT, STABLE_TO_KMAX, NOT_CONVEX).              */
+int ibs_marginal_batch(const double* base, const double* dPdrho, const double* theta0, const int* line_of_solve,
+                       int nth0, int nsolve, int N, double h, double kappa_max, double rtol,
+                       double* kappa_out, double* dlam_dkappa_out, double* dkappa_dtheta0_out, double* X_out,
+                       int* info_out, void* stream);
 
 /* ---- end-to-end host entry point -----------------------------------------------------------------
  * Coarse scan of ball_scan.py:248-295 for ns surfaces with HOST buffers: copies the tables to the
