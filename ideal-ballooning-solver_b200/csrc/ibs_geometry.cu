@@ -71,7 +71,8 @@ struct GeoParams {
     int nfp;                // toroidal stride of the packed n index
     double phi_center, psi_e, L_ref;
     double* base_out; double* theta_vmec_out; int* info_out;
-    int fold;               // axisymmetric tables: allow the periodicity fold (IBS_GEO_FOLD=0 turns it off)
+    int fold;               // axisymmetric tables: allow the periodicity and mirror folds (IBS_GEO_FOLD=0 turns them off)
+    int tab_slots;          // axisymmetric tables: surfaces whose tables fit in shared memory at once (the mirror fold needs 2)
 };
 
 // ---- pack kernels: (ns, rows, mn) tables -> dense (m, n_idx) grid with the n-weights folded in -----------
@@ -213,9 +214,11 @@ __device__ __forceinline__ void geo_point_epilogue(const GeoParams& p, const Geo
 
 template <int NT1, int NT2>
 #if IBS_GEO_MINB > 1
-__global__ void __launch_bounds__(GeoThreads<NT1>::value, (NT1 > 0) ? IBS_GEO_MINB : 1)
+__global__ void __launch_bounds__(GeoThreads<NT1>::value, (NT1 > 0) ? IBS_GEO_MINB : 4)
 #else
-__global__ void __launch_bounds__(GeoThreads<NT1>::value)          // (a min-blocks argument of 1 lets ptxas take 254 registers: 3 instead of 4 CTAs / SM on the axisymmetric path)
+// The axisymmetric path asks for 4 CTAs / SM (without a minimum ptxas gives its mirror fold 148 registers: 3 CTAs / SM); the
+// 3-D paths ask for none (0): a min-blocks argument of 1 lets ptxas take 254 registers there
+__global__ void __launch_bounds__(GeoThreads<NT1>::value, (NT1 > 0) ? 0 : 4)
 #endif
 geometry_kernel(const GeoParams p) {
     constexpr int W1 = 2 * NT1 + 1, W2 = 2 * NT2 + 1, NT = (NT1 > NT2 ? NT1 : NT2);
@@ -227,6 +230,324 @@ geometry_kernel(const GeoParams p) {
     const int n_nyq = (NT2 > 0) ? p.M2 * (NT2 + 1) * ROWP_NYQ : p.M2 * W2 * ROW_NYQ;
     double* s_nyq = s_mn + n_mn;
     const int tid = threadIdx.x;
+    // Newton solve for theta_vmec at one point of the line and its 19 mode sums, from the tables at (t_mn, t_nyq)
+    auto point_sums = [&](const double* t_mn, double* t_nyq, double theta_p, double phi, double& th, int& nit, bool& ok) {
+        // cos/sin(k nfp phi), k = 0..NT
+        double cn[NT + 1], sn[NT + 1];
+        cn[0] = 1.0; sn[0] = 0.0;
+        if (NT > 0) {
+            sincos((double)p.nfp * phi, &sn[1], &cn[1]);
+#pragma unroll
+            for (int k = 2; k <= NT; ++k) {
+                cn[k] = fma(cn[k - 1], cn[1], -(sn[k - 1] * sn[1]));
+                sn[k] = fma(sn[k - 1], cn[1], cn[k - 1] * sn[1]);
+            }
+        }
+        // ---- Newton for theta_vmec:  th + sum_m [ sin(m th) A_m - cos(m th) B_m ] = theta_p
+        // A_m, B_m: per-thread columns of a shared-memory array [2 m + {0, 1}][thread] (conflict-free), or thread-local
+        // arrays when mpol is too large for that
+        double AmBm_local[NT1 > 0 ? 2 * MAX_M_NEWTON : 2];
+        const bool newton_smem = IBS_GEO_SMEM_NEWTON && NT1 > 0 && p.M1 <= GEO_SMEM_NEWTON_MAX_M;
+        double* const ab = newton_smem ? (t_nyq + n_nyq + tid) : AmBm_local;
+        const int abs_ = newton_smem ? GEO_THREADS : 1;
+#define Am(m) ab[(2 * (m)) * abs_]
+#define Bm(m) ab[(2 * (m) + 1) * abs_]
+        if (NT1 > 0) {
+            for (int m = 0; m < p.M1; ++m) {
+                const double* row = t_mn + (size_t)m * (NT1 + 1) * ROWP_MN + 12;      // (E, O) of the l row
+                double a = row[0], b = 0.0;
+#pragma unroll
+                for (int k = 1; k <= NT1; ++k) {
+                    const double2 eo = *reinterpret_cast<const double2*>(row + k * ROWP_MN);
+                    a = fma(eo.x, cn[k], a);
+                    b = fma(eo.y, sn[k], b);
+                }
+                Am(m) = a; Bm(m) = b;
+            }
+        }
+        th = theta_p;
+        nit = 0; ok = false;
+        double dprev = 1e300;
+        for (nit = 1; nit <= 25; ++nit) {
+            double s1, c1;
+            sincos(th, &s1, &c1);
+            double cm = 1.0, sm = 0.0, fsum = 0.0, dsum = 0.0;
+            if constexpr (NT1 == 0) {
+                // axisymmetric tables (n = 0 only): B_m = 0, no toroidal angle; 7 FP64 operations per mode
+                double dm = 0.0;
+                for (int m = 0; m < p.M1; ++m) {
+                    const double a = t_mn[(size_t)m * ROW_MN + 6];
+                    fsum = fma(sm, a, fsum);
+                    dsum = fma(dm * cm, a, dsum);
+                    const double cnx = fma(cm, c1, -(sm * s1));
+                    sm = fma(sm, c1, cm * s1);
+                    cm = cnx;
+                    dm += 1.0;
+                }
+            } else {
+                for (int m = 0; m < p.M1; ++m) {
+                    const double a = Am(m);
+                    const double b = Bm(m);
+                    fsum = fma(sm, a, fsum); fsum = fma(-cm, b, fsum);
+                    const double dm = (double)m;
+                    dsum = fma(dm * cm, a, dsum); dsum = fma(dm * sm, b, dsum);
+                    const double cnx = fma(cm, c1, -(sm * s1));
+                    sm = fma(sm, c1, cm * s1);
+                    cm = cnx;
+                }
+            }
+            const double res = (th + fsum) - theta_p;
+            const double dth = res / (1.0 + dsum);
+            th -= dth;
+            const double ad = fabs(dth), scale_th = fmax(1.0, fabs(th));
+            if (ad <= 4.5e-16 * scale_th) { ok = true; break; }
+            // quadratic convergence: the error left after this step is ~ ad^3 / dprev^2 -- no confirming iteration
+            // once that is below the rounding level
+            if (dprev < 1.0 && ad < 1e-3 * dprev) {           // (needs a previous correction, itself already small)
+                const double q = ad / dprev;
+                if (ad * q * q <= 2e-16 * scale_th) { ok = true; break; }
+            }
+            dprev = ad;
+        }
+#undef Am
+#undef Bm
+        // ---- mode sums (utils.py:420-468)
+        double s1, c1;
+        sincos(th, &s1, &c1);
+        double R = 0, R_s = 0, R_t = 0, R_p = 0, Z_s = 0, Z_t = 0, Z_p = 0, L_s = 0, L_t = 0, L_p = 0;
+        if (NT1 > 0) {
+            double cm = 1.0, sm = 0.0;
+            for (int m = 0; m < p.M1; ++m) {
+                const double* row = t_mn + (size_t)m * (NT1 + 1) * ROWP_MN;
+                double A[9], Bv[9];
+#pragma unroll
+                for (int j = 0; j < 9; ++j) { A[j] = row[2 * j]; Bv[j] = 0.0; }
+#if IBS_GEO_NROWS_DERIVED
+                // The n-weighted rows (n r, n z, n l) are never loaded: with v(-n) the coefficient of -n,
+                //   E_{n v} = k nfp (v(+n) - v(-n)) = k nfp O_v,   O_{n v} = k nfp E_v,
+                // so the pair (E_v, O_v) just loaded feeds FOUR FMAs.  The kernel is bound by the shared-memory data pipe
+                // (one wavefront per loaded double): 12 instead of 18 wavefronts per (m, k) here, 14 instead of 16 below.
+                A[1] = 0.0; A[4] = 0.0; A[7] = 0.0;
+#pragma unroll
+                for (int k = 1; k <= NT1; ++k) {
+                    const double kn = (double)k * (double)p.nfp;
+                    double kc = kn * cn[k], ks = kn * sn[k];
+#if IBS_GEO_KC_INLOOP
+                    asm volatile("" : "+d"(kc), "+d"(ks));       // (formed here, per m: hoisted they cost 4 NT1 registers)
+#endif
+#pragma unroll
+                    for (int j = 0; j < 9; ++j) {
+                        if (j == 1 || j == 4 || j == 7) continue;
+                        const double2 eo = *reinterpret_cast<const double2*>(row + k * ROWP_MN + 2 * j);
+                        A[j] = fma(eo.x, cn[k], A[j]);
+                        Bv[j] = fma(eo.y, sn[k], Bv[j]);
+                        if (j == 0 || j == 3 || j == 6) {
+                            A[j + 1] = fma(eo.y, kc, A[j + 1]);
+                            Bv[j + 1] = fma(eo.x, ks, Bv[j + 1]);
+                        }
+                    }
+                }
+#else
+#pragma unroll
+                for (int k = 1; k <= NT1; ++k) {
+#pragma unroll
+                    for (int j = 0; j < 9; ++j) {
+                        const double2 eo = *reinterpret_cast<const double2*>(row + k * ROWP_MN + 2 * j);
+                        A[j] = fma(eo.x, cn[k], A[j]);
+                        Bv[j] = fma(eo.y, sn[k], Bv[j]);
+                    }
+                }
+#endif
+                // rows: 0 r, 1 n r, 2 r_s, 3 z, 4 n z, 5 z_s, 6 l, 7 n l, 8 l_s
+                const double dm = (double)m;
+                R += fma(cm, A[0], sm * Bv[0]);
+                R_t = fma(-dm, fma(sm, A[0], -(cm * Bv[0])), R_t);
+                R_p += fma(sm, A[1], -(cm * Bv[1]));
+                R_s += fma(cm, A[2], sm * Bv[2]);
+                Z_t = fma(dm, fma(cm, A[3], sm * Bv[3]), Z_t);
+                Z_p -= fma(cm, A[4], sm * Bv[4]);
+                Z_s += fma(sm, A[5], -(cm * Bv[5]));
+                L_t = fma(dm, fma(cm, A[6], sm * Bv[6]), L_t);
+                L_p -= fma(cm, A[7], sm * Bv[7]);
+                L_s += fma(sm, A[8], -(cm * Bv[8]));
+                const double cnx = fma(cm, c1, -(sm * s1));
+                sm = fma(sm, c1, cm * s1);
+                cm = cnx;
+            }
+        } else if constexpr (NT1 == 0) {
+            // axisymmetric tables: one entry (n = 0) per m, the angle is m theta itself and the n-weighted sums
+            // (d/dphi) vanish: 10 FP64 operations per mode + the recurrence
+            double cm = 1.0, sm = 0.0, dm = 0.0;
+            for (int m = 0; m < p.M1; ++m) {
+                const double* row = t_mn + (size_t)m * ROW_MN;
+                const double2 v0 = *reinterpret_cast<const double2*>(row + 0);   // r, n r (= 0)
+                const double2 v1 = *reinterpret_cast<const double2*>(row + 2);   // r_s, z
+                const double2 v2 = *reinterpret_cast<const double2*>(row + 4);   // n z (= 0), z_s
+                const double2 v3 = *reinterpret_cast<const double2*>(row + 6);   // l, n l (= 0)
+                const double v4 = row[8];                                          // l_s
+                const double msm = dm * sm, mcm = dm * cm;
+                R = fma(v0.x, cm, R);
+                R_t = fma(-v0.x, msm, R_t);
+                R_s = fma(v1.x, cm, R_s);
+                Z_t = fma(v1.y, mcm, Z_t);
+                Z_s = fma(v2.y, sm, Z_s);
+                L_t = fma(v3.x, mcm, L_t);
+                L_s = fma(v4, sm, L_s);
+                const double cnx = fma(cm, c1, -(sm * s1));
+                sm = fma(sm, c1, cm * s1);
+                cm = cnx;
+                dm += 1.0;
+            }
+        } else {
+            double cm = 1.0, sm = 0.0;
+            for (int m = 0; m < p.M1; ++m) {
+                const double* row = t_mn + (size_t)m * W1 * ROW_MN;
+                double a0 = 0, a1 = 0, a2 = 0, a3 = 0, a4 = 0, a5 = 0, a6 = 0, a7 = 0, a8 = 0, a9 = 0;
+#pragma unroll
+                for (int q = 0; q < W1; ++q) {
+                    const int k = q - NT1, ak = k < 0 ? -k : k;
+                    double ca, sa;
+                    if (k >= 0) angle<1>(cm, sm, cn[ak], sn[ak], ca, sa);
+                    else angle<-1>(cm, sm, cn[ak], sn[ak], ca, sa);
+                    const double2 v0 = *reinterpret_cast<const double2*>(row + q * ROW_MN + 0);   // r, n r
+                    const double2 v1 = *reinterpret_cast<const double2*>(row + q * ROW_MN + 2);   // r_s, z
+                    const double2 v2 = *reinterpret_cast<const double2*>(row + q * ROW_MN + 4);   // n z, z_s
+                    const double2 v3 = *reinterpret_cast<const double2*>(row + q * ROW_MN + 6);   // l, n l
+                    const double v4 = row[q * ROW_MN + 8];                                          // l_s
+                    a0 = fma(v0.x, ca, a0);   // sum r cos
+                    a1 = fma(v0.x, sa, a1);   // sum r sin
+                    a2 = fma(v0.y, sa, a2);   // sum n r sin
+                    a3 = fma(v1.x, ca, a3);   // sum r_s cos
+                    a4 = fma(v1.y, ca, a4);   // sum z cos
+                    a5 = fma(v2.x, ca, a5);   // sum n z cos
+                    a6 = fma(v2.y, sa, a6);   // sum z_s sin
+                    a7 = fma(v3.x, ca, a7);   // sum l cos
+                    a8 = fma(v3.y, ca, a8);   // sum n l cos
+                    a9 = fma(v4, sa, a9);     // sum l_s sin
+                }
+                const double dm = (double)m;
+                R += a0; R_t = fma(-dm, a1, R_t); R_p += a2; R_s += a3;
+                Z_t = fma(dm, a4, Z_t); Z_p -= a5; Z_s += a6;
+                L_t = fma(dm, a7, L_t); L_p -= a8; L_s += a9;
+                const double cnx = fma(cm, c1, -(sm * s1));
+                sm = fma(sm, c1, cm * s1);
+                cm = cnx;
+            }
+        }
+        double sqrtg = 0, B = 0, B_s = 0, B_t = 0, B_p = 0, Bsup_p = 0, Bsub_s = 0, Bsub_t = 0, Bsub_p = 0;
+        if (NT2 > 0) {
+            double cm = 1.0, sm = 0.0;
+            for (int m = 0; m < p.M2; ++m) {
+                const double* row = t_nyq + (size_t)m * (NT2 + 1) * ROWP_NYQ;
+                double A[8], Bv[8];
+#pragma unroll
+                for (int j = 0; j < 8; ++j) { A[j] = row[2 * j]; Bv[j] = 0.0; }
+#if IBS_GEO_NROWS_DERIVED
+                A[2] = 0.0;                           // (n b) from (b): see the (R, Z, lambda) set above
+#pragma unroll
+                for (int k = 1; k <= NT2; ++k) {
+                    const double kn = (double)k * (double)p.nfp;
+                    double kc = kn * cn[k], ks = kn * sn[k];
+#if IBS_GEO_KC_INLOOP
+                    asm volatile("" : "+d"(kc), "+d"(ks));
+#endif
+#pragma unroll
+                    for (int j = 0; j < 8; ++j) {
+                        if (j == 2) continue;
+                        const double2 eo = *reinterpret_cast<const double2*>(row + k * ROWP_NYQ + 2 * j);
+                        A[j] = fma(eo.x, cn[k], A[j]);
+                        Bv[j] = fma(eo.y, sn[k], Bv[j]);
+                        if (j == 1) {
+                            A[2] = fma(eo.y, kc, A[2]);
+                            Bv[2] = fma(eo.x, ks, Bv[2]);
+                        }
+                    }
+                }
+#else
+#pragma unroll
+                for (int k = 1; k <= NT2; ++k) {
+#pragma unroll
+                    for (int j = 0; j < 8; ++j) {
+                        const double2 eo = *reinterpret_cast<const double2*>(row + k * ROWP_NYQ + 2 * j);
+                        A[j] = fma(eo.x, cn[k], A[j]);
+                        Bv[j] = fma(eo.y, sn[k], Bv[j]);
+                    }
+                }
+#endif
+                // rows: 0 g, 1 b, 2 n b, 3 b_s, 4 bsupv, 5 bsubs, 6 bsubu, 7 bsubv
+                const double dm = (double)m;
+                sqrtg += fma(cm, A[0], sm * Bv[0]);
+                B += fma(cm, A[1], sm * Bv[1]);
+                B_t = fma(-dm, fma(sm, A[1], -(cm * Bv[1])), B_t);
+                B_p += fma(sm, A[2], -(cm * Bv[2]));
+                B_s += fma(cm, A[3], sm * Bv[3]);
+                Bsup_p += fma(cm, A[4], sm * Bv[4]);
+                Bsub_s += fma(sm, A[5], -(cm * Bv[5]));
+                Bsub_t += fma(cm, A[6], sm * Bv[6]);
+                Bsub_p += fma(cm, A[7], sm * Bv[7]);
+                const double cnx = fma(cm, c1, -(sm * s1));
+                sm = fma(sm, c1, cm * s1);
+                cm = cnx;
+            }
+        } else if constexpr (NT2 == 0) {
+            double cm = 1.0, sm = 0.0, dm = 0.0;
+            for (int m = 0; m < p.M2; ++m) {
+                const double* row = t_nyq + (size_t)m * ROW_NYQ;
+                const double2 v0 = *reinterpret_cast<const double2*>(row + 0);  // g, b
+                const double2 v1 = *reinterpret_cast<const double2*>(row + 2);  // n b (= 0), b_s
+                const double2 v2 = *reinterpret_cast<const double2*>(row + 4);  // bsupv, bsubs
+                const double2 v3 = *reinterpret_cast<const double2*>(row + 6);  // bsubu, bsubv
+                sqrtg = fma(v0.x, cm, sqrtg);
+                B = fma(v0.y, cm, B);
+                B_t = fma(-v0.y, dm * sm, B_t);
+                B_s = fma(v1.y, cm, B_s);
+                Bsup_p = fma(v2.x, cm, Bsup_p);
+                Bsub_s = fma(v2.y, sm, Bsub_s);
+                Bsub_t = fma(v3.x, cm, Bsub_t);
+                Bsub_p = fma(v3.y, cm, Bsub_p);
+                const double cnx = fma(cm, c1, -(sm * s1));
+                sm = fma(sm, c1, cm * s1);
+                cm = cnx;
+                dm += 1.0;
+            }
+        } else {
+            double cm = 1.0, sm = 0.0;
+            for (int m = 0; m < p.M2; ++m) {
+                const double* row = t_nyq + (size_t)m * W2 * ROW_NYQ;
+                double a0 = 0, a1 = 0, a2 = 0, a3 = 0, a4 = 0, a5 = 0, a6 = 0, a7 = 0, a8 = 0;
+#pragma unroll
+                for (int q = 0; q < W2; ++q) {
+                    const int k = q - NT2, ak = k < 0 ? -k : k;
+                    double ca, sa;
+                    if (k >= 0) angle<1>(cm, sm, cn[ak], sn[ak], ca, sa);
+                    else angle<-1>(cm, sm, cn[ak], sn[ak], ca, sa);
+                    const double2 v0 = *reinterpret_cast<const double2*>(row + q * ROW_NYQ + 0);  // g, b
+                    const double2 v1 = *reinterpret_cast<const double2*>(row + q * ROW_NYQ + 2);  // n b, b_s
+                    const double2 v2 = *reinterpret_cast<const double2*>(row + q * ROW_NYQ + 4);  // bsupv, bsubs
+                    const double2 v3 = *reinterpret_cast<const double2*>(row + q * ROW_NYQ + 6);  // bsubu, bsubv
+                    a0 = fma(v0.x, ca, a0);   // sqrt g
+                    a1 = fma(v0.y, ca, a1);   // B
+                    a2 = fma(v0.y, sa, a2);   // sum b sin
+                    a3 = fma(v1.x, sa, a3);   // sum n b sin
+                    a4 = fma(v1.y, ca, a4);   // dB/ds
+                    a5 = fma(v2.x, ca, a5);   // B^phi
+                    a6 = fma(v2.y, sa, a6);   // B_s
+                    a7 = fma(v3.x, ca, a7);   // B_theta
+                    a8 = fma(v3.y, ca, a8);   // B_phi
+                }
+                const double dm = (double)m;
+                sqrtg += a0; B += a1; B_t = fma(-dm, a2, B_t); B_p += a3; B_s += a4;
+                Bsup_p += a5; Bsub_s += a6; Bsub_t += a7; Bsub_p += a8;
+                const double cnx = fma(cm, c1, -(sm * s1));
+                sm = fma(sm, c1, cm * s1);
+                cm = cnx;
+            }
+        }
+        GeoSums g;
+        g.R = R; g.R_s = R_s; g.R_t = R_t; g.R_p = R_p; g.Z_s = Z_s; g.Z_t = Z_t; g.Z_p = Z_p; g.L_s = L_s; g.L_t = L_t; g.L_p = L_p;
+        g.sqrtg = sqrtg; g.B = B; g.B_s = B_s; g.B_t = B_t; g.B_p = B_p; g.Bsup_p = Bsup_p; g.Bsub_s = Bsub_s; g.Bsub_t = Bsub_t; g.Bsub_p = Bsub_p;
+        return g;
+    };
     // Periodicity fold (axisymmetric tables only).  Every mode sum is 2 pi-periodic in theta_vmec and does not depend on phi,
     // and theta_vmec(theta_pest + 2 pi) = theta_vmec(theta_pest) + 2 pi, so grid points one poloidal turn apart share their
     // Newton solve and their 19 sums; only the pointwise epilogue (secular shear term, phi) is per point.  The reference's
@@ -254,6 +575,96 @@ geometry_kernel(const GeoParams p) {
     unsigned parity = 0;
     if (tid == 0) { mbar_init(bar, 1); asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory"); }
     __syncthreads();
+
+    if constexpr (NT1 == 0 && NT2 == 0) {
+        // Mirror fold (on top of the periodicity fold).  The tables are stellarator-symmetric, so with n = 0 theta_vmec is odd
+        // in theta_pest and every mode sum is even (cos series) or odd (sin series: R_t, Z_s, lambda_s, B_t, B_s) in
+        // theta_vmec.  When theta[r] + theta[(c - r) mod P] = 2 pi k for every residue r (a grid symmetric about theta = 0
+        // modulo one turn), residues r and (c - r) mod P share one Newton solve and one set of sums: at every point j of
+        // the mirror residue theta_vmec = (theta[j] + theta[r]) - theta_vmec(theta[r]), and the odd sums change sign.
+        // c comes from theta[0] and h and is used only if EVERY residue pair satisfies the relation to 2e-12.
+        int C = -1;
+        if (P < p.nl && p.tab_slots >= 2) {
+            const double TWO_PI = 6.283185307179586;
+            double cr = -2.0 * p.theta[0] / (p.theta[1] - p.theta[0]);
+            cr -= (double)P * floor(cr / (double)P);
+            int cc = (int)rint(cr);
+            if (cc == P) cc = 0;
+            bool okm = cc >= 0 && cc < P;
+            for (int r = tid; okm && r < P; r += GEO_THREADS) {
+                const double x = p.theta[r] + p.theta[cc >= r ? cc - r : cc - r + P];
+                okm = fabs(x - TWO_PI * rint(x / TWO_PI)) <= 2e-12;
+            }
+            if (__syncthreads_and(okm)) C = cc;
+        }
+        if (C >= 0) {
+            // Work = (surface, alpha, orbit) units flattened, orbit o standing for residue r = o (o <= c / 2) or
+            // r = o + c - c / 2 (r up to (c + P) / 2) and its mirror (c - r) mod P.  Every CTA takes one contiguous,
+            // equally sized range of units and runs it in chunks of GEO_THREADS units across surface boundaries, so that
+            // no tile is left partly empty at the end of a surface.  A chunk ends at the latest at the second surface
+            // boundary (which shortens chunks only when a surface has fewer units than a chunk); surface js is staged in
+            // table slot js & 1.
+            const int hc = C >> 1, orbits = hc + 1 + ((C + P) >> 1) - C;
+            const long long U = (long long)p.nalpha * orbits, Wu = (long long)p.ns * U;
+            const long long u_begin = Wu * blockIdx.x / gridDim.x, u_end = Wu * (blockIdx.x + 1) / gridDim.x;
+            const int n_tab = n_mn + n_nyq;
+            int staged[2] = {-1, -1};
+            for (long long u0 = u_begin; u0 < u_end;) {
+                const int js0 = (int)(u0 / U);
+                const long long u1 = min(min(u0 + GEO_THREADS, u_end), (long long)(js0 + 2) * U);
+                const int js1 = (int)((u1 - 1) / U);
+                const bool need0 = staged[js0 & 1] != js0, need1 = js1 != js0 && staged[js1 & 1] != js1;
+                if (need0 || need1) {
+                    __syncthreads();                       // everyone is done with the slots' previous tables
+                    if (tid == 0) {
+                        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+                        mbar_expect_tx(bar, (unsigned)((need0 + need1) * n_tab * sizeof(double)));
+                        for (int k = 0; k < 2; ++k) {
+                            const int jk = k ? js1 : js0;
+                            if (!(k ? need1 : need0)) continue;
+                            double* t = s_mn + (size_t)(jk & 1) * n_tab;
+                            tma_bulk_g2s(t, p.pk_mn + (size_t)jk * n_mn, (unsigned)(n_mn * sizeof(double)), bar);
+                            tma_bulk_g2s(t + n_mn, p.pk_nyq + (size_t)jk * n_nyq, (unsigned)(n_nyq * sizeof(double)), bar);
+                        }
+                    }
+                    if (need0) staged[js0 & 1] = js0;
+                    if (need1) staged[js1 & 1] = js1;
+                    mbar_wait(bar, parity);
+                    parity ^= 1;
+                }
+                const long long u = u0 + tid;
+                u0 = u1;
+                if (u >= u1) continue;
+                const int js = (int)(u / U);
+                const int rem = (int)(u - (long long)js * U);
+                const int ja = rem / orbits, o = rem - ja * orbits;
+                const int r = (o <= hc) ? o : o + C - hc;
+                const int rm = (C >= r) ? C - r : C - r + P;
+                double* t_mn = s_mn + (size_t)(js & 1) * n_tab;
+                const double* sc = p.scal + (size_t)js * IBS_NSCAL;
+                const double s_val = sc[0], iota = sc[1], d_iota = sc[2], dpds = sc[3], shat = sc[4];
+                const double al = p.alpha_per_surface ? p.alpha[(size_t)js * p.nalpha + ja] : p.alpha[ja];
+                const double theta_p = p.theta[r];
+                double th; int nit; bool ok;
+                const GeoSums g = point_sums(t_mn, t_mn + n_mn, theta_p, p.phi_center + (theta_p - al) / iota, th, nit, ok);
+                for (int jf = r; jf < p.nl; jf += P) {
+                    const double tp = p.theta[jf];
+                    geo_point_epilogue(p, g, js, ja, jf, p.phi_center + (tp - al) / iota, th + (tp - theta_p), nit, ok, s_val, iota, d_iota,
+                                       dpds, shat);
+                }
+                if (rm != r) {
+                    GeoSums gm = g;
+                    gm.R_t = -g.R_t; gm.Z_s = -g.Z_s; gm.L_s = -g.L_s; gm.B_t = -g.B_t; gm.Bsub_s = -g.Bsub_s;
+                    for (int jf = rm; jf < p.nl; jf += P) {
+                        const double tp = p.theta[jf];
+                        geo_point_epilogue(p, gm, js, ja, jf, p.phi_center + (tp - al) / iota, (tp + theta_p) - th, nit, ok, s_val, iota,
+                                           d_iota, dpds, shat);
+                    }
+                }
+            }
+            return;
+        }
+    }
 
     // Work = (surface, tile) pairs flattened; every CTA takes one contiguous, equally sized range of them (perfect
     // balance, no tail wave) and re-stages the tables only when its range crosses into the next surface.
@@ -286,321 +697,8 @@ geometry_kernel(const GeoParams p) {
             const double al = p.alpha_per_surface ? p.alpha[(size_t)js * p.nalpha + ja] : p.alpha[ja];
             const double theta_p = p.theta[jl];
             const double phi = p.phi_center + (theta_p - al) / iota;            // utils.py:373
-
-            // cos/sin(k nfp phi), k = 0..NT
-            double cn[NT + 1], sn[NT + 1];
-            cn[0] = 1.0; sn[0] = 0.0;
-            if (NT > 0) {
-                sincos((double)p.nfp * phi, &sn[1], &cn[1]);
-#pragma unroll
-                for (int k = 2; k <= NT; ++k) {
-                    cn[k] = fma(cn[k - 1], cn[1], -(sn[k - 1] * sn[1]));
-                    sn[k] = fma(sn[k - 1], cn[1], cn[k - 1] * sn[1]);
-                }
-            }
-            // ---- Newton for theta_vmec:  th + sum_m [ sin(m th) A_m - cos(m th) B_m ] = theta_p
-            // A_m, B_m: per-thread columns of a shared-memory array [2 m + {0, 1}][thread] (conflict-free), or thread-local
-            // arrays when mpol is too large for that
-            double AmBm_local[NT1 > 0 ? 2 * MAX_M_NEWTON : 2];
-            const bool newton_smem = IBS_GEO_SMEM_NEWTON && NT1 > 0 && p.M1 <= GEO_SMEM_NEWTON_MAX_M;
-            double* const ab = newton_smem ? (s_nyq + n_nyq + tid) : AmBm_local;
-            const int abs_ = newton_smem ? GEO_THREADS : 1;
-#define Am(m) ab[(2 * (m)) * abs_]
-#define Bm(m) ab[(2 * (m) + 1) * abs_]
-            if (NT1 > 0) {
-                for (int m = 0; m < p.M1; ++m) {
-                    const double* row = s_mn + (size_t)m * (NT1 + 1) * ROWP_MN + 12;      // (E, O) of the l row
-                    double a = row[0], b = 0.0;
-#pragma unroll
-                    for (int k = 1; k <= NT1; ++k) {
-                        const double2 eo = *reinterpret_cast<const double2*>(row + k * ROWP_MN);
-                        a = fma(eo.x, cn[k], a);
-                        b = fma(eo.y, sn[k], b);
-                    }
-                    Am(m) = a; Bm(m) = b;
-                }
-            }
-            double th = theta_p;
-            int nit = 0; bool ok = false;
-            double dprev = 1e300;
-            for (nit = 1; nit <= 25; ++nit) {
-                double s1, c1;
-                sincos(th, &s1, &c1);
-                double cm = 1.0, sm = 0.0, fsum = 0.0, dsum = 0.0;
-                if constexpr (NT1 == 0) {
-                    // axisymmetric tables (n = 0 only): B_m = 0, no toroidal angle; 7 FP64 operations per mode
-                    double dm = 0.0;
-                    for (int m = 0; m < p.M1; ++m) {
-                        const double a = s_mn[(size_t)m * ROW_MN + 6];
-                        fsum = fma(sm, a, fsum);
-                        dsum = fma(dm * cm, a, dsum);
-                        const double cnx = fma(cm, c1, -(sm * s1));
-                        sm = fma(sm, c1, cm * s1);
-                        cm = cnx;
-                        dm += 1.0;
-                    }
-                } else {
-                    for (int m = 0; m < p.M1; ++m) {
-                        const double a = Am(m);
-                        const double b = Bm(m);
-                        fsum = fma(sm, a, fsum); fsum = fma(-cm, b, fsum);
-                        const double dm = (double)m;
-                        dsum = fma(dm * cm, a, dsum); dsum = fma(dm * sm, b, dsum);
-                        const double cnx = fma(cm, c1, -(sm * s1));
-                        sm = fma(sm, c1, cm * s1);
-                        cm = cnx;
-                    }
-                }
-                const double res = (th + fsum) - theta_p;
-                const double dth = res / (1.0 + dsum);
-                th -= dth;
-                const double ad = fabs(dth), scale_th = fmax(1.0, fabs(th));
-                if (ad <= 4.5e-16 * scale_th) { ok = true; break; }
-                // quadratic convergence: the error left after this step is ~ ad^3 / dprev^2 -- no confirming iteration
-                // once that is below the rounding level
-                if (dprev < 1.0 && ad < 1e-3 * dprev) {           // (needs a previous correction, itself already small)
-                    const double q = ad / dprev;
-                    if (ad * q * q <= 2e-16 * scale_th) { ok = true; break; }
-                }
-                dprev = ad;
-            }
-#undef Am
-#undef Bm
-            // ---- mode sums (utils.py:420-468)
-            double s1, c1;
-            sincos(th, &s1, &c1);
-            double R = 0, R_s = 0, R_t = 0, R_p = 0, Z_s = 0, Z_t = 0, Z_p = 0, L_s = 0, L_t = 0, L_p = 0;
-            if (NT1 > 0) {
-                double cm = 1.0, sm = 0.0;
-                for (int m = 0; m < p.M1; ++m) {
-                    const double* row = s_mn + (size_t)m * (NT1 + 1) * ROWP_MN;
-                    double A[9], Bv[9];
-#pragma unroll
-                    for (int j = 0; j < 9; ++j) { A[j] = row[2 * j]; Bv[j] = 0.0; }
-#if IBS_GEO_NROWS_DERIVED
-                    // The n-weighted rows (n r, n z, n l) are never loaded: with v(-n) the coefficient of -n,
-                    //   E_{n v} = k nfp (v(+n) - v(-n)) = k nfp O_v,   O_{n v} = k nfp E_v,
-                    // so the pair (E_v, O_v) just loaded feeds FOUR FMAs.  The kernel is bound by the shared-memory data pipe
-                    // (one wavefront per loaded double): 12 instead of 18 wavefronts per (m, k) here, 14 instead of 16 below.
-                    A[1] = 0.0; A[4] = 0.0; A[7] = 0.0;
-#pragma unroll
-                    for (int k = 1; k <= NT1; ++k) {
-                        const double kn = (double)k * (double)p.nfp;
-                        double kc = kn * cn[k], ks = kn * sn[k];
-#if IBS_GEO_KC_INLOOP
-                        asm volatile("" : "+d"(kc), "+d"(ks));       // (formed here, per m: hoisted they cost 4 NT1 registers)
-#endif
-#pragma unroll
-                        for (int j = 0; j < 9; ++j) {
-                            if (j == 1 || j == 4 || j == 7) continue;
-                            const double2 eo = *reinterpret_cast<const double2*>(row + k * ROWP_MN + 2 * j);
-                            A[j] = fma(eo.x, cn[k], A[j]);
-                            Bv[j] = fma(eo.y, sn[k], Bv[j]);
-                            if (j == 0 || j == 3 || j == 6) {
-                                A[j + 1] = fma(eo.y, kc, A[j + 1]);
-                                Bv[j + 1] = fma(eo.x, ks, Bv[j + 1]);
-                            }
-                        }
-                    }
-#else
-#pragma unroll
-                    for (int k = 1; k <= NT1; ++k) {
-#pragma unroll
-                        for (int j = 0; j < 9; ++j) {
-                            const double2 eo = *reinterpret_cast<const double2*>(row + k * ROWP_MN + 2 * j);
-                            A[j] = fma(eo.x, cn[k], A[j]);
-                            Bv[j] = fma(eo.y, sn[k], Bv[j]);
-                        }
-                    }
-#endif
-                    // rows: 0 r, 1 n r, 2 r_s, 3 z, 4 n z, 5 z_s, 6 l, 7 n l, 8 l_s
-                    const double dm = (double)m;
-                    R += fma(cm, A[0], sm * Bv[0]);
-                    R_t = fma(-dm, fma(sm, A[0], -(cm * Bv[0])), R_t);
-                    R_p += fma(sm, A[1], -(cm * Bv[1]));
-                    R_s += fma(cm, A[2], sm * Bv[2]);
-                    Z_t = fma(dm, fma(cm, A[3], sm * Bv[3]), Z_t);
-                    Z_p -= fma(cm, A[4], sm * Bv[4]);
-                    Z_s += fma(sm, A[5], -(cm * Bv[5]));
-                    L_t = fma(dm, fma(cm, A[6], sm * Bv[6]), L_t);
-                    L_p -= fma(cm, A[7], sm * Bv[7]);
-                    L_s += fma(sm, A[8], -(cm * Bv[8]));
-                    const double cnx = fma(cm, c1, -(sm * s1));
-                    sm = fma(sm, c1, cm * s1);
-                    cm = cnx;
-                }
-            } else if constexpr (NT1 == 0) {
-                // axisymmetric tables: one entry (n = 0) per m, the angle is m theta itself and the n-weighted sums
-                // (d/dphi) vanish: 10 FP64 operations per mode + the recurrence
-                double cm = 1.0, sm = 0.0, dm = 0.0;
-                for (int m = 0; m < p.M1; ++m) {
-                    const double* row = s_mn + (size_t)m * ROW_MN;
-                    const double2 v0 = *reinterpret_cast<const double2*>(row + 0);   // r, n r (= 0)
-                    const double2 v1 = *reinterpret_cast<const double2*>(row + 2);   // r_s, z
-                    const double2 v2 = *reinterpret_cast<const double2*>(row + 4);   // n z (= 0), z_s
-                    const double2 v3 = *reinterpret_cast<const double2*>(row + 6);   // l, n l (= 0)
-                    const double v4 = row[8];                                          // l_s
-                    const double msm = dm * sm, mcm = dm * cm;
-                    R = fma(v0.x, cm, R);
-                    R_t = fma(-v0.x, msm, R_t);
-                    R_s = fma(v1.x, cm, R_s);
-                    Z_t = fma(v1.y, mcm, Z_t);
-                    Z_s = fma(v2.y, sm, Z_s);
-                    L_t = fma(v3.x, mcm, L_t);
-                    L_s = fma(v4, sm, L_s);
-                    const double cnx = fma(cm, c1, -(sm * s1));
-                    sm = fma(sm, c1, cm * s1);
-                    cm = cnx;
-                    dm += 1.0;
-                }
-            } else {
-                double cm = 1.0, sm = 0.0;
-                for (int m = 0; m < p.M1; ++m) {
-                    const double* row = s_mn + (size_t)m * W1 * ROW_MN;
-                    double a0 = 0, a1 = 0, a2 = 0, a3 = 0, a4 = 0, a5 = 0, a6 = 0, a7 = 0, a8 = 0, a9 = 0;
-#pragma unroll
-                    for (int q = 0; q < W1; ++q) {
-                        const int k = q - NT1, ak = k < 0 ? -k : k;
-                        double ca, sa;
-                        if (k >= 0) angle<1>(cm, sm, cn[ak], sn[ak], ca, sa);
-                        else angle<-1>(cm, sm, cn[ak], sn[ak], ca, sa);
-                        const double2 v0 = *reinterpret_cast<const double2*>(row + q * ROW_MN + 0);   // r, n r
-                        const double2 v1 = *reinterpret_cast<const double2*>(row + q * ROW_MN + 2);   // r_s, z
-                        const double2 v2 = *reinterpret_cast<const double2*>(row + q * ROW_MN + 4);   // n z, z_s
-                        const double2 v3 = *reinterpret_cast<const double2*>(row + q * ROW_MN + 6);   // l, n l
-                        const double v4 = row[q * ROW_MN + 8];                                          // l_s
-                        a0 = fma(v0.x, ca, a0);   // sum r cos
-                        a1 = fma(v0.x, sa, a1);   // sum r sin
-                        a2 = fma(v0.y, sa, a2);   // sum n r sin
-                        a3 = fma(v1.x, ca, a3);   // sum r_s cos
-                        a4 = fma(v1.y, ca, a4);   // sum z cos
-                        a5 = fma(v2.x, ca, a5);   // sum n z cos
-                        a6 = fma(v2.y, sa, a6);   // sum z_s sin
-                        a7 = fma(v3.x, ca, a7);   // sum l cos
-                        a8 = fma(v3.y, ca, a8);   // sum n l cos
-                        a9 = fma(v4, sa, a9);     // sum l_s sin
-                    }
-                    const double dm = (double)m;
-                    R += a0; R_t = fma(-dm, a1, R_t); R_p += a2; R_s += a3;
-                    Z_t = fma(dm, a4, Z_t); Z_p -= a5; Z_s += a6;
-                    L_t = fma(dm, a7, L_t); L_p -= a8; L_s += a9;
-                    const double cnx = fma(cm, c1, -(sm * s1));
-                    sm = fma(sm, c1, cm * s1);
-                    cm = cnx;
-                }
-            }
-            double sqrtg = 0, B = 0, B_s = 0, B_t = 0, B_p = 0, Bsup_p = 0, Bsub_s = 0, Bsub_t = 0, Bsub_p = 0;
-            if (NT2 > 0) {
-                double cm = 1.0, sm = 0.0;
-                for (int m = 0; m < p.M2; ++m) {
-                    const double* row = s_nyq + (size_t)m * (NT2 + 1) * ROWP_NYQ;
-                    double A[8], Bv[8];
-#pragma unroll
-                    for (int j = 0; j < 8; ++j) { A[j] = row[2 * j]; Bv[j] = 0.0; }
-#if IBS_GEO_NROWS_DERIVED
-                    A[2] = 0.0;                           // (n b) from (b): see the (R, Z, lambda) set above
-#pragma unroll
-                    for (int k = 1; k <= NT2; ++k) {
-                        const double kn = (double)k * (double)p.nfp;
-                        double kc = kn * cn[k], ks = kn * sn[k];
-#if IBS_GEO_KC_INLOOP
-                        asm volatile("" : "+d"(kc), "+d"(ks));
-#endif
-#pragma unroll
-                        for (int j = 0; j < 8; ++j) {
-                            if (j == 2) continue;
-                            const double2 eo = *reinterpret_cast<const double2*>(row + k * ROWP_NYQ + 2 * j);
-                            A[j] = fma(eo.x, cn[k], A[j]);
-                            Bv[j] = fma(eo.y, sn[k], Bv[j]);
-                            if (j == 1) {
-                                A[2] = fma(eo.y, kc, A[2]);
-                                Bv[2] = fma(eo.x, ks, Bv[2]);
-                            }
-                        }
-                    }
-#else
-#pragma unroll
-                    for (int k = 1; k <= NT2; ++k) {
-#pragma unroll
-                        for (int j = 0; j < 8; ++j) {
-                            const double2 eo = *reinterpret_cast<const double2*>(row + k * ROWP_NYQ + 2 * j);
-                            A[j] = fma(eo.x, cn[k], A[j]);
-                            Bv[j] = fma(eo.y, sn[k], Bv[j]);
-                        }
-                    }
-#endif
-                    // rows: 0 g, 1 b, 2 n b, 3 b_s, 4 bsupv, 5 bsubs, 6 bsubu, 7 bsubv
-                    const double dm = (double)m;
-                    sqrtg += fma(cm, A[0], sm * Bv[0]);
-                    B += fma(cm, A[1], sm * Bv[1]);
-                    B_t = fma(-dm, fma(sm, A[1], -(cm * Bv[1])), B_t);
-                    B_p += fma(sm, A[2], -(cm * Bv[2]));
-                    B_s += fma(cm, A[3], sm * Bv[3]);
-                    Bsup_p += fma(cm, A[4], sm * Bv[4]);
-                    Bsub_s += fma(sm, A[5], -(cm * Bv[5]));
-                    Bsub_t += fma(cm, A[6], sm * Bv[6]);
-                    Bsub_p += fma(cm, A[7], sm * Bv[7]);
-                    const double cnx = fma(cm, c1, -(sm * s1));
-                    sm = fma(sm, c1, cm * s1);
-                    cm = cnx;
-                }
-            } else if constexpr (NT2 == 0) {
-                double cm = 1.0, sm = 0.0, dm = 0.0;
-                for (int m = 0; m < p.M2; ++m) {
-                    const double* row = s_nyq + (size_t)m * ROW_NYQ;
-                    const double2 v0 = *reinterpret_cast<const double2*>(row + 0);  // g, b
-                    const double2 v1 = *reinterpret_cast<const double2*>(row + 2);  // n b (= 0), b_s
-                    const double2 v2 = *reinterpret_cast<const double2*>(row + 4);  // bsupv, bsubs
-                    const double2 v3 = *reinterpret_cast<const double2*>(row + 6);  // bsubu, bsubv
-                    sqrtg = fma(v0.x, cm, sqrtg);
-                    B = fma(v0.y, cm, B);
-                    B_t = fma(-v0.y, dm * sm, B_t);
-                    B_s = fma(v1.y, cm, B_s);
-                    Bsup_p = fma(v2.x, cm, Bsup_p);
-                    Bsub_s = fma(v2.y, sm, Bsub_s);
-                    Bsub_t = fma(v3.x, cm, Bsub_t);
-                    Bsub_p = fma(v3.y, cm, Bsub_p);
-                    const double cnx = fma(cm, c1, -(sm * s1));
-                    sm = fma(sm, c1, cm * s1);
-                    cm = cnx;
-                    dm += 1.0;
-                }
-            } else {
-                double cm = 1.0, sm = 0.0;
-                for (int m = 0; m < p.M2; ++m) {
-                    const double* row = s_nyq + (size_t)m * W2 * ROW_NYQ;
-                    double a0 = 0, a1 = 0, a2 = 0, a3 = 0, a4 = 0, a5 = 0, a6 = 0, a7 = 0, a8 = 0;
-#pragma unroll
-                    for (int q = 0; q < W2; ++q) {
-                        const int k = q - NT2, ak = k < 0 ? -k : k;
-                        double ca, sa;
-                        if (k >= 0) angle<1>(cm, sm, cn[ak], sn[ak], ca, sa);
-                        else angle<-1>(cm, sm, cn[ak], sn[ak], ca, sa);
-                        const double2 v0 = *reinterpret_cast<const double2*>(row + q * ROW_NYQ + 0);  // g, b
-                        const double2 v1 = *reinterpret_cast<const double2*>(row + q * ROW_NYQ + 2);  // n b, b_s
-                        const double2 v2 = *reinterpret_cast<const double2*>(row + q * ROW_NYQ + 4);  // bsupv, bsubs
-                        const double2 v3 = *reinterpret_cast<const double2*>(row + q * ROW_NYQ + 6);  // bsubu, bsubv
-                        a0 = fma(v0.x, ca, a0);   // sqrt g
-                        a1 = fma(v0.y, ca, a1);   // B
-                        a2 = fma(v0.y, sa, a2);   // sum b sin
-                        a3 = fma(v1.x, sa, a3);   // sum n b sin
-                        a4 = fma(v1.y, ca, a4);   // dB/ds
-                        a5 = fma(v2.x, ca, a5);   // B^phi
-                        a6 = fma(v2.y, sa, a6);   // B_s
-                        a7 = fma(v3.x, ca, a7);   // B_theta
-                        a8 = fma(v3.y, ca, a8);   // B_phi
-                    }
-                    const double dm = (double)m;
-                    sqrtg += a0; B += a1; B_t = fma(-dm, a2, B_t); B_p += a3; B_s += a4;
-                    Bsup_p += a5; Bsub_s += a6; Bsub_t += a7; Bsub_p += a8;
-                    const double cnx = fma(cm, c1, -(sm * s1));
-                    sm = fma(sm, c1, cm * s1);
-                    cm = cnx;
-                }
-            }
-            GeoSums g;
-            g.R = R; g.R_s = R_s; g.R_t = R_t; g.R_p = R_p; g.Z_s = Z_s; g.Z_t = Z_t; g.Z_p = Z_p; g.L_s = L_s; g.L_t = L_t; g.L_p = L_p;
-            g.sqrtg = sqrtg; g.B = B; g.B_s = B_s; g.B_t = B_t; g.B_p = B_p; g.Bsup_p = Bsup_p; g.Bsub_s = Bsub_s; g.Bsub_t = Bsub_t; g.Bsub_p = Bsub_p;
+            double th; int nit; bool ok;
+            const GeoSums g = point_sums(s_mn, s_nyq, theta_p, phi, th, nit, ok);
             if constexpr (NT1 == 0 && NT2 == 0) {
                 for (int jf = jl; jf < p.nl; jf += P) {           // the same sums zero, one, two, ... poloidal turns on
                     const double tp = p.theta[jf];
@@ -1074,7 +1172,7 @@ static int launch_geometry(const GeoParams& p, cudaStream_t st) {
     constexpr int GEO_THREADS = GeoThreads<NT1>::value;
     const size_t e_mn = (NT1 > 0) ? (size_t)(NT1 + 1) * ROWP_MN : (size_t)ROW_MN, e_nyq = (NT2 > 0) ? (size_t)(NT2 + 1) * ROWP_NYQ : (size_t)ROW_NYQ;
     const bool newton_smem = IBS_GEO_SMEM_NEWTON && NT1 > 0 && p.M1 <= GEO_SMEM_NEWTON_MAX_M;
-    const size_t smem = 16 + ((size_t)p.M1 * e_mn + (size_t)p.M2 * e_nyq + (newton_smem ? (size_t)2 * p.M1 * GEO_THREADS : 0)) * sizeof(double);
+    size_t smem = 16 + ((size_t)p.M1 * e_mn + (size_t)p.M2 * e_nyq + (newton_smem ? (size_t)2 * p.M1 * GEO_THREADS : 0)) * sizeof(double);
     if (smem > 220 * 1024) { set_error("Fourier tables of one surface do not fit in shared memory"); return IBS_ERR_UNSUPPORTED; }
     static bool configured[IBS_MAX_DEVICES] = {false};     // per instantiation and per device (the attribute is per device)
     const int dslot = current_device_slot();
@@ -1084,13 +1182,23 @@ static int launch_geometry(const GeoParams& p, cudaStream_t st) {
     }
     int per_sm = 0;
     IBS_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, GEO_THREADS, smem));
+    // The mirror fold stages two surfaces' tables.  Whether the grid allows it is only known in the kernel, so the second
+    // slot is reserved only when it costs no CTAs / SM (at mpol = 80 it is 12 KB; above ~55 KB per surface it would lower
+    // the occupancy of every axisymmetric launch, and such tables then keep the periodicity fold alone).
+    GeoParams q = p;
+    q.tab_slots = 1;
+    if (NT1 == 0 && p.fold && 2 * smem - 16 <= 220 * 1024) {
+        int per_sm2 = 0;
+        IBS_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm2, kern, GEO_THREADS, 2 * smem - 16));
+        if (per_sm2 >= per_sm) { q.tab_slots = 2; smem = 2 * smem - 16; }
+    }
     if (per_sm < 1) per_sm = 1;
     const int tiles = (p.nalpha * p.nl + GEO_THREADS - 1) / GEO_THREADS;
     const long long slots = (long long)num_sms() * per_sm;
     // persistent 1-D grid: one CTA per resident slot (or per tile when there is less work than that)
     const long long W = (long long)p.ns * tiles;
     const int grid = (int)(W < slots ? W : slots);
-    kern<<<grid, GEO_THREADS, smem, st>>>(p);
+    kern<<<grid, GEO_THREADS, smem, st>>>(q);
     IBS_CUDA_CHECK(cudaGetLastError());
     return IBS_OK;
 }
@@ -1219,6 +1327,7 @@ static int geometry_run(const double* tab_mn, const double* tab_nyq, const doubl
     p.phi_center = phi_center; p.psi_e = -phiedge / (2.0 * 3.141592653589793); p.L_ref = aminor_p;
     p.base_out = base_out; p.theta_vmec_out = theta_vmec_out; p.info_out = info_out;
     { const char* e = std::getenv("IBS_GEO_FOLD"); p.fold = !(e && e[0] == '0'); }
+    p.tab_slots = 1;
     if (info_out) IBS_CUDA_CHECK(cudaMemsetAsync(info_out, 0, (size_t)ns * nalpha * sizeof(int), st));
     int rc;
     if (NT1 == 0) rc = launch_geometry<0, 0>(p, st);
