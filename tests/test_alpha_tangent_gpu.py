@@ -5,13 +5,13 @@ Argument checks without a GPU; on the GPU: the value outputs equal ``geometry_ba
 tangent against Richardson-extrapolated central differences of the long-double field-line reference; the gradient against the
 three-line finite-difference path (bit-identical value, theta0 part, eigenfunction and flags; the finite difference converges
 to it at second order), against re-solved eigenvalues, and in the refinement of 64 surfaces."""
-import inspect
 
 import numpy as np
 import pytest
 
 from helpers import tables_from_fixture
-from test_geometry_shapes_gpu import LD, SHAPES, Shape, fieldlines_ld
+from geometry_ld import LD, fieldlines_ld
+from test_geometry_shapes_gpu import SHAPES, Shape
 
 FIXTURES = ["synthetic_d3d", "synthetic_ncsx", "synthetic_hberg", "ncsx_wout_op"]
 NBASE = 8
@@ -24,17 +24,7 @@ TAN_RTOL = 1e-11
 def _fieldlines_ld_alpha(tab, alpha, theta, phi_center=0.0, cols=None):
     """``fieldlines_ld`` with alpha and phi = phi_center + (theta - alpha) / iota in long double, so that central differences
     in alpha with steps ~1e-5 are not limited by the float64 rounding of phi."""
-    src = inspect.getsource(fieldlines_ld).replace("def fieldlines_ld(", "def _f(", 1)
-    subs = [("alpha = np.asarray(alpha, dtype=np.float64)", "alpha = np.asarray(alpha, dtype=LD)"),
-            ("phi64 = phi_center + (th_p[None, :] - alpha2[js][:, None]) / sc[1]",
-             "phi_ld = LD(phi_center) + (th_p.astype(LD)[None, :] - alpha2[js][:, None]) / LD(sc[1]); phi64 = phi_ld.astype(np.float64)"),
-            ("phi, tp = phi64.astype(LD).ravel(),", "phi, tp = phi_ld.ravel(),")]
-    for a, b in subs:
-        assert a in src, a
-        src = src.replace(a, b)
-    ns = dict(fieldlines_ld.__globals__)
-    exec(src, ns)
-    return ns["_f"](tab, alpha, theta, phi_center, cols)
+    return fieldlines_ld(tab, np.asarray(alpha, dtype=LD), theta, phi_center, cols, phi_ld=True)
 
 
 def richardson_alpha(tab, alpha, theta, phi_center, cols, h=2.0 ** -15):

@@ -3,7 +3,7 @@
 ``geometry_dispatch`` picks the kernel from the toroidal width of the two mode sets (nt1 = max |xn| / nfp of the ``mn`` set,
 nt2 the same for the Nyquist set): ``geometry_kernel<0,0>`` for axisymmetric tables, ``<6,8>``, ``<11,13>``, ``<16,18>``, and
 ``geometry3d_kernel`` above that (or with ``IBS_GEO3D=1``).  Each shape below is a synthetic equilibrium made to land on one of
-them, at the widths on either side of every switch and at several field periods.  The reference, ``fieldlines_ld``, restates
+them, at the widths on either side of every switch and at several field periods.  The reference, ``geometry_ld.fieldlines_ld``, restates
 ``oracle.ballooning_oracle.fieldlines`` in long double (64-bit mantissa): it is ~1000x sharper than float64, so the bound on the
 kernel is the kernel's own rounding and not the reference's.  ``engine.geometry_full`` is held to the same reference.
 
@@ -14,8 +14,8 @@ import re
 import numpy as np
 import pytest
 
-LD = np.longdouble
-PI_LD = np.arccos(LD(-1))
+from geometry_ld import fieldlines_ld, make_tables
+
 EPS = np.finfo(np.float64).eps
 
 # Bounds, set from the worst case over all shapes measured on an NVIDIA B200 (1000 W power limit):
@@ -29,96 +29,6 @@ BASE_RTOL = 2e-13          # each base array, relative to the maximum of its row
 THETA_VMEC_EPS = 24        # theta_vmec within THETA_VMEC_EPS * eps * max(1, |theta_vmec|)
 
 IBS_ERR_INVALID, IBS_ERR_UNSUPPORTED = 1, 3
-
-
-# ---------------------------------------------------------------------------------------------------------------------
-# extended-precision reference
-# ---------------------------------------------------------------------------------------------------------------------
-def fieldlines_ld(tab, alpha, theta, phi_center=0.0, cols=None):
-    """``oracle.ballooning_oracle.fieldlines`` (utils.py:161-720, hot subset) in long double.
-
-    phi is formed in float64 exactly as K1 forms it, ``phi_center + (theta - alpha) / iota``; from there on everything is long
-    double.  theta_vmec is solved by Newton to the long-double rounding level (a float64 Newton only supplies the start).
-    ``alpha`` is ``(nalpha,)`` or ``(ns, nalpha)``; ``cols`` picks the points of the line to evaluate (each point is
-    independent).  Returns a dict of ``(ns, nalpha, ncols)`` long-double arrays: the eight base arrays and ``theta_vmec``."""
-    from ideal_ballooning_solver_b200.engine import BASE_NAMES
-    theta = np.asarray(theta, dtype=np.float64)
-    cols = np.arange(theta.size) if cols is None else np.asarray(cols)
-    th_p = theta[cols]
-    ns = tab.tab_mn.shape[0]
-    alpha = np.asarray(alpha, dtype=np.float64)
-    alpha2 = np.broadcast_to(alpha, (ns, alpha.shape[-1]))
-    na, nc = alpha2.shape[1], th_p.size
-    xm, xn, xmq, xnq = (np.asarray(a, dtype=LD) for a in (tab.xm, tab.xn, tab.xm_nyq, tab.xn_nyq))
-    xm64, xn64 = np.asarray(tab.xm, np.float64), np.asarray(tab.xn, np.float64)
-    psi_e = -LD(tab.phiedge) / (2 * PI_LD)
-    L_ref = LD(tab.Aminor_p)
-    B_ref = 2 * abs(psi_e) / (L_ref * L_ref)
-    sgn = LD(np.sign(float(psi_e)))
-    MU0 = 4 * PI_LD * LD(10) ** -7
-    out = {k: np.empty((ns, na, nc), dtype=LD) for k in BASE_NAMES + ("theta_vmec",)}
-    for js in range(ns):
-        sc = tab.scal[js]
-        s, iota, d_iota, dpds, shat = (LD(v) for v in sc[:5])
-        phi64 = phi_center + (th_p[None, :] - alpha2[js][:, None]) / sc[1]                   # utils.py:373, float64 as in K1
-        phi, tp = phi64.astype(LD).ravel(), np.broadcast_to(th_p.astype(LD), (na, nc)).ravel()
-        lm64 = tab.tab_mn[js, 2]
-        lm = lm64.astype(LD)
-        # theta_vmec + sum l sin(m theta_vmec - n phi) = theta_pest  (utils.py:391-416)
-        th64 = tp.astype(np.float64)
-        for _ in range(40):
-            ang = xm64[:, None] * th64[None] - xn64[:, None] * phi64.ravel()[None]
-            d = (th64 + lm64 @ np.sin(ang) - th_p[None, :].repeat(na, 0).ravel()) / (1 + (lm64 * xm64) @ np.cos(ang))
-            th64 = th64 - d
-            if np.max(np.abs(d)) < 1e-13:
-                break
-        th = th64.astype(LD)
-        for _ in range(8):
-            ang = xm[:, None] * th[None] - xn[:, None] * phi[None]
-            d = (th + lm @ np.sin(ang) - tp) / (1 + (lm * xm) @ np.cos(ang))
-            th = th - d
-            if np.all(np.abs(d) <= 1e-18 * np.maximum(1, np.abs(th))):
-                break
-        else:
-            raise AssertionError("long-double Newton for theta_vmec did not converge")
-        # the 19 mode sums (utils.py:420-468)
-        row = lambda k: tab.tab_mn[js, k].astype(LD)
-        rowq = lambda k: tab.tab_nyq[js, k].astype(LD)
-        r, z, l, r_s, z_s, l_s = (row(k) for k in range(6))
-        ang = xm[:, None] * th[None] - xn[:, None] * phi[None]
-        c, sn = np.cos(ang), np.sin(ang)
-        R, R_s, Z_t, Z_p, L_t, L_p = np.stack([r, r_s, z * xm, -z * xn, l * xm, -l * xn]) @ c
-        R_t, R_p, Z_s, L_s = np.stack([-r * xm, r * xn, z_s, l_s]) @ sn
-        g, b, b_s, bsupv, bsubs, bsubu, bsubv = (rowq(k) for k in range(7))
-        ang = xmq[:, None] * th[None] - xnq[:, None] * phi[None]
-        c, sn = np.cos(ang), np.sin(ang)
-        sqrtg, B, B_s, Bsup_p, Bsub_t, Bsub_p = np.stack([g, b, b_s, bsupv, bsubu, bsubv]) @ c
-        B_t, B_p, Bsub_s = np.stack([-b * xmq, b * xnq, bsubs]) @ sn
-        # Cartesian dual basis, grad psi, grad alpha, drifts, GS2 normalisations (utils.py:474-720)
-        sp, cp = np.sin(phi), np.cos(phi)
-        X_t, X_p, X_s = R_t * cp, R_p * cp - R * sp, R_s * cp
-        Y_t, Y_p, Y_s = R_t * sp, R_p * sp + R * cp, R_s * sp
-        gs = [(Y_t * Z_p - Z_t * Y_p) / sqrtg, (Z_t * X_p - X_t * Z_p) / sqrtg, (X_t * Y_p - Y_t * X_p) / sqrtg]
-        gt = [(Y_p * Z_s - Z_p * Y_s) / sqrtg, (Z_p * X_s - X_p * Z_s) / sqrtg, (X_p * Y_s - Y_p * X_s) / sqrtg]
-        gp = [(Y_s * Z_t - Z_s * Y_t) / sqrtg, (Z_s * X_t - X_s * Z_t) / sqrtg, (X_s * Y_t - Y_s * X_t) / sqrtg]
-        gpsi = [v * psi_e for v in gs]
-        a_s = L_s - (phi - LD(phi_center)) * d_iota
-        ga = [a_s * gs[k] + ((1 + L_t) * gt[k] + (-iota + L_p) * gp[k]) for k in range(3)]
-        BxgB_ga = (Bsub_s * B_t * (L_p - iota) + Bsub_t * B_p * a_s + Bsub_p * B_s * (1 + L_t) - Bsub_p * B_t * a_s
-                   - Bsub_t * B_s * (L_p - iota) - Bsub_s * B_p * (1 + L_t)) / sqrtg
-        ga_ga = ga[0] * ga[0] + ga[1] * ga[1] + ga[2] * ga[2]
-        ga_gp = ga[0] * gpsi[0] + ga[1] * gpsi[1] + ga[2] * gpsi[2]
-        gp_gp = gpsi[0] * gpsi[0] + gpsi[1] * gpsi[1] + gpsi[2] * gpsi[2]
-        BxgB_gpsi = (Bsub_t * B_p - Bsub_p * B_t) / sqrtg * psi_e
-        sqrt_s = np.sqrt(s)
-        o = {"bmag": B / B_ref, "gradpar_theta_pest": L_ref * (iota * Bsup_p) / B, "gds2": ga_ga * L_ref * L_ref * s,
-             "gds21": ga_gp * shat / B_ref, "gds22": gp_gp * shat * shat / (L_ref * L_ref * B_ref * B_ref * s),
-             "gbdrift": -2 * B_ref * L_ref * L_ref * sqrt_s * BxgB_ga / (B * B * B) * sgn,
-             "cvdrift0": -BxgB_gpsi * 2 * shat / (B * B * B * sqrt_s) * sgn, "theta_vmec": th}
-        o["cvdrift"] = o["gbdrift"] - 2 * B_ref * L_ref * L_ref * sqrt_s * MU0 * dpds * sgn / (psi_e * B * B)
-        for k, v in o.items():
-            out[k][js] = v.reshape(na, nc)
-    return out
 
 
 # ---------------------------------------------------------------------------------------------------------------------
@@ -148,39 +58,6 @@ SHAPES = {
     "ntor24_long":   dict(kernel=K3D, mpol=18, ntor=24, nfp=2, nl=4097, span=20, phi_center=-1.3),
 }
 MAX_REF_POINTS = 400       # longer lines: the reference is evaluated on a seeded sample of this many points (and both ends)
-
-
-def _append_nyq(st, n, frac=1e-4):
-    """Append Nyquist modes (m, +-n nfp) for m = 0..3 with coefficients frac x the (m, 0) row."""
-    import dataclasses
-    xm, xn = [], []
-    for m in range(4):
-        for sgn in ((1,) if m == 0 else (1, -1)):
-            xm.append(m)
-            xn.append(sgn * n * st.nfp)
-    src = [int(np.flatnonzero((st.xm_nyq == m) & (st.xn_nyq == 0))[0]) for m in xm]
-    rng = np.random.default_rng(n)
-    w = frac * rng.uniform(0.5, 1.0, len(xm))
-    return dataclasses.replace(st, xm_nyq=np.concatenate([st.xm_nyq, xm]), xn_nyq=np.concatenate([st.xn_nyq, xn]),
-                               tab_nyq=np.concatenate([st.tab_nyq, st.tab_nyq[:, :, src] * w], axis=2),
-                               bsupumnc=np.concatenate([st.bsupumnc, st.bsupumnc[:, src] * w], axis=1))
-
-
-def make_tables(mpol, ntor, nfp, s, extra_nyq=None, seed=1):
-    """Surface tables of a synthetic equilibrium: a modified copy of the NCSX-shaped template (synthetic.py is unchanged)."""
-    from ideal_ballooning_solver_b200 import synthetic, tables
-    cfg = dict(synthetic.KINDS["ncsx"], mpol=mpol, ntor=ntor, nfp=nfp, ns=32)
-    if ntor == 0:
-        cfg["eps3d"] = 0.0
-    kinds = dict(synthetic.KINDS, shape=cfg)
-    orig = synthetic.KINDS
-    synthetic.KINDS = kinds
-    try:
-        w = synthetic.make_equilibrium("shape", seed=seed)
-    finally:
-        synthetic.KINDS = orig
-    st = tables.RadialSplines(w).evaluate(np.asarray(s, dtype=float))
-    return _append_nyq(st, extra_nyq) if extra_nyq else st
 
 
 def expected_kernel(st):
