@@ -47,6 +47,9 @@ SIGNATURES = {
     "ibs_count_above_batch": (c_int, [_D, _D, _D, c_int, c_int, c_double, _D, _I, c_void_p]),
     "ibs_marginal_batch": (c_int, [_D, _D, _D, _I, c_int, c_int, c_int, c_double, c_double, c_double, _D, _D, _D, _D, _I,
                                    c_void_p]),
+    "ibs_marginal_tangent_batch": (c_int, [_D, _D, _D, _D, _D, _I, c_int, c_int, c_int, c_double, c_double, c_double, _D, _D, _D,
+                                           _I, c_void_p]),
+    "ibs_marginal_sensitivities": (c_int, [_D, _D, _D, _I, c_int, c_int, c_int, c_double, _D, _D, _D, _D, c_void_p]),
     "ibs_scan_solve_argmax": (c_int, [_D, _D, _D, c_int, c_int, c_int, c_int, c_double, _D, c_int, _D, _D, _D, _I, _D, _D, c_void_p]),
     "ibs_scan_host": (c_int, [_D, _D, _D, _D, _D, _D, _D, c_int, c_int, c_int, c_double, c_double,
                               _D, c_int, _D, c_int, _D, c_int, c_double, _D, _D, _I, _D, _D, _D, _I]),

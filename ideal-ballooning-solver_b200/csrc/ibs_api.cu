@@ -31,6 +31,12 @@ int launch_identity_lines(int* line, int n, cudaStream_t st);
 int marginal_dispatch(const double* base, const double* dPdrho, const double* theta0, const int* line_of_solve, int nth0, int nsolve,
                       int N, double h, double kappa_max, double rtol, double* kappa_out, double* dlam_dkappa_out,
                       double* dkappa_dtheta0_out, double* X_out, int* info_out, cudaStream_t st);
+int marginal_tangent_dispatch(const double* base, const double* dbase, const double* dPdrho, const double* ddPdrho, const double* theta0,
+                              const int* line_of_solve, int nth0, int nsolve, int N, double h, double kappa_max, double rtol,
+                              double* kappa_out, double* grad_out, double* X_out, int* info_out, cudaStream_t st);
+int marginal_sensitivity_dispatch(const double* base, const double* dPdrho, const double* theta0, const int* line_of_solve, int nth0,
+                                  int nsolve, int N, double h, const double* kappa, const double* X, double* dk_dg, double* dk_dc,
+                                  cudaStream_t st);
 int launch_adjoint(const double* lam, const double* X, const double* dX, const double* f, const double* g_p,
                    const double* c_p, const double* f_p, int nsolve, int nparam, int N, double* grad, cudaStream_t st);
 int launch_sensitivity(const double* lam, const double* X, const double* dX, const double* f, int nsolve, int N,
@@ -366,6 +372,33 @@ int ibs_marginal_batch(const double* base, const double* dPdrho, const double* t
     keep_pool_cached();
     return marginal_dispatch(base, dPdrho, theta0, line_of_solve, nth0 > 0 ? nth0 : 1, nsolve, N, h, kappa_max, rtol, kappa_out,
                              dlam_dkappa_out, dkappa_dtheta0_out, X_out, info_out, (cudaStream_t)stream);
+}
+
+int ibs_marginal_tangent_batch(const double* base, const double* dbase, const double* dPdrho, const double* ddPdrho,
+                               const double* theta0, const int* line_of_solve, int nth0, int nsolve, int N, double h,
+                               double kappa_max, double rtol, double* kappa_out, double* grad_out, double* X_out, int* info_out,
+                               void* stream) {
+    IBS_REQUIRE(nsolve >= 0 && N >= 5 && N <= 65538, "need nsolve >= 0 and 5 <= N <= 65538");
+    if (nsolve == 0) return IBS_OK;
+    IBS_REQUIRE(base && dbase && dPdrho && ddPdrho && theta0 && kappa_out && grad_out, "null pointer");
+    IBS_REQUIRE(line_of_solve || nth0 >= 1, "need line_of_solve or nth0 >= 1");
+    IBS_REQUIRE(h > 0.0, "h must be positive");
+    IBS_REQUIRE(kappa_max > 0.0 && rtol > 0.0 && rtol < 1.0, "need kappa_max > 0 and 0 < rtol < 1");
+    keep_pool_cached();
+    return marginal_tangent_dispatch(base, dbase, dPdrho, ddPdrho, theta0, line_of_solve, nth0 > 0 ? nth0 : 1, nsolve, N, h, kappa_max,
+                                     rtol, kappa_out, grad_out, X_out, info_out, (cudaStream_t)stream);
+}
+
+int ibs_marginal_sensitivities(const double* base, const double* dPdrho, const double* theta0, const int* line_of_solve, int nth0,
+                               int nsolve, int N, double h, const double* kappa, const double* X, double* dkappa_dg_out,
+                               double* dkappa_dc_out, void* stream) {
+    IBS_REQUIRE(nsolve >= 0 && N >= 5 && N <= 65538, "need nsolve >= 0 and 5 <= N <= 65538");
+    if (nsolve == 0) return IBS_OK;
+    IBS_REQUIRE(base && dPdrho && theta0 && kappa && X && dkappa_dg_out && dkappa_dc_out, "null pointer");
+    IBS_REQUIRE(line_of_solve || nth0 >= 1, "need line_of_solve or nth0 >= 1");
+    IBS_REQUIRE(h > 0.0, "h must be positive");
+    return marginal_sensitivity_dispatch(base, dPdrho, theta0, line_of_solve, nth0 > 0 ? nth0 : 1, nsolve, N, h, kappa, X,
+                                         dkappa_dg_out, dkappa_dc_out, (cudaStream_t)stream);
 }
 
 int ibs_adjoint_batch(const double* lam, const double* X, const double* dX, const double* f, const double* g_p,

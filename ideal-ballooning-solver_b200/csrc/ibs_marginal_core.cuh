@@ -25,6 +25,9 @@
 //
 // The optional outputs come from the null vector x* of K(kappa*), one twisted factorisation: forward pivots (kept in the
 // caller's X row as scratch), backward pivots, the twist row k = argmin |p_k + q_k - d_k|, then x from row k outwards.
+//
+// The first-order response of kappa* at x* (point_forms, point_sensitivities) gives d kappa* / d alpha from the records'
+// alpha-tangent and the per-point sensitivities d kappa* / d g_j, d kappa* / d c_j that the reverse mode of K1 consumes.
 #pragma once
 #include <cmath>
 #include <cstdint>
@@ -285,6 +288,68 @@ IBS_HD Derivs null_vector(const double* rec, const double* b, int N, double h2, 
     o.dlam_dkappa = qk / qf;
     o.dkappa_dtheta0 = -qt / qk;
     return o;
+}
+
+// ---- first-order response of kappa* at the null vector: alpha-tangent and per-point sensitivities ------------------------
+// For any quantity q that K depends on, d kappa* / dq = -x^T (dK/dq) x / qk with qk = x^T (dK/dkappa) x.  With the rows of
+// K as above, x^T K x = -sum_cells a_j (x_j - x_{j-1})^2 + sum_j C_j x_j^2, so point j enters through its g (the cells j and
+// j+1 that exist) and through its C (interior points only).  These terms are summed per point; the caller adds them up.
+
+// alpha-tangent of a point's record along (d8, ddP): the chain rule through marginal_record / raw_record
+IBS_HD MRec record_tangent(const double* b8, const double* d8, double dP, double ddP, double h2) {
+    const double B = b8[IBS_BASE_BMAG], dB = d8[IBS_BASE_BMAG];
+    const double gp = fabs(b8[IBS_BASE_GRADPAR]), dgp = (b8[IBS_BASE_GRADPAR] < 0.0 ? -1.0 : 1.0) * d8[IBS_BASE_GRADPAR];
+    const double gpB = gp * B, gpoB = gp / B, mdP = -2.0 * h2 * dP / gpB;
+    const double d_gpoB = (dgp - gpoB * dB) / B;                                  // d (gp / B)
+    const double d_mdP = -2.0 * h2 * ddP / gpB - mdP * (dgp / gp + dB / B);       // d (-2 h^2 dP / (gp B))
+    const double gb = b8[IBS_BASE_GBDRIFT], dgb = d8[IBS_BASE_GBDRIFT];
+    MRec t;
+    t.G0 = d_gpoB * b8[IBS_BASE_GDS2] + gpoB * d8[IBS_BASE_GDS2];
+    t.G1 = 2.0 * (d_gpoB * b8[IBS_BASE_GDS21] + gpoB * d8[IBS_BASE_GDS21]);
+    t.G2 = d_gpoB * b8[IBS_BASE_GDS22] + gpoB * d8[IBS_BASE_GDS22];
+    t.Cg = d_mdP * gb + mdP * dgb;
+    t.C1 = d_mdP * b8[IBS_BASE_CVDRIFT0] + mdP * d8[IBS_BASE_CVDRIFT0];
+    t.Cd = d_mdP * (b8[IBS_BASE_CVDRIFT] - gb) + mdP * (d8[IBS_BASE_CVDRIFT] - dgb);
+    return t;
+}
+
+// (x_j - x_{j-1})^2 + (x_{j+1} - x_j)^2 over the cells of point j that exist (x: the solve's N values)
+IBS_HD double cell_weight(const double* x, int N, int j) {
+    double w = 0.0;
+    if (j > 0) { const double d = x[j] - x[j - 1]; w = d * d; }
+    if (j < N - 1) { const double d = x[j + 1] - x[j]; w = fma(d, d, w); }
+    return w;
+}
+
+struct PointForms { double qk, qa; };
+
+// point j's share of qk = x^T dK/dkappa x and of qa = x^T dK/dalpha x.  b, db: the line's 8 x N base arrays and their alpha-
+// tangent (db = null: qk only); dP, ddP: dPdrho and its tangent.
+IBS_HD PointForms point_forms(const double* b, const double* db, int N, int j, double dP, double ddP, double h2, double th0, double kap,
+                              const double* x) {
+    double b8[IBS_NBASE];
+    for (int q = 0; q < IBS_NBASE; ++q) b8[q] = b[(size_t)q * N + j];
+    double R;
+    const MRec m = marginal_record(b8, dP, h2, R);
+    const bool inner = j > 0 && j < N - 1;
+    const double x2 = inner ? x[j] * x[j] : 0.0;
+    PointForms o;
+    o.qk = fma(2.0 * kap, m.Cd, c1_of(m, th0)) * x2;
+    o.qa = 0.0;
+    if (db) {
+        double d8[IBS_NBASE];
+        for (int q = 0; q < IBS_NBASE; ++q) d8[q] = db[(size_t)q * N + j];
+        const MRec t = record_tangent(b8, d8, dP, ddP, h2);
+        o.qa = fma(kap * fma(kap, t.Cd, c1_of(t, th0)), x2, -g_of(t, th0) * cell_weight(x, N, j));
+    }
+    return o;
+}
+
+// per-point sensitivities of kappa* in the reference's unscaled coefficients (utils.py:1560-1562) at kappa*:
+//   d kappa* / d g_j = cell_weight_j / qk,   d kappa* / d c_j = -2 h^2 x_j^2 / qk (0 at the Dirichlet ends)
+IBS_HD void point_sensitivities(const double* x, int N, int j, double h2, double inv_qk, double& dk_dg, double& dk_dc) {
+    dk_dg = cell_weight(x, N, j) * inv_qk;
+    dk_dc = (j > 0 && j < N - 1) ? -2.0 * h2 * x[j] * x[j] * inv_qk : 0.0;
 }
 
 // ---- one lane: CHAIN consecutive solves ----------------------------------------------------------------------------------

@@ -325,13 +325,9 @@ class Marginal:
         return self.info >> 16
 
 
-def marginal_batch(base, dPdrho, theta0, h: float, nth0: Optional[int] = None, line_of_solve=None, kappa_max: float = 1e3,
-                   rtol: float = 1e-12, want_X: bool = False, want_derivs: bool = False) -> Marginal:
-    """Critical pressure-gradient factor of each solve: the smallest ``kappa`` at which the discrete pencil, with ``p'``
-    scaled by ``kappa`` at fixed geometry (``cvdrift -> gbdrift + kappa (cvdrift - gbdrift)``, ``dPdrho -> kappa dPdrho``),
-    has an eigenvalue above 0.  ``kappa* < 1`` means unstable as given.  Batch shape as :func:`solve_base_batch`."""
-    _lib.require_cuda()
-    lib = _lib.load()
+def _marginal_batch_args(base, dPdrho, theta0, nth0, line_of_solve):
+    """Batch shape of the marginal entry points (as :func:`solve_base_batch`): ``base (nline, 8, N)``, ``dPdrho (nline,)``,
+    ``theta0 (nsolve,)`` and the line of each solve (``line_of_solve`` or ``nth0``)."""
     dev = base.device
     N = base.shape[-1]
     base = _f64(base, dev, "base").reshape(-1, NBASE, N)
@@ -348,6 +344,18 @@ def marginal_batch(base, dPdrho, theta0, h: float, nth0: Optional[int] = None, l
         nth0 = n // base.shape[0]
     if line_of_solve is None and nth0 * base.shape[0] < n:
         raise ValueError("not enough field lines for the requested solves")
+    return base, dP, theta0, line_of_solve, nth0
+
+
+def marginal_batch(base, dPdrho, theta0, h: float, nth0: Optional[int] = None, line_of_solve=None, kappa_max: float = 1e3,
+                   rtol: float = 1e-12, want_X: bool = False, want_derivs: bool = False) -> Marginal:
+    """Critical pressure-gradient factor of each solve: the smallest ``kappa`` at which the discrete pencil, with ``p'``
+    scaled by ``kappa`` at fixed geometry (``cvdrift -> gbdrift + kappa (cvdrift - gbdrift)``, ``dPdrho -> kappa dPdrho``),
+    has an eigenvalue above 0.  ``kappa* < 1`` means unstable as given.  Batch shape as :func:`solve_base_batch`."""
+    _lib.require_cuda()
+    lib = _lib.load()
+    base, dP, theta0, line_of_solve, nth0 = _marginal_batch_args(base, dPdrho, theta0, nth0, line_of_solve)
+    dev, n, N = base.device, theta0.numel(), base.shape[-1]
     new = lambda: torch.empty((n,), dtype=torch.float64, device=dev)
     kappa = new()
     dl, dk = (new(), new()) if want_derivs else (None, None)
@@ -358,6 +366,55 @@ def marginal_batch(base, dPdrho, theta0, h: float, nth0: Optional[int] = None, l
                                     float(kappa_max), float(rtol), _ptr(kappa), _ptr(dl), _ptr(dk), _ptr(X), _ptr(info), _stream())
     _lib.check(rc, "ibs_marginal_batch")
     return Marginal(kappa, dl, dk, X, info)
+
+
+@dataclasses.dataclass
+class MarginalTangent(Marginal):
+    grad: Optional[torch.Tensor] = None        # (nsolve, 2) (d kappa* / d alpha, d kappa* / d theta0); NaN where kappa* is not finite
+
+
+def marginal_tangent_batch(base, dbase, dPdrho, ddPdrho, theta0, h: float, nth0: Optional[int] = None, line_of_solve=None,
+                           kappa_max: float = 1e3, rtol: float = 1e-12, want_X: bool = False) -> MarginalTangent:
+    """:func:`marginal_batch` with the exact alpha-derivative of kappa* (``ibs_marginal_tangent_batch``): ``dbase (nline, 8, N)``
+    and ``ddPdrho (nline,)`` are the alpha-tangent of the lines (``geometry_tangent_batch``).  ``kappa``, ``X``, ``info`` and
+    ``grad[:, 1]`` (also ``dkappa_dtheta0``) are ``marginal_batch``'s bits on the same batch; ``grad[:, 0]`` is
+    ``-x^T dK/dalpha x / x^T dK/dkappa x`` at the null vector."""
+    _lib.require_cuda()
+    lib = _lib.load()
+    base, dP, theta0, line_of_solve, nth0 = _marginal_batch_args(base, dPdrho, theta0, nth0, line_of_solve)
+    dev, n, N = base.device, theta0.numel(), base.shape[-1]
+    dbase = _f64(dbase, dev, "dbase").reshape(base.shape)
+    ddP = _f64(ddPdrho, dev, "ddPdrho").reshape(dP.shape)
+    kappa = torch.empty((n,), dtype=torch.float64, device=dev)
+    grad = torch.empty((n, 2), dtype=torch.float64, device=dev)
+    X = torch.empty((n, N), dtype=torch.float64, device=dev) if want_X else None
+    info = torch.empty((n,), dtype=torch.int32, device=dev)
+    with torch.cuda.device(dev):
+        rc = lib.ibs_marginal_tangent_batch(_ptr(base), _ptr(dbase), _ptr(dP), _ptr(ddP), _ptr(theta0), _ptr(line_of_solve),
+                                            int(nth0 or 1), n, N, float(h), float(kappa_max), float(rtol), _ptr(kappa), _ptr(grad),
+                                            _ptr(X), _ptr(info), _stream())
+    _lib.check(rc, "ibs_marginal_tangent_batch")
+    return MarginalTangent(kappa, None, grad[:, 1], X, info, grad)
+
+
+def marginal_sensitivities(base, dPdrho, theta0, h: float, kappa, X, nth0: Optional[int] = None, line_of_solve=None):
+    """Per-point ``(d kappa* / d g_j, d kappa* / d c_j)`` (each ``(nsolve, N)``) in the coefficients of
+    :func:`solve_base_batch` at kappa* (``ibs_marginal_sensitivities``): the derivatives of the matrix eigenvalue that defines
+    kappa*, from ``kappa`` and the null vector ``X`` as ``marginal_batch(..., want_X=True)`` returns them.  NaN rows where
+    kappa* is not finite.  Batch shape as :func:`marginal_batch`."""
+    _lib.require_cuda()
+    lib = _lib.load()
+    base, dP, theta0, line_of_solve, nth0 = _marginal_batch_args(base, dPdrho, theta0, nth0, line_of_solve)
+    dev, n, N = base.device, theta0.numel(), base.shape[-1]
+    kappa = _f64(kappa, dev, "kappa").reshape(n)
+    X = _f64(X, dev, "X").reshape(n, N)
+    dk_dg = torch.empty((n, N), dtype=torch.float64, device=dev)
+    dk_dc = torch.empty_like(dk_dg)
+    with torch.cuda.device(dev):
+        rc = lib.ibs_marginal_sensitivities(_ptr(base), _ptr(dP), _ptr(theta0), _ptr(line_of_solve), int(nth0 or 1), n, N, float(h),
+                                            _ptr(kappa), _ptr(X), _ptr(dk_dg), _ptr(dk_dc), _stream())
+    _lib.check(rc, "ibs_marginal_sensitivities")
+    return dk_dg, dk_dc
 
 
 # ---------------------------------------------------------------------------------------------

@@ -500,14 +500,19 @@ class TableGradient:
     def predict(self, tables0: engine.DeviceTables, tables_pert) -> np.ndarray:
         """First-order change of every surface's growth rate for each perturbed table set: ``(ndof, ns)``.  With the scalar
         gradients present the changes of ``scal``, ``phiedge`` and ``Aminor_p`` count too; without them they are ignored."""
-        out = []
-        for tp in tables_pert:
-            d = ((tp.tab_mn - tables0.tab_mn) * self.grad_mn).sum(dim=(1, 2)) + ((tp.tab_nyq - tables0.tab_nyq) * self.grad_nyq).sum(dim=(1, 2))
-            if self.grad_scal is not None:
-                d = (d + ((tp.scal - tables0.scal) * self.grad_scal).sum(1) + (tp.phiedge - tables0.phiedge) * self.grad_glob[:, 0]
-                     + (tp.Aminor_p - tables0.Aminor_p) * self.grad_glob[:, 1])
-            out.append(d.cpu().numpy())
-        return np.array(out).reshape(len(out), -1)
+        return _predict(self, tables0, tables_pert)
+
+
+def _predict(g, tables0: engine.DeviceTables, tables_pert) -> np.ndarray:
+    """Dot products of the table (and, when present, scalar) gradients of ``g`` with each perturbation: ``(ndof, ns)``."""
+    out = []
+    for tp in tables_pert:
+        d = ((tp.tab_mn - tables0.tab_mn) * g.grad_mn).sum(dim=(1, 2)) + ((tp.tab_nyq - tables0.tab_nyq) * g.grad_nyq).sum(dim=(1, 2))
+        if g.grad_scal is not None:
+            d = (d + ((tp.scal - tables0.scal) * g.grad_scal).sum(1) + (tp.phiedge - tables0.phiedge) * g.grad_glob[:, 0]
+                 + (tp.Aminor_p - tables0.Aminor_p) * g.grad_glob[:, 1])
+        out.append(d.cpu().numpy())
+    return np.array(out).reshape(len(out), -1)
 
 
 def table_gradient(tables0: engine.DeviceTables, alpha_star, theta0_star, theta, scalars: bool = False) -> TableGradient:
@@ -530,6 +535,105 @@ def table_gradient(tables0: engine.DeviceTables, alpha_star, theta0_star, theta,
     Q = (sc * sol.c).sum(dim=1) / (-dP)
     grads = engine.geometry_adjoint(tables0, a.reshape(-1), theta_np, t0, dP, sg, sc, sf, Q, want_scalars=scalars)
     return TableGradient(sol.lam.cpu().numpy(), *grads)
+
+
+# ---------------------------------------------------------------------------------------------
+# Marginal stability for an optimiser: refined per-surface minimum of kappa* and its gradient with respect to the equilibrium
+# ---------------------------------------------------------------------------------------------
+def refine_marginal(tables: engine.DeviceTables, alpha_guess, theta0_guess, theta, maxiter: int = 30, ftol: float = 5.0e-11,
+                    gtol: float = 2.0e-08, kappa_max: float = 1e3, rtol: float = 1e-12, max_rounds: int = 200, sync_every: int = 4,
+                    bounds=((0.0, float(np.pi)), (0.0, 0.5 * float(np.pi)))) -> RefineResult:
+    """Refinement of every surface's coarse minimum of kappa* (``marginal_scan``'s ``alpha_crit``, ``theta0_crit``): minimise
+    kappa*(alpha, theta0) per surface over the box ``bounds`` -- the ranges of the coarse grid the guesses come from (the
+    default is the reference's grid, alpha in [0, pi], theta0 in [0, pi/2]).  The method and the options are those of
+    ``refine_maxima(alpha_derivative="exact")``: the batched projected quasi-Newton method of ``csrc/ibs_refine_core.cuh``,
+    one round = K1 and its alpha-tangent on one line per surface (``engine.geometry_tangent_batch``) + ``engine.
+    marginal_tangent_batch`` (value kappa*, gradient (d kappa*/d alpha, d kappa*/d theta0)) + ``ibs_refine_step``.
+
+    A trial point stable up to ``kappa_max`` (kappa* = +inf) is not usable and the line search backtracks from it.  A surface
+    whose starting kappa* is not finite is not refined: it keeps its start and its value there (``success`` False).
+    ``fun`` is kappa* at the result."""
+    dev = tables.tab_mn.device
+    ns = tables.ns
+    theta_np = theta.cpu().numpy() if isinstance(theta, torch.Tensor) else np.asarray(theta, dtype=np.float64)
+    theta_d = torch.from_numpy(theta_np).to(dev)
+    h = engine.grid_spacing(theta_np)
+    as_dev = lambda a: (a if isinstance(a, torch.Tensor) else torch.as_tensor(np.asarray(a, dtype=np.float64))).to(dev).reshape(ns)
+    st = engine.RefineState(as_dev(alpha_guess), as_dev(theta0_guess), bounds=bounds)
+    rounds = 0
+    k_start = None
+    while rounds < max_rounds:
+        for _ in range(sync_every):
+            geo = engine.geometry_tangent_batch(tables, st.alphas3[:, 1:2], theta_d)
+            m = engine.marginal_tangent_batch(geo.base, geo.dbase, geo.dPdrho, geo.ddPdrho, st.theta0, h, nth0=1, kappa_max=kappa_max,
+                                              rtol=rtol)
+            if k_start is None:
+                k_start = m.kappa.clone()          # the first round evaluates every starting point
+            st.step(m.kappa, m.grad, m.info, ftol, gtol, maxiter)
+            rounds += 1
+        if int(st.nactive.item()) == 0:
+            break
+    S = st.state.cpu().numpy()
+    why = S[:, 19].astype(int)
+    unrefined = why == 5                           # failed at the start: kappa* not finite (or the solve flagged it) there
+    fun = np.where(unrefined, k_start.cpu().numpy(), S[:, 2])
+    return RefineResult(alpha=S[:, 0].copy(), theta0=S[:, 1].copy(), fun=fun, nit=S[:, 20].astype(int), nfev=S[:, 21].astype(int),
+                        success=np.isin(why, (1, 2, 3, 4)), nbatches=rounds)
+
+
+@dataclasses.dataclass
+class MarginalGradient:
+    kappa: np.ndarray          # (ns,) kappa* at (alpha*, theta0*)
+    finite: np.ndarray         # (ns,) bool: kappa* finite (the other rows of the gradients are 0)
+    grad_mn: torch.Tensor      # (ns, 6, mnmax)      d kappa* / d tab_mn
+    grad_nyq: torch.Tensor     # (ns, 7, mnmax_nyq)  d kappa* / d tab_nyq
+    grad_scal: Optional[torch.Tensor] = None    # (ns, 8)  d kappa* / d scal (marginal_gradient(..., scalars=True))
+    grad_glob: Optional[torch.Tensor] = None    # (ns, 2)  d kappa* / d (phiedge, Aminor_p)
+
+    def predict(self, tables0: engine.DeviceTables, tables_pert) -> np.ndarray:
+        """First-order change of every surface's kappa* for each perturbed table set: ``(ndof, ns)`` (as
+        ``TableGradient.predict``)."""
+        return _predict(self, tables0, tables_pert)
+
+
+def marginal_gradient(tables0: engine.DeviceTables, alpha_star, theta0_star, theta, scalars: bool = False, kappa_max: float = 1e3,
+                      rtol: float = 1e-12) -> MarginalGradient:
+    """Gradient of every surface's kappa* at (alpha*, theta0*) with respect to every Fourier table coefficient (and with
+    ``scalars=True`` the surface scalars and phiedge / Aminor_p): one kappa* solve per surface and one reverse-mode pass
+    through K1, with no adjoint code of its own.
+
+    kappa* scales as kappa*(t p') = kappa*(p') / t.  So on the tables T_kappa, whose p' (``scal[:, 3]``) is multiplied by each
+    surface's kappa*, K1 gives exactly the kappa*-scaled base arrays, and ``ibs_geometry_adjoint_scal`` fed with the per-point
+    sensitivities of kappa* (``engine.marginal_sensitivities``, with f not entering) returns d kappa* / d T_kappa.  Its p'
+    column multiplied by kappa* is d kappa* / d p'; every other column is d kappa* / dT as it stands.
+
+    At a refined interior minimum (``refine_marginal``) the minimum is stationary in (alpha, theta0), so this is the gradient of
+    the surface's refined ``kappa_min`` itself (envelope theorem).  At an unrefined grid point it is the gradient of kappa* at
+    that fixed (alpha, theta0).  Rows of surfaces whose kappa* is not finite (stable up to ``kappa_max``, bad input) are 0."""
+    dev = tables0.tab_mn.device
+    theta_np = theta.cpu().numpy() if isinstance(theta, torch.Tensor) else np.asarray(theta, dtype=np.float64)
+    h = engine.grid_spacing(theta_np)
+    a = torch.as_tensor(np.asarray(alpha_star, dtype=np.float64)).reshape(-1, 1).to(dev)
+    t0 = torch.as_tensor(np.asarray(theta0_star, dtype=np.float64)).reshape(-1).to(dev)
+    geo = engine.geometry_batch(tables0, a, theta_np)
+    m = engine.marginal_batch(geo.base, geo.dPdrho, t0, h, nth0=1, kappa_max=kappa_max, rtol=rtol, want_X=True)
+    fin = (m.kappa > 0) & (m.kappa < float("inf"))
+    ks = torch.where(fin, m.kappa, torch.ones_like(m.kappa))
+    scal_k = tables0.scal.clone()
+    scal_k[:, 3] *= ks
+    tk = dataclasses.replace(tables0, scal=scal_k)
+    geo_k = engine.geometry_batch(tk, a, theta_np)
+    c_k = _gcf_exact(geo_k, t0)[1]
+    dk_dg, dk_dc = engine.marginal_sensitivities(geo.base, geo.dPdrho, t0, h, m.kappa, m.X, nth0=1)
+    dk_dg = torch.where(fin[:, None], dk_dg, 0.0)
+    dk_dc = torch.where(fin[:, None], dk_dc, 0.0)
+    dPk = geo_k.dPdrho.reshape(-1)
+    Q = torch.where(fin, (dk_dc * c_k).sum(dim=1) / (-dPk), 0.0)
+    grads = engine.geometry_adjoint(tk, a.reshape(-1), theta_np, t0, dPk, dk_dg, dk_dc, torch.zeros_like(dk_dg), Q, want_scalars=scalars)
+    grads = [torch.where(fin.reshape((-1,) + (1,) * (g.dim() - 1)), g, 0.0) for g in grads]
+    if scalars:
+        grads[2][:, 3] *= ks
+    return MarginalGradient(m.kappa.cpu().numpy(), fin.cpu().numpy(), *grads)
 
 
 def save_results(path: str, dof_idx: int, iter0: int, result: BallScanResult) -> None:

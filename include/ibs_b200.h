@@ -288,6 +288,27 @@ int ibs_marginal_batch(const double* base, const double* dPdrho, const double* t
                        double* kappa_out, double* dlam_dkappa_out, double* dkappa_dtheta0_out, double* X_out,
                        int* info_out, void* stream);
 
+/* kappa* with its exact alpha-derivative: the lines' base arrays and their alpha-tangent from ibs_geometry_tangent_batch
+ * (dbase [nline][8][N], ddPdrho [nline]).  kappa_out, X_out, info_out and grad_out[:, 1] are the bits of ibs_marginal_batch's
+ * kappa_out, X_out, info_out and dkappa_dtheta0_out on the same batch;
+ *   grad_out [nsolve][2] = (d kappa* / d alpha, d kappa* / d theta0), d kappa* / d alpha = -x^T dK/dalpha x / x^T dK/dkappa x
+ *     at the null vector (the chain rule through the records); NaN where kappa* is not finite.
+ *   X_out [nsolve][N] or NULL; info_out [nsolve] or NULL.                                                               */
+int ibs_marginal_tangent_batch(const double* base, const double* dbase, const double* dPdrho, const double* ddPdrho,
+                               const double* theta0, const int* line_of_solve, int nth0, int nsolve, int N, double h,
+                               double kappa_max, double rtol, double* kappa_out, double* grad_out, double* X_out, int* info_out,
+                               void* stream);
+
+/* Per-point sensitivities of kappa* in the coefficients g, c of ibs_solve_base_batch (utils.py:1560-1562) at kappa*, i.e. of
+ * the matrix eigenvalue that defines kappa* (not the Simpson form of ibs_adjoint_sensitivities):
+ *   dkappa_dg [j] = ((x_j - x_{j-1})^2 + (x_{j+1} - x_j)^2) / qk  (only the cells that exist at j = 0 and N - 1),
+ *   dkappa_dc [j] = -2 h^2 x_j^2 / qk (0 at j = 0 and N - 1),   qk = x^T dK/dkappa x;  f does not enter at lam = 0.
+ * Batch shape as ibs_marginal_batch; kappa [nsolve] and X [nsolve][N] as it returns them (X_out, max 1).  Outputs
+ * [nsolve][N]; NaN rows where kappa* is not finite.                                                                   */
+int ibs_marginal_sensitivities(const double* base, const double* dPdrho, const double* theta0, const int* line_of_solve, int nth0,
+                               int nsolve, int N, double h, const double* kappa, const double* X, double* dkappa_dg_out,
+                               double* dkappa_dc_out, void* stream);
+
 /* ---- end-to-end host entry point -----------------------------------------------------------------
  * Coarse scan of ball_scan.py:248-295 for ns surfaces with HOST buffers: copies the tables to the
  * device, runs K1 (ns x nalpha lines) and K2+K3 with the fused arg-max (ns x nalpha x nth0 solves), and

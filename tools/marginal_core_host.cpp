@@ -31,3 +31,34 @@ extern "C" int marginal_host_sweep(const double* rec, int N, double th0, double 
     *phi = s.phi;
     return s.bad ? -1 : s.count;
 }
+
+// first-order response at kappa* (the per-point forms of marginal_tangent_kernel / marginal_sensitivity_kernel, summed in
+// point order): grad_a [nsolve] = d kappa* / d alpha = -qa / qk; dk_dg, dk_dc [nsolve][N]
+extern "C" void marginal_host_tangent(const double* base, const double* dbase, const double* dPdrho, const double* ddPdrho,
+                                      const double* theta0, const int* line_of_solve, int nth0, int nsolve, int N, double h,
+                                      const double* kappa, const double* X, double* grad_a) {
+    for (int s = 0; s < nsolve; ++s) {
+        const int line = line_of_solve ? line_of_solve[s] : s / nth0;
+        const size_t o = (size_t)line * IBS_NBASE * N;
+        double qk = 0.0, qa = 0.0;
+        for (int j = 0; j < N; ++j) {
+            const PointForms f = point_forms(base + o, dbase + o, N, j, dPdrho[line], ddPdrho[line], h * h, theta0[s], kappa[s],
+                                             X + (size_t)s * N);
+            qk += f.qk; qa += f.qa;
+        }
+        grad_a[s] = -qa / qk;
+    }
+}
+
+extern "C" void marginal_host_sensitivities(const double* base, const double* dPdrho, const double* theta0, const int* line_of_solve,
+                                            int nth0, int nsolve, int N, double h, const double* kappa, const double* X, double* dk_dg,
+                                            double* dk_dc) {
+    for (int s = 0; s < nsolve; ++s) {
+        const int line = line_of_solve ? line_of_solve[s] : s / nth0;
+        const double* b = base + (size_t)line * IBS_NBASE * N;
+        const double* x = X + (size_t)s * N;
+        double qk = 0.0;
+        for (int j = 0; j < N; ++j) qk += point_forms(b, nullptr, N, j, dPdrho[line], 0.0, h * h, theta0[s], kappa[s], x).qk;
+        for (int j = 0; j < N; ++j) point_sensitivities(x, N, j, h * h, 1.0 / qk, dk_dg[(size_t)s * N + j], dk_dc[(size_t)s * N + j]);
+    }
+}

@@ -31,6 +31,8 @@ def build(outdir="/tmp/mch"):
     lib.marginal_host_solve.argtypes = [v, v, v, v, v, v, i, i, i, d, d, d, v, v, v, v, v]
     lib.marginal_host_sweep.argtypes = [v, i, d, d, ctypes.POINTER(d)]
     lib.marginal_host_sweep.restype = i
+    lib.marginal_host_tangent.argtypes = [v, v, v, v, v, v, i, i, i, d, v, v, v]
+    lib.marginal_host_sensitivities.argtypes = [v, v, v, v, i, i, i, d, v, v, v, v]
     return lib
 
 
@@ -63,6 +65,26 @@ def solve(lib, base, dPdrho, theta0, h, nth0=None, line_of_solve=None, kappa_max
                             float(kappa_max), float(rtol), _p(kappa), _p(dl) if want_X else None, _p(dk) if want_X else None,
                             _p(X), _p(info))
     return dict(kappa=kappa, dlam_dkappa=dl, dkappa_dtheta0=dk, X=X, info=info, rec=rec, line_flags=flags)
+
+
+def tangent(lib, base, dbase, dPdrho, ddPdrho, theta0, h, kappa, X, nth0=1):
+    """d kappa* / d alpha of each solve along (dbase, ddPdrho) at (kappa, X) as ``solve`` returns them (scan-shaped batch)."""
+    c = lambda a: np.ascontiguousarray(a, dtype=np.float64)
+    base, dbase, dP, ddP, th0, kappa, X = (c(a) for a in (base, dbase, dPdrho, ddPdrho, theta0, kappa, X))
+    out = np.zeros(th0.size)
+    lib.marginal_host_tangent(_p(base), _p(dbase), _p(dP), _p(ddP), _p(th0), None, int(nth0), th0.size, base.shape[-1], float(h),
+                              _p(kappa), _p(X), _p(out))
+    return out
+
+
+def sensitivities(lib, base, dPdrho, theta0, h, kappa, X, nth0=1):
+    """(d kappa* / d g, d kappa* / d c) per point, each (nsolve, N)."""
+    c = lambda a: np.ascontiguousarray(a, dtype=np.float64)
+    base, dP, th0, kappa, X = (c(a) for a in (base, dPdrho, theta0, kappa, X))
+    dg, dc = np.zeros_like(X), np.zeros_like(X)
+    lib.marginal_host_sensitivities(_p(base), _p(dP), _p(th0), None, int(nth0), th0.size, base.shape[-1], float(h), _p(kappa), _p(X),
+                                    _p(dg), _p(dc))
+    return dg, dc
 
 
 def count_at(lib, rec_line, theta0, kappa):
